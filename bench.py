@@ -45,8 +45,9 @@ SAMPLINGS = ("global_uniform_balanced", "rank_strided_uniform", "stratified")
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
-    ap.add_argument("--warmup", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 200); --workload infer: timed batches (default one pass over the resident set)")
+    ap.add_argument("--warmup", type=int, default=None, help="warm-up steps (default 20); --workload infer: warm-up batches (default 3)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--molecules", type=int, default=0, help="molecules in the resident set (0 = BASELINE config)")
     ap.add_argument("--gemm", default="tcgen05", choices=["tcgen05", "simt"])
@@ -74,7 +75,39 @@ def parse():
     ap.add_argument("--workload", default="train", choices=["train", "infer", "wide"],
                     help="train = BASELINE configs[1]/[3] (the metric); wide = configs[4] (6 layers, hidden 1024, <=128 atoms; "
                          "data-parallel under torchrun like train); infer = configs[2] (batch 4096 eval forward, 1 GPU)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (rank 0); the inputs "
+                         "are seeded, so two builds run with the same arguments can be compared output for output "
+                         "(tools/compare_dumps.py). Training sums with atomics, so repeated runs agree up to summation order, not "
+                         "bit for bit; profiles/r3_dump_repeatability.json records how far apart two runs of one build were")
+    a = ap.parse_args()
+    if a.steps is not None and a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.warmup is not None and a.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if a.impl == "reference" or a.workload != "infer":
+        a.steps = 200 if a.steps is None else a.steps
+        a.warmup = 20 if a.warmup is None else a.warmup
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return a
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Writes every array as path/<name>.npy in the dtype it was computed in (float32 / float64)."""
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    for k, v in arrays.items():
+        if v.dtype not in (np.float32, np.float64):
+            raise TypeError(f"output {k}: {v.dtype}, expected float32 or float64")
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs, more than {DUMP_LIMIT_BYTES}")
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v)
 
 
 def peaks():
@@ -426,6 +459,15 @@ class TrainBench:
         if self.graphed is not None:
             self.graphed.flush()
 
+    def outputs(self):
+        """What a caller of the last step receives: the model after its optimiser update (flat parameters in
+        param_spec order, BatchNorm running statistics [L, 2, H]), the step's predicted spectra [batch, M] and its
+        loss and mean cosine."""
+        import torch
+        return {"params": self.fp.params, "bn_running": self.fp.bn_running,
+                "spectra": self.plan.buffer("prob", torch.float32, (self.batch, M)),
+                "loss": self.metrics[4:5], "cosine": self.metrics[5:6]}
+
     def device_barrier(self):
         """All ranks leave together, ON THE DEVICE: a tiny all-reduce on the compute stream; what is enqueued next
         (the first timing event) executes only after every rank has arrived."""
@@ -550,6 +592,8 @@ def run_ours(args):
     # ---- the timed region
     tb.plan.profile(False)  # resets the launch counter
     ms, per_step, clocks = tb.timed(ids_dev, W, K, with_sampler=True)
+    if args.dump_outputs and rank == 0:   # before the passes below run more steps on the same model
+        dump_outputs(args.dump_outputs, tb.outputs())
     _, launches = tb.plan.profile_read()
     if tb.graphed is not None:
         launches = int(round(K * tb.launches_per_step))
@@ -865,8 +909,10 @@ def pack_into(packer, k, ids):
 # ------------------------------------------------------------------------------------------
 # configs[2] and configs[4] on one GPU: secondary numbers carried by the N=1 line
 # ------------------------------------------------------------------------------------------
-def infer_bench(args, dev, n_mols, batch=4096, with_stages=True):
-    """BASELINE configs[2]: one pass of batched eval-mode prediction over n_mols resident molecules."""
+def infer_bench(args, dev, n_mols, batch=4096, with_stages=True, dump=None, steps=None, warmup=None):
+    """BASELINE configs[2]: batched eval-mode prediction over n_mols resident molecules, by default one pass (steps=None)
+    after 3 warm-up batches; `steps` batches run through a seeded permutation of the set, wrapping around it.
+    dump: directory for the spectra of the last timed batch (dump_outputs)."""
     import torch
     from eims_b200.engine import DeviceDataset, FlatParams, ModelDims, Plan
     from eims_b200.synth import synth_molecules
@@ -876,12 +922,17 @@ def infer_bench(args, dev, n_mols, batch=4096, with_stages=True):
     plan = Plan(d, batch, batch * MAX_ATOMS, 2 * (batch * MAX_ATOMS + 3 * batch), dev)
     fp = FlatParams(d, dev)
     init_weights(fp, d)
-    n_batches = n_mols // batch
+    per_pass = n_mols // batch
+    if per_pass == 0:
+        raise SystemExit(f"--workload infer: {n_mols} molecules are fewer than one batch of {batch}")
+    n_batches = per_pass if steps is None else steps
+    warmup = 3 if warmup is None else warmup
+    ids = lambda i: perm[i % per_pass * batch:(i % per_pass + 1) * batch]
     perm_h = np.random.default_rng(5).permutation(n_mols).astype(np.int32)
     perm = torch.from_numpy(perm_h).to(dev)
     out = torch.empty(batch, M, device=dev)
-    for i in range(3):
-        plan.infer_batch(ds, perm[i * batch:(i + 1) * batch], fp, out)
+    for i in range(warmup):
+        plan.infer_batch(ds, ids(i), fp, out)
     plan.check()
     torch.cuda.synchronize()
     sampler = ClockSampler(dev.index or 0)
@@ -889,14 +940,18 @@ def infer_bench(args, dev, n_mols, batch=4096, with_stages=True):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(n_batches):
-        plan.infer_batch(ds, perm[i * batch:(i + 1) * batch], fp, out)
+        plan.infer_batch(ds, ids(i), fp, out)
     e1.record()
     torch.cuda.synchronize()
     clocks = sampler.stop()
     ms = e0.elapsed_time(e1)
+    if dump:
+        dump_outputs(dump, {"spectra": out})
     res = {"metric": "gcn_eims_infer_molecules_per_sec", "value": n_batches * batch / (ms * 1e-3), "unit": UNIT, "ms_per_batch": ms / n_batches,
-           "batches": n_batches, "batch": batch, "resident_molecules": n_mols, "clocks": clocks,
-           "workload": f"BASELINE configs[2]: inference-only spectrum prediction for {n_mols} synthetic molecules (<=64 heavy atoms), batch {batch}, single B200; one pass over the resident set, spectra written to HBM"}
+           "batches": n_batches, "warmup": warmup, "batch": batch, "resident_molecules": n_mols, "clocks": clocks,
+           "workload": f"BASELINE configs[2]: inference-only spectrum prediction for {n_mols} synthetic molecules (<=64 heavy atoms), batch {batch}, single B200; "
+                       + ("one pass over the resident set" if steps is None else f"{n_batches} batches through a seeded permutation of the resident set")
+                       + ", spectra written to HBM"}
     if with_stages:
         plan.profile(True)
         n_prof = 5
@@ -996,8 +1051,8 @@ def run_infer(args):
     import torch
     dev = torch.device("cuda", int(os.environ.get("LOCAL_RANK", "0")))
     torch.cuda.set_device(dev)
-    r = infer_bench(args, dev, args.molecules or 1_000_000)
-    print(json.dumps({"metric": r["metric"], "value": r["value"], "unit": UNIT, "n_gpus": 1, "steps": r["batches"], "warmup": 3,
+    r = infer_bench(args, dev, args.molecules or 1_000_000, dump=args.dump_outputs, steps=args.steps, warmup=args.warmup)
+    print(json.dumps({"metric": r["metric"], "value": r["value"], "unit": UNIT, "n_gpus": 1, "steps": r["batches"], "warmup": r["warmup"],
                       "ms_per_step": r["ms_per_batch"], "higher_is_better": True, "dtype": "f32", "data": "synthetic", "clocks": r["clocks"],
                       "config": {"workload": r["workload"], "batch_per_gpu": r["batch"], "hidden_dim": H, "num_gcn_layers": L, "max_mz": M,
                                  "resident_molecules": r["resident_molecules"]}, "stages": r.get("stages")}))
