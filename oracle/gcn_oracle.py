@@ -126,20 +126,23 @@ def mol_edges(begin: np.ndarray, end: np.ndarray):
 
 
 def batch_graphs(mols):
-    """`dgl.batch` (GCN:295).  `mols` = list of (feat[n,6], bond_begin, bond_end)."""
+    """`dgl.batch` (GCN:295).  `mols` = list of (feat[n,F], bond_begin, bond_end); a 2-D feature array
+    keeps its own width F, a flat one is read as rows of 6 (the reference's atom features)."""
     srcs, dsts, feats, nn, ne = [], [], [], [], []
-    off = 0
+    off, width = 0, 6
     for feat, b, e in mols:
         s, d = mol_edges(np.asarray(b, np.int64), np.asarray(e, np.int64))
         srcs.append(s + off)
         dsts.append(d + off)
-        feats.append(np.asarray(feat, np.float32).reshape(-1, 6) if len(feat) else np.zeros((0, 6), np.float32))
+        f = np.asarray(feat, np.float32)
+        width = f.shape[1] if f.ndim == 2 else 6
+        feats.append(f.reshape(-1, width) if len(feat) else np.zeros((0, width), np.float32))
         nn.append(len(feat))
         ne.append(len(s))
         off += len(feat)
     cat = lambda xs, dt: np.concatenate(xs).astype(dt) if xs else np.zeros(0, dt)
     return dict(src=cat(srcs, np.int64), dst=cat(dsts, np.int64),
-                feat=np.concatenate(feats) if feats else np.zeros((0, 6), np.float32),
+                feat=np.concatenate(feats) if feats else np.zeros((0, width), np.float32),
                 batch_num_nodes=np.asarray(nn, np.int64), batch_num_edges=np.asarray(ne, np.int64),
                 num_nodes=off)
 
