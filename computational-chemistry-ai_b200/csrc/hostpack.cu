@@ -32,13 +32,8 @@ static int pack_impl(const eims_dataset* ds, const int32_t* ids, int32_t n, int3
   }
   const int64_t mzsz = pk ? (pk->mz_is_f64 ? 8 : 4) : 0;
   const bool fixed = cap_nodes > 0;
-  if (fixed && (atoms > cap_nodes || bonds > cap_bonds || (pk && peaks > cap_peaks))) {
-    eims_host_batch L{};
-    L.num_graphs = n; L.num_nodes = (int32_t)atoms; L.num_edges = (int32_t)(2 * bonds);
-    *lay = L;
-    return EIMS_ERR_CAPACITY;
-  }
-  const int64_t sz_atoms = fixed ? cap_nodes : atoms, sz_bonds = fixed ? cap_bonds : bonds, sz_peaks = fixed ? cap_peaks : peaks;
+  const int64_t sz_atoms = fixed ? cap_nodes : atoms, sz_peaks = fixed ? cap_peaks : peaks;
+  const int64_t sz_bonds = fixed ? (cap_bonds > 0 ? cap_bonds : 1) : bonds;
   eims_host_batch L{};
   int64_t off = 0;
   L.node_ptr = off; off = align256(off + 8 * (int64_t)(n + 1));
@@ -57,6 +52,8 @@ static int pack_impl(const eims_dataset* ds, const int32_t* ids, int32_t n, int3
   L.num_graphs = n; L.num_nodes = (int32_t)atoms; L.num_edges = (int32_t)(2 * bonds); L.feat_dim = node_feat_dim;
   L.mz_is_f64 = pk ? pk->mz_is_f64 : 0;
   *lay = L;
+  // the fixed layout comes back whatever the batch holds: a layout query (out == NULL) may name any molecules
+  if (fixed && (atoms > cap_nodes || bonds > cap_bonds || (pk && peaks > cap_peaks))) return EIMS_ERR_CAPACITY;
   if (off > capacity || (n > 0 && !out)) return EIMS_ERR_CAPACITY;  // out == NULL: layout query
   char* base = reinterpret_cast<char*>(out);
   int64_t* np_ = reinterpret_cast<int64_t*>(base + L.node_ptr);
@@ -99,6 +96,6 @@ extern "C" int eims_host_pack_batch_fixed(const eims_dataset* ds, const int32_t*
                                           int32_t max_mz, int64_t cap_nodes, int64_t cap_bonds, int64_t cap_peaks, void* out,
                                           int64_t capacity, eims_host_batch* lay) {
   if (cap_nodes < 1 || cap_bonds < 0 || cap_peaks < 0) return EIMS_ERR_ARG;
-  return pack_impl(ds, ids, n, node_feat_dim, max_mz, out, capacity, lay, cap_nodes, cap_bonds > 0 ? cap_bonds : 1, cap_peaks);
+  return pack_impl(ds, ids, n, node_feat_dim, max_mz, out, capacity, lay, cap_nodes, cap_bonds, cap_peaks);
 }
 #pragma GCC visibility pop

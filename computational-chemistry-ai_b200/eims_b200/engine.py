@@ -498,10 +498,11 @@ class Plan:
         return C.c_void_p(self._step_block.data_ptr() + int(index) * self._step_block_bytes)
 
     def step_blocks_args(self, steps, ids_list, dp_seqs):
-        """The host-side half of step_blocks_upload: the ctypes arrays of one launch (<= 16 blocks)."""
+        """The host-side half of step_blocks_upload: the ctypes arrays of one launch (<= 16 blocks).  An ids entry of
+        None makes that step's indirect batch build take molecules 0..n-1 of its dataset."""
         n = len(steps)
         arr = (Step * n)(*steps)
-        pid = (C.c_void_p * n)(*[t.data_ptr() for t in ids_list])
+        pid = (C.c_void_p * n)(*[None if t is None else t.data_ptr() for t in ids_list])
         seq = (C.c_uint32 * n)(*[int(x) & 0xffffffff for x in dp_seqs])
         return arr, pid, seq, n
 

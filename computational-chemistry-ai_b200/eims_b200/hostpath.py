@@ -376,14 +376,16 @@ class GraphedHostTrainer:
         self.out_host[n_local].copy_(self.metrics, non_blocking=True)      # the step's loss / cosine back to the host
         with torch.cuda.stream(self.copy_stream):
             self.slots[nxt].copy_(self.pinned[(n_local + 1) % (2 * self.G)], non_blocking=True)
-            check(self.lib.eims_batch_build(plan.h, C.byref(self._ds[nxt]), None, self.batch, C.c_void_p(self.copy_stream.cuda_stream)))
+            # indirect: K1 takes its sequence number (the zero-degree tag) from the step block, so every replay tags its
+            # batches anew; a number baked in at capture would repeat every other launch
+            check(self.lib.eims_batch_build_indirect(plan.h, C.byref(self._ds[nxt]), self.batch, C.c_void_p(self.copy_stream.cuda_stream)))
         cur.wait_stream(self.copy_stream)            # join
 
     def capture(self, step):
         """After prime() and a few eager steps elsewhere (modules loaded): capture the two group graphs."""
         plan = self.plan
         plan.select_step_block(0)
-        plan.step_blocks_upload([step], [self.slots[0]], [0], 0)   # loads the upload kernel (ids unused: K1 is not indirect here)
+        plan.step_blocks_upload([step], [None], [0], 0)   # loads the upload kernel; ids None: K1 reads the slot in order
         torch.cuda.synchronize(plan.device)
         seq0 = self.fused.seq if self.fused is not None else 0
         for s in range(2):
@@ -410,7 +412,7 @@ class GraphedHostTrainer:
                 seqs.append(self.fused.seq)
             else:
                 seqs.append(0)
-        self.plan.step_blocks_upload(list(steps), [self.slots[0]] * self.G, seqs, 0)
+        self.plan.step_blocks_upload(list(steps), [None] * self.G, seqs, 0)
         self.graphs[l % 2].replay()
         ev = torch.cuda.Event()
         ev.record(torch.cuda.current_stream(self.plan.device))

@@ -237,7 +237,8 @@ int eims_host_pack_batch(const eims_dataset* ds, const int32_t* ids, int32_t n, 
                          void* out, int64_t capacity, eims_host_batch* lay);
 /* The same with a FIXED layout: sections sized for cap_nodes atoms / cap_bonds bonds / cap_peaks peaks, so every batch
  * of n molecules has the same section offsets and nbytes - constant device pointers after the upload, which is what a
- * captured CUDA graph (copy + K1 + step, replayed) needs.  EIMS_ERR_CAPACITY when the batch does not fit. */
+ * captured CUDA graph (copy + K1 + step, replayed) needs.  EIMS_ERR_CAPACITY when the batch does not fit; `lay` then
+ * still holds the fixed layout and the batch's true num_nodes / num_edges, so a layout query may name any molecules. */
 int eims_host_pack_batch_fixed(const eims_dataset* ds, const int32_t* ids, int32_t n, int32_t node_feat_dim, int32_t max_mz,
                                int64_t cap_nodes, int64_t cap_bonds, int64_t cap_peaks, void* out, int64_t capacity,
                                eims_host_batch* lay);
