@@ -175,7 +175,7 @@ __device__ __forceinline__ bool last_block_ticket(unsigned int* counter, unsigne
 // pdl_sync(): `griddepcontrol.wait` blocks until the preceding kernel has completed and its
 // writes are visible (nothing - not even the device-side sizes in dims[] - is read before it),
 // then `griddepcontrol.launch_dependents` lets the next kernel's blocks be scheduled as soon as
-// this grid leaves room.  EIMS_PDL=0 in the environment turns the attribute off.
+// this grid leaves room.
 // -DEIMS_TIMELINE (tools/step_timeline.py; never in the product library): block 0 of every kernel
 // stamps the global timer right after its grid-dependency wait, i.e. when the preceding kernel of
 // the chain has completed, so consecutive stamps give the in-situ duration of every launch of a
@@ -231,15 +231,6 @@ inline int& dims_early_ref() {
   return v;
 }
 
-inline bool pdl_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("EIMS_PDL");
-    on = (e && e[0] == '0') ? 0 : 1;
-  }
-  return on != 0;
-}
-
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
   cudaLaunchConfig_t cfg = {};
@@ -251,7 +242,7 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 

@@ -202,33 +202,10 @@ struct DhSrc {
   const int* gptr;       // [B+1]
   const int* argmax;     // [B,H]
   int pooling;
-  // third source: the GraphConv input gradient computed on the fly from the layer above,
-  //   dh_i = (sum_{j in row i} da_j) * c_i * dropmask_i      (K2 backward form, A symmetric)
-  // which saves materialising dh (one launch, one [N,H] write and two reads per layer)
-  const float* da;       // [N,H] or null
-  const int* rowptr;
-  const int* col;
-  const float* norm;
-  DropCfg drop;
 };
 
 __device__ __forceinline__ float4 load_dh(const DhSrc& s, int i, int c, int H) {
   if (s.dh) return ldg4(s.dh + (int64_t)i * H + c);
-  if (s.da) {
-    const int e0 = __ldg(s.rowptr + i), e1 = __ldg(s.rowptr + i + 1);
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-    for (int e = e0; e < e1; ++e) {
-      const float4 v = ldg4(s.da + (int64_t)__ldg(s.col + e) * H + c);
-      acc.x = __fadd_rn(acc.x, v.x); acc.y = __fadd_rn(acc.y, v.y); acc.z = __fadd_rn(acc.z, v.z); acc.w = __fadd_rn(acc.w, v.w);
-    }
-    const float ci = __ldg(s.norm + i);
-    acc.x *= ci; acc.y *= ci; acc.z *= ci; acc.w *= ci;
-    if (s.drop.active()) {
-      const float4 m = drop_mask4(s.drop, (uint64_t)i * H + c);
-      acc.x *= m.x; acc.y *= m.y; acc.z *= m.z; acc.w *= m.w;
-    }
-    return acc;
-  }
   const int g = __ldg(s.gid + i);
   const int pd = s.pooling == EIMS_POOL_COMBINED ? 2 * H : H;
   float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -251,14 +228,13 @@ __device__ __forceinline__ float4 load_dh(const DhSrc& s, int i, int c, int H) {
 }
 
 // pass 1: column sums of dh and dh*xhat (fp64) -> dgamma, dbeta (into grads) and the two column means.
-__global__ void __launch_bounds__(256, 4) bn_bwd_stats_kernel(const int* __restrict__ dims, DhSrc src,
+__global__ void __launch_bounds__(256, 4) bn_bwd_stats_kernel(const int* __restrict__ dims, const float* __restrict__ dh,
                                                            const float* __restrict__ z, int H,
                                                            const float* __restrict__ mean, const float* __restrict__ invstd,
                                                            float* __restrict__ dgamma, float* __restrict__ dbeta,
                                                            float* __restrict__ means /*[2][H]*/, float* __restrict__ scratch,
                                                            int early) {
   const int N = pdl_sync_dims(dims, early).N;
-  src.drop = resolve_drop(src.drop);
   unsigned int* counter = reinterpret_cast<unsigned int*>(scratch);
   double* acc = reinterpret_cast<double*>(scratch + 16);
   const int cl = threadIdx.x & 15, rl = threadIdx.x >> 4;
@@ -270,7 +246,7 @@ __global__ void __launch_bounds__(256, 4) bn_bwd_stats_kernel(const int* __restr
     const int stride = gridDim.y * kRowLanes;
 #pragma unroll 4
     for (int r = blockIdx.y * kRowLanes + rl; r < N; r += stride) {
-      const float4 d = load_dh(src, r, c, H);
+      const float4 d = ldg4(dh + (int64_t)r * H + c);
       const float4 v = ldg4(z + (int64_t)r * H + c);
       af[0] += d.x; af[1] += d.y; af[2] += d.z; af[3] += d.w;
       bf[0] = fmaf(d.x, (v.x - mu.x) * is.x, bf[0]); bf[1] = fmaf(d.y, (v.y - mu.y) * is.y, bf[1]);
@@ -350,10 +326,9 @@ int launch_bn_bwd_stats_top(const int* dims, const float* dG, const float* zstat
   const int slabs = (H + kSlab - 1) / kSlab;
   // one graph per thread up to 37 row groups per slab (148 blocks at H = 256): the kernel is a chain of dependent
   // round trips (sizes -> operands -> shared-memory reduce -> atomics -> ticket -> finalize), so the four graphs a thread
-  // used to walk one after the other were pure latency (EIMS_BN_TOP_GPT = graphs per thread, for A/B)
-  static int gpt = 0;
-  if (!gpt) { const char* e = getenv("EIMS_BN_TOP_GPT"); gpt = e ? atoi(e) : 1; if (gpt < 1) gpt = 1; }
-  int rg = (max_graphs + gpt * kRowLanes - 1) / (gpt * kRowLanes);
+  // used to walk one after the other were pure latency
+  constexpr int kGraphsPerThread = 1;
+  int rg = (max_graphs + kGraphsPerThread * kRowLanes - 1) / (kGraphsPerThread * kRowLanes);
   if (rg > 37) rg = 37;
   if (rg < 1) rg = 1;
   launch_pdl(bn_bwd_stats_top_kernel, dim3(slabs, rg), dim3(256), 0, st, dims, dG, zstat, gptr, pooling, H, mean, invstd, dgamma, dbeta,
@@ -373,7 +348,6 @@ __global__ void __launch_bounds__(256, LAYER0 ? 2 : 4) bn_bwd_apply_kernel(
     const float* __restrict__ norm, float* __restrict__ q, float* __restrict__ dbias, const float* __restrict__ a0,
     int F, float* __restrict__ dW0, int early, int64_t q_lo_off) {
   const int N = pdl_sync_dims(dims, early).N;
-  src.drop = resolve_drop(src.drop);
   __shared__ float red[kRowLanes][kSlab];
   const int cl = threadIdx.x & 15, rl = threadIdx.x >> 4;
   const int c0 = blockIdx.x * kSlab, c = c0 + cl * 4;
@@ -448,14 +422,10 @@ __global__ void __launch_bounds__(256, LAYER0 ? 2 : 4) bn_bwd_apply_kernel(
   }
 }
 
-int launch_bn_bwd_stats(const int* dims, const float* dh, const float* dG, const int* gid, const int* gptr,
-                        const int* argmax, int pooling, const float* z, int H, const float* mean, const float* invstd,
-                        float* dgamma, float* dbeta, float* means, float* partials, int max_nodes, cudaStream_t st,
-                        const GatherSrc* gs) {
+int launch_bn_bwd_stats(const int* dims, const float* dh, const float* z, int H, const float* mean, const float* invstd,
+                        float* dgamma, float* dbeta, float* means, float* partials, int max_nodes, cudaStream_t st) {
   if (H % 4 || H > 4096) return EIMS_ERR_ARG;
-  DhSrc src{dh, dG, gid, gptr, argmax, pooling, nullptr, nullptr, nullptr, nullptr, DropCfg{}};
-  if (gs) { src.da = gs->da; src.rowptr = gs->rowptr; src.col = gs->col; src.norm = gs->norm; src.drop = gs->drop; }
-  launch_pdl(bn_bwd_stats_kernel, bn_grid(H, max_nodes), dim3(256), 0, st, dims, src, z, H, mean, invstd, dgamma, dbeta, means, partials,
+  launch_pdl(bn_bwd_stats_kernel, bn_grid(H, max_nodes), dim3(256), 0, st, dims, dh, z, H, mean, invstd, dgamma, dbeta, means, partials,
              dims_early_ref());
   return 0;
 }
@@ -463,16 +433,14 @@ int launch_bn_bwd_stats(const int* dims, const float* dh, const float* dG, const
 int launch_bn_bwd_apply(const int* dims, const float* dh, const float* dG, const int* gid, const int* gptr,
                         const int* argmax, int pooling, const float* z, int H, const float* mean, const float* invstd,
                         const float* gamma, const float* norm, float* dbias, const float* means, float* q, int max_nodes,
-                        cudaStream_t st, const float* a0, int F, float* dW0, const GatherSrc* gs, int64_t q_lo_off) {
+                        cudaStream_t st, const float* a0, int F, float* dW0, int64_t q_lo_off) {
   if (H % 4 || H > 4096 || (dW0 && (F < 1 || F > kMaxF0d)) || (q_lo_off & 3) || (dW0 && q_lo_off)) return EIMS_ERR_ARG;
-  DhSrc src{dh, dG, gid, gptr, argmax, pooling, nullptr, nullptr, nullptr, nullptr, DropCfg{}};
-  if (gs) { src.da = gs->da; src.rowptr = gs->rowptr; src.col = gs->col; src.norm = gs->norm; src.drop = gs->drop; }
+  const DhSrc src{dh, dG, gid, gptr, argmax, pooling};
   const dim3 grid = bn_grid(H, max_nodes);
   // the layer-0 variant (104 registers: two resident blocks per SM) is launched as one wave: 12.7 us against 16.3
-  static int l0_per_sm = 0;
-  if (!l0_per_sm) { const char* e = getenv("EIMS_BN_L0_BLOCKS_PER_SM"); l0_per_sm = e ? atoi(e) : 2; if (l0_per_sm < 1) l0_per_sm = 1; }
+  constexpr int kL0BlocksPerSm = 2;
   if (dW0)
-    launch_pdl(bn_bwd_apply_kernel<true>, bn_grid(H, max_nodes, l0_per_sm), dim3(256), 0, st, dims, src, z, H, mean, invstd, gamma, means, norm, q, dbias, a0, F, dW0, dims_early_ref(), (int64_t)0);
+    launch_pdl(bn_bwd_apply_kernel<true>, bn_grid(H, max_nodes, kL0BlocksPerSm), dim3(256), 0, st, dims, src, z, H, mean, invstd, gamma, means, norm, q, dbias, a0, F, dW0, dims_early_ref(), (int64_t)0);
   else
     launch_pdl(bn_bwd_apply_kernel<false>, grid, dim3(256), 0, st, dims, src, z, H, mean, invstd, gamma, means, norm, q, dbias, nullptr, 0, nullptr, dims_early_ref(), q_lo_off);
   return 0;
@@ -632,9 +600,8 @@ int launch_ln_bwd(const int* dims, const float* u, const float* y, const float* 
                   const float* stats, float drop_scale, float* du, float* dgamma, float* dbeta, float* dbias,
                   int max_graphs, cudaStream_t st) {
   if (W % 4 || W > 2048 || W < 4) return EIMS_ERR_ARG;
-  static int rpb = 0;  // rows per block (8 warps): one row per warp measured best (cfg 2: 9.7 us for the two launches, 11.9 with two rows)
-  if (!rpb) { const char* e = getenv("EIMS_LN_BWD_ROWS_PER_BLOCK"); rpb = e ? atoi(e) : 8; if (rpb < 1) rpb = 1; }
-  int blocks = (max_graphs + rpb - 1) / rpb;
+  constexpr int kRowsPerBlock = 8;  // (8 warps): one row per warp measured best (cfg 2: 9.7 us for the two launches, 11.9 with two rows)
+  int blocks = (max_graphs + kRowsPerBlock - 1) / kRowsPerBlock;
   if (blocks < 1) blocks = 1;
   if (blocks > 148) blocks = 148;
   size_t smem = (size_t)8 * 3 * W * sizeof(float);

@@ -205,9 +205,8 @@ extern "C" int eims_dp_adamw_fused_blk(int32_t rank, int32_t world, const uint64
   // runs NEXT TO the backward kernels, and every one of its blocks spins in wait_all until the slowest peer arrives:
   // with a block on every SM it took more from the backward pass than the overlap gave back (0.3558 vs 0.3473 ms per
   // step at N=2).  A handful of blocks is plenty for ~0.5 MB per rank with ~130 us of backward to hide under.
-  static int early_blocks = 0;
-  if (!early_blocks) { const char* e = getenv("EIMS_DP_EARLY_BLOCKS"); early_blocks = e ? atoi(e) : 16; if (early_blocks < 1) early_blocks = 1; }
-  if (bucket > 0 && blocks > early_blocks) blocks = early_blocks;
+  constexpr int kEarlyBlocks = 16;
+  if (bucket > 0 && blocks > kEarlyBlocks) blocks = kEarlyBlocks;
   launch_pdl(dp_adamw_kernel, dim3((unsigned)blocks), dim3(256), 0, (cudaStream_t)stream, pr, rank, world, m_slice, v_slice,
              zero_buf, range_off / 4, n4, per, seq, (int)bucket, ticket, k, reinterpret_cast<const StepBlock*>(step_block),
              timeout_ns);

@@ -17,7 +17,6 @@
 //              or red.global.add.v4.f32 (split-K).
 // Sizes M and K may live in device memory (atoms in the current batch) so a captured step
 // can be replayed; tiles past the live range exit before touching barriers or TMEM.
-#include <cstdlib>
 
 #include "common.cuh"
 #include "gemm_persist.cuh"
@@ -565,12 +564,10 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_3xtf32_kernel(const __grid_c
 
 
 // ---------------------------------------------------------------------------------------------
-// Persistent variant: one CTA per SM walks over a list of work items with two 256-column accumulators in TMEM, so the
-// epilogue of item i runs under the main loop of item i + 1.  Used for (a) launches with several 128 x 256 tiles per SM
-// (inference forwards when the planes kernel of gemm_tma.cu is off) and (b) the grouped data-gradient + weight-gradient
-// launch of a GraphConv layer: non-persistent, its 264 live CTAs at BASELINE cfg 2 are two waves of one tile each, i.e.
-// two pipeline fills and two exposed epilogues per SM; here every CTA takes one data-gradient tile and a k-slice of the
-// weight gradient sized ON THE DEVICE from the live atom count so that all CTAs end together (gemm_persist.cuh).
+// Persistent variant: one CTA per SM walks over the 128 x 256 output tiles of one store problem with two 256-column
+// accumulators in TMEM, so the epilogue of tile i runs under the main loop of tile i + 1.  Used for launches with several
+// tiles per SM (inference forwards when the planes kernel of gemm_tma.cu is off); the tiles are dealt out on the device
+// from the live row count (gemm_persist.cuh).
 // A kernel that allocates tensor memory runs ONE CTA per SM on this driver (cudaOccupancyMaxActiveBlocksPerMultiprocessor
 // says 1 for any kernel containing tcgen05.alloc, tools/ubench/occ_probe.cu), so overlap has to come from inside the CTA.
 //   warps 0-7  : A tile of every k-block of the CTA's item sequence, warps 8-15: B tile (global -> registers, prefetched
@@ -594,25 +591,23 @@ constexpr int kPersistSmem = kPersistOffStats + pg::kEpiWarps * 2 * pg::kStatCol
 // thread keeps the prefetched k-block at 16 / 32 registers.  `op_off` = byte offset of the operand's hi tile inside a
 // stage; its lo tile follows it.
 template <int ROWS, bool IS_B>
-__device__ __forceinline__ void persistent_producer(const Group& grp, const pg::Sched& sch, const int (&Mv)[2], const int (&Kv)[2],
-                                                    uint32_t smem_base, uint32_t full0, uint32_t empty0, uint32_t op_off) {
+__device__ __forceinline__ void persistent_producer(const Args& g, const pg::Sched& sch, int M, int K, uint32_t smem_base,
+                                                    uint32_t full0, uint32_t empty0, uint32_t op_off) {
   const int t = threadIdx.x & (kPersistGroupThreads - 1), lane = threadIdx.x & 31;
   TileRegs<ROWS, kPersistGroupThreads> regs;
   Operand<ROWS, kPersistGroupThreads> op;
   pg::Cursor cur{0, sch.u0};
   pg::Item it;
-  int i = 0, klim = 0;
+  int i = 0;
   auto enter = [&]() -> bool {
     if (!pg::next_item<1>(sch, cur, it)) return false;
-    const Args& g = it.prob ? grp.g[1] : grp.g[0];
-    klim = it.prob ? Kv[1] : Kv[0];
-    if (!IS_B) op.init(g.A, g.lda, g.a_mn, g.vec_a, it.m0, it.prob ? Mv[1] : Mv[0], it.kb0 * BK, t, 1);
+    if (!IS_B) op.init(g.A, g.lda, g.a_mn, g.vec_a, it.m0, M, it.kb0 * BK, t, 1);
     else op.init(g.B, g.ldb, g.b_mn, g.vec_b, it.n0, g.N, it.kb0 * BK, t, 1);
     i = 0;
     return true;
   };
   bool valid = enter();
-  if (valid) op.load(regs, it.kb0 * BK, klim, t);
+  if (valid) op.load(regs, it.kb0 * BK, K, t);
   uint32_t n = 0;
   while (valid) {
     const uint32_t sidx = n & 1u;
@@ -624,11 +619,11 @@ __device__ __forceinline__ void persistent_producer(const Group& grp, const pg::
     if (lane == 0) mbar_arrive(full0 + 8 * sidx);
     ++n;
     if (++i >= it.nkb) valid = enter();
-    if (valid) op.load(regs, (it.kb0 + i) * BK, klim, t);
+    if (valid) op.load(regs, (it.kb0 + i) * BK, K, t);
   }
 }
 
-__global__ void __launch_bounds__(kPersistThreads, 1) gemm_3xtf32_persistent_kernel(const __grid_constant__ Group grp, int nprob, int ovh) {
+__global__ void __launch_bounds__(kPersistThreads, 1) gemm_3xtf32_persistent_kernel(const __grid_constant__ Args g) {
   constexpr int BN = 256;
   constexpr int A_TILE = BM * BK * 4, B_TILE = BN * BK * 4;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -653,45 +648,34 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_3xtf32_persistent_ker
   tc_fence_after();
   const uint32_t tmem_base = tmem_base_slot;
   const uint32_t smem_base = smem_u32(smem);
-  int Mv[2], Kv[2];
-  const bool early = grp.g[0].early != 0;
-#pragma unroll
-  for (int k = 0; k < 2; ++k) {
-    Mv[k] = grp.g[k].M; Kv[k] = grp.g[k].K;
-    if (early) { if (grp.g[k].m_dev) Mv[k] = __ldcg(grp.g[k].m_dev); if (grp.g[k].k_dev) Kv[k] = __ldcg(grp.g[k].k_dev); }
-  }
+  int Mv[2] = {g.M, 0}, Kv[2] = {g.K, 0};
+  if (g.early) { if (g.m_dev) Mv[0] = __ldcg(g.m_dev); if (g.k_dev) Kv[0] = __ldcg(g.k_dev); }
   pdl_sync();
   if (warp == 0) TRACE(0);
-  if (!early) {
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      if (grp.g[k].m_dev) Mv[k] = __ldcg(grp.g[k].m_dev);
-      if (grp.g[k].k_dev) Kv[k] = __ldcg(grp.g[k].k_dev);
-    }
-  }
+  if (!g.early) { if (g.m_dev) Mv[0] = __ldcg(g.m_dev); if (g.k_dev) Kv[0] = __ldcg(g.k_dev); }
+  const int M = Mv[0], K = Kv[0];
   pg::SchedIn sin;
-  sin.nprob = nprob; sin.ovh = ovh;
-  sin.red[0] = grp.g[0].accumulate; sin.red[1] = grp.g[1].accumulate; sin.N[0] = grp.g[0].N; sin.N[1] = grp.g[1].N;
+  sin.nprob = 1; sin.ovh = 0;   // one store problem: no split-K items to balance against
+  sin.red[0] = sin.red[1] = 0; sin.N[0] = sin.N[1] = g.N;
   const pg::Sched sch = pg::make_sched<1>(sin, Mv, Kv);
 
   if (warp < kPersistProducerWarps) {
     // ---------------------------------------------------------------- producers
-    if (warp < kPersistProducerWarps / 2) persistent_producer<BM, false>(grp, sch, Mv, Kv, smem_base, full0, empty0, 0u);
-    else persistent_producer<BN, true>(grp, sch, Mv, Kv, smem_base, full0, empty0, 2u * A_TILE);
+    if (warp < kPersistProducerWarps / 2) persistent_producer<BM, false>(g, sch, M, K, smem_base, full0, empty0, 0u);
+    else persistent_producer<BN, true>(g, sch, M, K, smem_base, full0, empty0, 2u * A_TILE);
   } else if (warp == kMmaWarp) {
     // ---------------------------------------------------------------- MMA issuer
+    const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)g.a_mn << 15) | ((uint32_t)g.b_mn << 16) |
+                           ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
+    const uint32_t a_lbo = g.a_mn ? 512u : 16u, a_sbo = g.a_mn ? (uint32_t)(BM / 32 * 512) : 1024u;
+    const uint32_t b_lbo = g.b_mn ? 512u : 16u, b_sbo = g.b_mn ? (uint32_t)(BN / 32 * 512) : 1024u;
+    const uint32_t a_kstep = g.a_mn ? (uint32_t)(BM / 32 * 1024) : 32u;
+    const uint32_t b_kstep = g.b_mn ? (uint32_t)(BN / 32 * 1024) : 32u;
+    const uint32_t a_lt = g.a_mn ? 1u : 2u, b_lt = g.b_mn ? 1u : 2u;
     pg::Cursor cur{0, sch.u0};
     pg::Item it;
     uint32_t n = 0, tcount = 0;
     while (pg::next_item<1>(sch, cur, it)) {
-      const int a_mn = it.prob ? grp.g[1].a_mn : grp.g[0].a_mn, b_mn = it.prob ? grp.g[1].b_mn : grp.g[0].b_mn;
-      const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) |
-                             ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
-      const uint32_t a_lbo = a_mn ? 512u : 16u, a_sbo = a_mn ? (uint32_t)(BM / 32 * 512) : 1024u;
-      const uint32_t b_lbo = b_mn ? 512u : 16u, b_sbo = b_mn ? (uint32_t)(BN / 32 * 512) : 1024u;
-      const uint32_t a_kstep = a_mn ? (uint32_t)(BM / 32 * 1024) : 32u;
-      const uint32_t b_kstep = b_mn ? (uint32_t)(BN / 32 * 1024) : 32u;
-      const uint32_t a_lt = a_mn ? 1u : 2u, b_lt = b_mn ? 1u : 2u;
       const uint32_t b = tcount & 1u;
       if (tcount < 8) TRACE(16 + tcount * 8 + 0);
       mbar_wait(acce0 + 8 * b, ((tcount >> 1) & 1u) ^ 1u);  // accumulator b drained by the epilogue warps
@@ -733,26 +717,20 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_3xtf32_persistent_ker
     cx.stats = smem_base + kPersistOffStats;
     cx.e = e; cx.lane = lane; cx.et = threadIdx.x - kPersistProducerWarps * 32;
     cx.release_remote = false;
+    cx.bn_acc = g.bn.acc;
+    cx.bn_H = g.bn.H;
+    cx.M = M;
+    cx.ldc = g.ldc;
+    cx.floor = g.relu ? 0.f : -INFINITY;
     pg::Cursor cur{0, sch.u0};
     pg::Item it;
     uint32_t tcount = 0;
     while (pg::next_item<1>(sch, cur, it)) {
-      const bool p1 = it.prob != 0;
-      const float* const row_scale = p1 ? grp.g[1].row_scale : grp.g[0].row_scale;
-      const float* const bias = p1 ? grp.g[1].bias : grp.g[0].bias;
-      const bool relu = (p1 ? grp.g[1].relu : grp.g[0].relu) != 0, red = (p1 ? grp.g[1].accumulate : grp.g[0].accumulate) != 0;
-      cx.bn_acc = p1 ? grp.g[1].bn.acc : grp.g[0].bn.acc;
-      cx.bn_H = p1 ? grp.g[1].bn.H : grp.g[0].bn.H;
-      const int ldc = p1 ? grp.g[1].ldc : grp.g[0].ldc;
-      const int M = p1 ? Mv[1] : Mv[0];
       const uint32_t b = tcount & 1u;
       cx.m_q0 = it.m0 + q * 32;
-      cx.M = M;
       cx.n0 = it.n0;
-      cx.ldc = ldc;
-      cx.Cq = (p1 ? grp.g[1].C : grp.g[0].C) + (int64_t)cx.m_q0 * ldc + it.n0;
-      cx.bias = (bias && (!red || it.kb0 == 0)) ? bias + it.n0 : nullptr;
-      cx.floor = relu ? 0.f : -INFINITY;
+      cx.Cq = g.C + (int64_t)cx.m_q0 * g.ldc + it.n0;
+      cx.bias = g.bias ? g.bias + it.n0 : nullptr;
       cx.taddr = tmem_base + ((uint32_t)(q * 32) << 16) + b * BN;
       cx.release_bar = acce0 + 8 * b;
       if (tcount < 8 && q == 0) TRACE(16 + tcount * 8 + 4);
@@ -760,11 +738,9 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_3xtf32_persistent_ker
       tc_fence_after();
       if (tcount < 8 && q == 0) TRACE(16 + tcount * 8 + 5);
       const int m = cx.m_q0 + lane;
-      cx.rs = (row_scale && m < M) ? __ldg(row_scale + m) : 1.f;
+      cx.rs = (g.row_scale && m < M) ? __ldg(g.row_scale + m) : 1.f;
       const bool full = cx.m_q0 + 32 <= M;
-      if (red) {
-        if (full) pg::epilogue_tile<true, false, true, false, 4>(cx); else pg::epilogue_tile<true, false, false, false, 4>(cx);
-      } else if (cx.bn_acc) {
+      if (cx.bn_acc) {
         if (full) pg::epilogue_tile<false, true, true, false, 4>(cx); else pg::epilogue_tile<false, true, false, false, 4>(cx);
       } else {
         if (full) pg::epilogue_tile<false, false, true, false, 4>(cx); else pg::epilogue_tile<false, false, false, false, 4>(cx);
@@ -778,11 +754,8 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_3xtf32_persistent_ker
     tc_fence_after();
     tmem_dealloc(tmem_base, 512);
   }
-  for (int k = 0; k < nprob; ++k) {
-    if (grp.g[k].bn.acc) {  // uniform over the grid: every CTA takes a ticket, the last one finalises the statistics
-      if (last_block_ticket(grp.g[k].bn.ticket, gridDim.x)) bn_finalize(grp.g[k].bn, Mv[k]);
-    }
-  }
+  // uniform over the grid: every CTA takes a ticket, the last one finalises the statistics
+  if (g.bn.acc && last_block_ticket(g.bn.ticket, gridDim.x)) bn_finalize(g.bn, M);
 }
 
 }  // namespace tc
@@ -810,12 +783,7 @@ int configure(tc::Args& g, int accumulate, int budget, bool* wide_out, bool* nee
   const int BN = wide ? 256 : 128;
   const int mt = (g.M + BM - 1) / BM, nt = (g.N + BN - 1) / BN;
   const int kblocks = (g.K + BK - 1) / BK;
-  static int min_kb = 0;  // fewest k-blocks a split-K slice may get (tuning knob)
-  if (!min_kb) {
-    const char* e = getenv("EIMS_SPLITK_MIN_KB");
-    min_kb = e ? atoi(e) : 2;
-    if (min_kb < 1) min_kb = 1;
-  }
+  constexpr int min_kb = 2;  // fewest k-blocks a split-K slice may get
   int splits = 1;
   g.accumulate = accumulate;
   *need_memset = false;
@@ -858,33 +826,20 @@ int set_attrs() {
   return 0;
 }
 
-// The persistent kernel takes (a) a single store problem with >= 4 tiles of 128 x 256 per SM and (b) the grouped
-// launch of one store problem + one split-K problem (data gradient + weight gradient of a GraphConv layer), whatever
-// its size: full 256-wide column tiles, vector stores, K <= 512 per store item (single accumulator).
-// EIMS_GEMM_PERSISTENT=0: one CTA per tile everywhere (A/B timing).
-bool use_persistent(const tc::Group& grp, int nprob, bool wide) {
+// The persistent kernel takes a single store problem with >= 4 tiles of 128 x 256 per SM: full 256-wide column tiles,
+// vector stores, K <= 512 (single accumulator).  The grouped data-gradient + weight-gradient launch of a GraphConv layer
+// stays with one CTA per tile: in this kernel it measured 44.9 us against 40.0 us at BASELINE cfg 2 (B200, stage
+// timing), because four epilogue warps share the issue slots with sixteen producer warps that spend ~500 instructions
+// per k-block on the hi / lo split.  The planes kernel (gemm_tma.cu), whose producer is one lane driving the copy
+// engine, does not have that problem.
+bool use_persistent(const tc::Args& g, bool wide) {
   using namespace tc;
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("EIMS_GEMM_PERSISTENT"); on = (e && e[0] == '0') ? 0 : 1; }
-  if (!on || !wide) return false;
-  int reds = 0;
-  for (int k = 0; k < nprob; ++k) {
-    const Args& g = grp.g[k];
-    if ((g.N % 256) || (g.ldc & 3) || (reinterpret_cast<uintptr_t>(g.C) & 15)) return false;
-    if (g.bias && (reinterpret_cast<uintptr_t>(g.bias) & 15)) return false;
-    if (g.accumulate) { ++reds; if (g.bn.acc) return false; }
-    else if ((g.K + BK - 1) / BK > pg::kMaxKbPerItem) return false;   // upper bound when K lives on the device (capacity)
-    if ((int64_t)g.mt * g.nt * ((g.K + BK - 1) / BK) * 148 > (int64_t)1 << 30) return false;  // 32-bit schedule arithmetic
-  }
-  // (b) is OFF by default.  Measured at BASELINE cfg 2 (B200, stage timing): 44.9 us per grouped launch against 40.0 us
-  // for one CTA per tile in two waves.  The overlap does work - but four epilogue warps share the issue slots with
-  // sixteen producer warps that spend ~500 instructions per k-block on the hi / lo split, and the epilogue (17-20 k
-  // cycles per tile under that load, 5 k alone) becomes the period of the pipeline.  The planes kernel (gemm_tma.cu),
-  // whose producer is one lane driving the copy engine, does not have that problem.  EIMS_GEMM_PERSIST_PAIR=1 for A/B.
-  static int pair_on = -1;
-  if (pair_on < 0) { const char* e = getenv("EIMS_GEMM_PERSIST_PAIR"); pair_on = (e && e[0] == '1') ? 1 : 0; }
-  if (nprob == 2) return pair_on && reds == 1;
-  return reds == 0 && grp.g[0].mt * grp.g[0].nt >= 4 * 148;
+  if (!wide || g.accumulate) return false;
+  if ((g.N % 256) || (g.ldc & 3) || (reinterpret_cast<uintptr_t>(g.C) & 15)) return false;
+  if (g.bias && (reinterpret_cast<uintptr_t>(g.bias) & 15)) return false;
+  if ((g.K + BK - 1) / BK > pg::kMaxKbPerItem) return false;   // upper bound when K lives on the device (capacity)
+  if ((int64_t)g.mt * g.nt * ((g.K + BK - 1) / BK) * 148 > (int64_t)1 << 30) return false;  // 32-bit schedule arithmetic
+  return g.mt * g.nt >= 4 * 148;
 }
 
 int launch_group(const tc::Group& grp_in, int ctas, bool wide, cudaStream_t st, int nprob) {
@@ -892,13 +847,8 @@ int launch_group(const tc::Group& grp_in, int ctas, bool wide, cudaStream_t st, 
   const int BN = wide ? 256 : 128, stages = wide ? 2 : 3;
   const int smem_bytes = stages * (2 * BM * BK * 4 + 2 * BN * BK * 4) + 1024;
   cudaError_t e;
-  if (use_persistent(grp_in, nprob, wide)) {
-    static int ovh = -1;
-    if (ovh < 0) { const char* v = getenv("EIMS_GEMM_PERSIST_OVH"); ovh = v ? atoi(v) : 4; if (ovh < 0) ovh = 0; }
-    int64_t items = 0;
-    for (int k = 0; k < nprob; ++k) items += grp_in.g[k].accumulate ? 148 : (int64_t)grp_in.g[k].mt * grp_in.g[k].nt;
-    const int grid = items < 148 ? (int)items : 148;
-    e = launch_pdl(gemm_3xtf32_persistent_kernel, dim3(grid < 1 ? 1 : grid), dim3(kPersistThreads), kPersistSmem, st, grp_in, nprob, ovh);
+  if (nprob == 1 && use_persistent(grp_in.g[0], wide)) {
+    e = launch_pdl(gemm_3xtf32_persistent_kernel, dim3(148), dim3(kPersistThreads), kPersistSmem, st, grp_in.g[0]);
   } else {
     e = wide ? launch_pdl(gemm_3xtf32_kernel<256, 2>, dim3(ctas), dim3(kThreads), smem_bytes, st, grp_in)
              : launch_pdl(gemm_3xtf32_kernel<128, 3>, dim3(ctas), dim3(kThreads), smem_bytes, st, grp_in);

@@ -11,8 +11,8 @@
 //     K-major operand  (memory [mn][k]):  box {32 k, ROWS mn, 2}  CU_TENSOR_MAP_SWIZZLE_128B            -> SWIZZLE_128B
 //     MN-major operand (memory [k][mn]):  box {32 mn, 32 k, 2}    CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B   -> SWIZZLE_128B_BASE32B
 //                                         (one box per 32-wide mn atom, hi and lo of an atom adjacent: LBO = 8 KB)
-// One CTA per SM (192 threads): warp 0 = copy-engine producer (one lane), warp 1 = MMA issuer (one lane, owns TMEM),
-// warps 2-5 = epilogue.  The CTA walks over a list of work items - output tiles of a "store" problem (forward / data
+// A CTA pair per two SMs (192 threads each): warp 0 = copy-engine producer (one lane), warp 1 = MMA issuer (one lane of
+// the leader CTA, owns TMEM), warps 2-5 = epilogue.  The pair walks over a list of work items - output tiles of a "store" problem (forward / data
 // gradient: 128 x 256 tile, whole K) and k-slices of a "split-K" problem (weight gradient over the atoms: red.global.add)
 // - with two 256-column accumulators in TMEM, so the epilogue of item i (TMEM -> registers -> padded shared patch ->
 // 128-byte row segments) runs under the main loop of item i+1 and uses nothing the main loop needs.  The items of a
@@ -20,7 +20,6 @@
 // of the split-K problem in contiguous ranges sized so that every CTA ends at the same time.
 #include <cuda.h>
 
-#include <cstdlib>
 #include <cstring>
 
 #include "common.cuh"
@@ -47,23 +46,22 @@ __device__ unsigned long long g_ptrace[kTraceCtas * kTraceSlots];
 using namespace pg;   // tile constants, work-item schedule and tile epilogue shared with gemm_tc.cu (gemm_persist.cuh)
 constexpr int kThreads = (2 + kEpiWarps) * 32;
 constexpr int kMaxKbDeep = 64;                                     // "deep" launches (main + correction accumulator): K <= 2048
-// PAIR = 1: one CTA per 128 x 256 tile.  PAIR = 2: a CTA pair (cluster of two SMs) works on a 256 x 256 tile with
-// tcgen05.mma.cta_group::2 - each CTA stages its own 128 rows of A and HALF of B (128 of the 256 columns), the tensor
-// cores of both SMs read both halves: per CTA and k-block 64 KB instead of 96 KB enter shared memory and 96 KB instead
-// of 144 KB are read back by the MMAs, which takes the main loop from shared-memory-bandwidth-bound (240 KB / 128 B per
-// clock = 1.9 k cycles per k-block, measured) to MMA-issue-bound (1.54 k), and the smaller stage buys a third stage.
-template <int PAIR>
-struct Cfg {
-  static constexpr int STAGES = PAIR == 2 ? 3 : 2;
-  static constexpr int B_ROWS = BN / PAIR;
-  static constexpr int A_PLANE = BM * BK * 4, B_PLANE = B_ROWS * BK * 4;   // 16 KB; 32 / 16 KB
-  static constexpr int STAGE_BYTES = 2 * A_PLANE + 2 * B_PLANE;            // A hi, A lo, B hi, B lo: 96 / 64 KB
-  static constexpr int OFF_PATCH = STAGES * STAGE_BYTES;
-  static constexpr int OFF_STATS = OFF_PATCH + kEpiWarps * kPatchFloats * 4;
-  static constexpr int OFF_BARS = OFF_STATS + kEpiWarps * 2 * kStatCols * 8;
-  static constexpr int OFF_MISC = OFF_BARS + 16 * 8;                      // full[S], empty[S], acc_full[2], acc_empty[2]
-  static constexpr int kSmemBytes = OFF_MISC + 64 + 1024;                 // + slack for the 1024-byte round-up of the base
-};
+// A CTA pair (cluster of two SMs) works on a 256 x 256 tile with tcgen05.mma.cta_group::2 - each CTA stages its own
+// 128 rows of A and HALF of B (128 of the 256 columns), the tensor cores of both SMs read both halves: per CTA and
+// k-block 64 KB instead of 96 KB enter shared memory and 96 KB instead of 144 KB are read back by the MMAs, which takes
+// the main loop from shared-memory-bandwidth-bound (240 KB / 128 B per clock = 1.9 k cycles per k-block, measured with
+// one CTA per 128 x 256 tile) to MMA-issue-bound (1.54 k), and the smaller stage buys a third stage.
+constexpr int PAIR = 2;
+constexpr int STAGES = 3;
+constexpr int B_ROWS = BN / PAIR;
+static_assert(B_ROWS == kTmaBRows, "the B maps are encoded with a box of kTmaBRows rows");
+constexpr int A_PLANE = BM * BK * 4, B_PLANE = B_ROWS * BK * 4;   // 16 KB each
+constexpr int STAGE_BYTES = 2 * A_PLANE + 2 * B_PLANE;            // A hi, A lo, B hi, B lo: 64 KB
+constexpr int OFF_PATCH = STAGES * STAGE_BYTES;
+constexpr int OFF_STATS = OFF_PATCH + kEpiWarps * kPatchFloats * 4;
+constexpr int OFF_BARS = OFF_STATS + kEpiWarps * 2 * kStatCols * 8;
+constexpr int OFF_MISC = OFF_BARS + 16 * 8;                      // full[S], empty[S], acc_full[2], acc_empty[2]
+constexpr int kSmemBytes = OFF_MISC + 64 + 1024;                 // + slack for the 1024-byte round-up of the base
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
@@ -92,44 +90,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tmem_alloc(uint32_t dst_smem, uint32_t cols) {
-  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(dst_smem), "r"(cols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
-  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-__device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(acc)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr)
-      : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-// 3-D tiled tensor-map load: coordinates innermost first; completion in bytes on the mbarrier
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const void* map, int c0, int c1, int c2, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-      ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(bar)
-      : "memory");
-}
 __device__ __forceinline__ void tma_prefetch_desc(const void* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
 }
@@ -165,7 +125,7 @@ struct Group {
   int deep;
 };
 
-// ---- CTA-pair plumbing (PAIR = 2)
+// ---- CTA-pair plumbing
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -179,7 +139,8 @@ __device__ __forceinline__ uint32_t mapa_rank(uint32_t addr, uint32_t rank) {   
 __device__ __forceinline__ void cluster_sync_all() {
   asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
-// the same load issued by either CTA of a pair: completion bytes go to the LEADER's mbarrier (shared::cluster address)
+// 3-D tiled tensor-map load (coordinates innermost first), issued by either CTA of a pair: completion bytes go to the
+// LEADER's mbarrier (shared::cluster address)
 __device__ __forceinline__ void tma_load_3d_pair(uint32_t dst, const void* map, int c0, int c1, int c2, uint32_t leader_bar) {
   asm volatile(
       "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
@@ -207,17 +168,15 @@ __device__ __forceinline__ void umma_commit_pair(uint32_t bar) {   // arrives on
                ::"r"(bar), "h"(mask) : "memory");
 }
 
-template <int PAIR>
 __global__ void __launch_bounds__(kThreads, 1) gemm_planes_kernel(const __grid_constant__ Group grp) {
-  using C = Cfg<PAIR>;
-  constexpr int S = C::STAGES;
+  constexpr int S = STAGES;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + C::OFF_BARS);   // full[S], empty[S], acc_full[2], acc_empty[2]
-  uint32_t* misc = reinterpret_cast<uint32_t*>(smem + C::OFF_MISC);   // [0] TMEM base
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + OFF_BARS);   // full[S], empty[S], acc_full[2], acc_empty[2]
+  uint32_t* misc = reinterpret_cast<uint32_t*>(smem + OFF_MISC);   // [0] TMEM base
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (warp == 0) PTRACE(0);
-  const uint32_t rank = PAIR == 2 ? cluster_ctarank() : 0u;           // rank 0 of a pair issues the MMAs
+  const uint32_t rank = cluster_ctarank();                            // rank 0 of a pair issues the MMAs
   const uint32_t full0 = smem_u32(&bars[0]), empty0 = smem_u32(&bars[S]), accf0 = smem_u32(&bars[2 * S]), acce0 = smem_u32(&bars[2 * S + 2]);
   if (threadIdx.x == 0) {
     for (int s = 0; s < S; ++s) {
@@ -231,13 +190,10 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_planes_kernel(const __grid_c
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     for (int k = 0; k < grp.nprob; ++k) { tma_prefetch_desc(&grp.g[k].ta); tma_prefetch_desc(&grp.g[k].tb); }
   }
-  if (warp == 1) {
-    if (PAIR == 2) tmem_alloc_pair(smem_u32(&misc[0]), 512);
-    else tmem_alloc(smem_u32(&misc[0]), 512);
-  }
+  if (warp == 1) tmem_alloc_pair(smem_u32(&misc[0]), 512);
   tc_fence_before();
   __syncthreads();
-  if (PAIR == 2) cluster_sync_all();   // the peer's barriers are initialised before anything remote touches them
+  cluster_sync_all();   // the peer's barriers are initialised before anything remote touches them
   tc_fence_after();
   const uint32_t tmem_base = misc[0];
   const uint32_t smem_base = smem_u32(smem);
@@ -280,34 +236,28 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_planes_kernel(const __grid_c
         const void* const map_a = pi ? (const void*)&grp.g[1].ta : (const void*)&grp.g[0].ta;
         const void* const map_b = pi ? (const void*)&grp.g[1].tb : (const void*)&grp.g[0].tb;
         const int a_mn = pi ? grp.g[1].a_mn : grp.g[0].a_mn, b_mn = pi ? grp.g[1].b_mn : grp.g[0].b_mn;
-        const int m_own = it.m0 + (int)rank * BM, n_own = it.n0 + (int)rank * C::B_ROWS;
+        const int m_own = it.m0 + (int)rank * BM, n_own = it.n0 + (int)rank * B_ROWS;
         PTRACE(8 + tcount * 8 + 0);   // first copy of the item about to be issued
         ++tcount;
         for (int i = 0; i < it.nkb; ++i, ++n) {
           const uint32_t s = n % S;
           mbar_wait(empty0 + 8 * s, ((n / S) & 1u) ^ 1u);
           uint32_t bar = full0 + 8 * s;
-          if (rank == 0) mbar_expect_tx(bar, C::STAGE_BYTES * PAIR);
-          if (PAIR == 2) bar = mapa_rank(bar, 0);
-          const uint32_t sa = smem_base + s * C::STAGE_BYTES, sb = sa + 2 * C::A_PLANE;
+          if (rank == 0) mbar_expect_tx(bar, STAGE_BYTES * PAIR);
+          bar = mapa_rank(bar, 0);
+          const uint32_t sa = smem_base + s * STAGE_BYTES, sb = sa + 2 * A_PLANE;
           const int k0 = (it.kb0 + i) * BK;
           if (!a_mn) {
-            if (PAIR == 2) tma_load_3d_pair(sa, map_a, k0, m_own, 0, bar); else tma_load_3d(sa, map_a, k0, m_own, 0, bar);
+            tma_load_3d_pair(sa, map_a, k0, m_own, 0, bar);
           } else {
 #pragma unroll
-            for (int j = 0; j < BM / 32; ++j) {
-              if (PAIR == 2) tma_load_3d_pair(sa + j * 8192, map_a, m_own + 32 * j, k0, 0, bar);
-              else tma_load_3d(sa + j * 8192, map_a, m_own + 32 * j, k0, 0, bar);
-            }
+            for (int j = 0; j < BM / 32; ++j) tma_load_3d_pair(sa + j * 8192, map_a, m_own + 32 * j, k0, 0, bar);
           }
           if (!b_mn) {
-            if (PAIR == 2) tma_load_3d_pair(sb, map_b, k0, n_own, 0, bar); else tma_load_3d(sb, map_b, k0, n_own, 0, bar);
+            tma_load_3d_pair(sb, map_b, k0, n_own, 0, bar);
           } else {
 #pragma unroll
-            for (int j = 0; j < C::B_ROWS / 32; ++j) {
-              if (PAIR == 2) tma_load_3d_pair(sb + j * 8192, map_b, n_own + 32 * j, k0, 0, bar);
-              else tma_load_3d(sb + j * 8192, map_b, n_own + 32 * j, k0, 0, bar);
-            }
+            for (int j = 0; j < B_ROWS / 32; ++j) tma_load_3d_pair(sb + j * 8192, map_b, n_own + 32 * j, k0, 0, bar);
           }
         }
       }
@@ -327,7 +277,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_planes_kernel(const __grid_c
         //           SBO = 512 (next 4 k-rows), k-step (8 k-rows) = +1024 B, lo = hi + 4096.
         const uint32_t a_lbo = a_mn ? 8192u : 16u, a_sbo = a_mn ? 512u : 1024u, a_kstep = a_mn ? 1024u : 32u;
         const uint32_t b_lbo = b_mn ? 8192u : 16u, b_sbo = b_mn ? 512u : 1024u, b_kstep = b_mn ? 1024u : 32u;
-        const uint32_t a_lo_off = a_mn ? 4096u : (uint32_t)C::A_PLANE, b_lo_off = b_mn ? 4096u : (uint32_t)C::B_PLANE;
+        const uint32_t a_lo_off = a_mn ? 4096u : (uint32_t)A_PLANE, b_lo_off = b_mn ? 4096u : (uint32_t)B_PLANE;
         const uint32_t a_lt = a_mn ? 1u : 2u, b_lt = b_mn ? 1u : 2u;
         const uint32_t b = grp.deep ? 0u : (tcount & 1u);
         const uint32_t bph = grp.deep ? (tcount & 1u) : ((tcount >> 1) & 1u);
@@ -343,7 +293,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_planes_kernel(const __grid_c
           if (i == 0) PTRACE(8 + tcount * 8 + 2);              // first k-block landed
           if (i == it.nkb - 1) PTRACE(8 + tcount * 8 + 3);     // last k-block landed
           if (lane == 0) {
-            const uint32_t sa = smem_base + s * C::STAGE_BYTES, sb = sa + 2 * C::A_PLANE;
+            const uint32_t sa = smem_base + s * STAGE_BYTES, sb = sa + 2 * A_PLANE;
 #pragma unroll
             for (int ks = 0; ks < BK / 8; ++ks) {
               const uint64_t dah = make_desc(sa + ks * a_kstep, a_lbo, a_sbo, a_lt);
@@ -352,23 +302,12 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_planes_kernel(const __grid_c
               const uint64_t dbl = make_desc(sb + b_lo_off + ks * b_kstep, b_lbo, b_sbo, b_lt);
               const uint32_t first = (i > 0 || ks > 0) ? 1u : 0u;
               const uint32_t mfirst = grp.deep ? first : 1u;   // deep: the main accumulator starts with this product
-              if (PAIR == 2) {
-                umma_tf32_pair(acc_corr, dal, dbh, idesc, first);  // smallest terms first
-                umma_tf32_pair(acc_corr, dah, dbl, idesc, 1u);
-                umma_tf32_pair(acc, dah, dbh, idesc, mfirst);
-              } else {
-                umma_tf32(acc_corr, dal, dbh, idesc, first);
-                umma_tf32(acc_corr, dah, dbl, idesc, 1u);
-                umma_tf32(acc, dah, dbh, idesc, mfirst);
-              }
+              umma_tf32_pair(acc_corr, dal, dbh, idesc, first);  // smallest terms first
+              umma_tf32_pair(acc_corr, dah, dbl, idesc, 1u);
+              umma_tf32_pair(acc, dah, dbh, idesc, mfirst);
             }
-            if (PAIR == 2) {
-              umma_commit_pair(empty0 + 8 * s);                        // frees the stage in both CTAs when these MMAs retire
-              if (i == it.nkb - 1) umma_commit_pair(accf0 + 8 * b);    // accumulator b complete (both halves)
-            } else {
-              umma_commit(empty0 + 8 * s);
-              if (i == it.nkb - 1) umma_commit(accf0 + 8 * b);
-            }
+            umma_commit_pair(empty0 + 8 * s);                        // frees the stage in both CTAs when these MMAs retire
+            if (i == it.nkb - 1) umma_commit_pair(accf0 + 8 * b);    // accumulator b complete (both halves)
           }
           __syncwarp();
         }
@@ -380,8 +319,8 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_planes_kernel(const __grid_c
     // ---------------------------------------------------------------- epilogue warps (each CTA drains its own 128 rows)
     const int e = warp - 2, q = warp & 3;  // q: the TMEM lane quarter this warp may read
     EpiCtx cx;
-    cx.patch = smem_base + C::OFF_PATCH + e * kPatchFloats * 4;   // shared-space byte addresses
-    cx.stats = smem_base + C::OFF_STATS;                          // double [kEpiWarps][2][kStatCols]
+    cx.patch = smem_base + OFF_PATCH + e * kPatchFloats * 4;   // shared-space byte addresses
+    cx.stats = smem_base + OFF_STATS;                             // double [kEpiWarps][2][kStatCols]
     cx.e = e; cx.lane = lane; cx.et = threadIdx.x - 64;
     Cursor cur{0, sch.u0};
     Item it;
@@ -408,8 +347,8 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_planes_kernel(const __grid_c
       cx.floor = relu ? 0.f : -INFINITY;
       cx.taddr = tmem_base + ((uint32_t)(q * 32) << 16) + b * BN;
       // what hands accumulator b back to the MMA issuer (the leader's barrier also counts the peer's warps)
-      cx.release_bar = (PAIR == 2 && rank != 0) ? mapa_rank(acce0 + 8 * b, 0) : acce0 + 8 * b;
-      cx.release_remote = PAIR == 2 && rank != 0;
+      cx.release_bar = rank != 0 ? mapa_rank(acce0 + 8 * b, 0) : acce0 + 8 * b;
+      cx.release_remote = rank != 0;
       if (e == 0) PTRACE(8 + tcount * 8 + 4);                  // epilogue waits for the accumulator
       mbar_wait(accf0 + 8 * b, bph);
       tc_fence_after();
@@ -434,11 +373,10 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_planes_kernel(const __grid_c
   }
   if (warp == 0) PTRACE(3);
   __syncthreads();
-  if (PAIR == 2) cluster_sync_all();   // nothing remote (barrier arrivals, the peer's MMA reads of this CTA's tiles) is still in flight
+  cluster_sync_all();   // nothing remote (barrier arrivals, the peer's MMA reads of this CTA's tiles) is still in flight
   if (warp == 1) {
     tc_fence_after();
-    if (PAIR == 2) tmem_dealloc_pair(tmem_base, 512);
-    else tmem_dealloc(tmem_base, 512);
+    tmem_dealloc_pair(tmem_base, 512);
   }
   for (int k = 0; k < grp.nprob; ++k) {
     if (grp.g[k].bn.acc) {  // uniform over the grid: every CTA takes a ticket, the last one finalises the statistics
@@ -521,31 +459,7 @@ int tma_make_map(TmaMap* out, const float* planes, int64_t plane_stride, int row
   return 0;
 }
 
-bool gemm_tma_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("EIMS_GEMM_TMA");
-    on = (e && e[0] == '0') ? 0 : 1;
-    if (on && !encode_fn()) on = 0;
-  }
-  return on != 0;
-}
-
-// EIMS_GEMM_TMA=1: the planes path wherever the shapes allow it (unset: the plan picks it for large batches only)
-bool gemm_tma_forced() {
-  static int f = -1;
-  if (f < 0) { const char* e = getenv("EIMS_GEMM_TMA"); f = (e && e[0] != '0') ? 1 : 0; }
-  return f != 0 && gemm_tma_enabled();
-}
-
-// 2 (default): CTA pairs with tcgen05.mma.cta_group::2; EIMS_GEMM_PAIR=1: one CTA per tile.  The B maps of a launch
-// must be encoded for the same mode (box of 256 / pair rows: gemm_tma_b_rows()).
-int gemm_tma_pair() {
-  static int pair = 0;
-  if (!pair) { const char* e = getenv("EIMS_GEMM_PAIR"); pair = (e && e[0] == '1') ? 1 : 2; }
-  return pair;
-}
-int gemm_tma_b_rows() { return tma::BN / gemm_tma_pair(); }
+bool gemm_tma_enabled() { return encode_fn() != nullptr; }
 
 // shapes the planes kernel takes: full 256-wide column tiles, vector stores, K of a store problem <= 2048 (> 512: deep mode)
 bool gemm_tma_supports(const GemmTmaProblem& q) {
@@ -560,16 +474,13 @@ int launch_gemm_tma(const GemmTmaProblem* p0, const GemmTmaProblem* p1, cudaStre
   using namespace tma;
   if (!p0 || !gemm_tma_supports(*p0) || (p1 && !gemm_tma_supports(*p1))) return EIMS_ERR_ARG;
   if (p1 && (p0->red != 0) == (p1->red != 0)) return EIMS_ERR_ARG;  // one store problem and one split-K problem at most
-  const int pair = gemm_tma_pair();
   static bool attr_done = false;
   if (!attr_done) {
-    if (cudaFuncSetAttribute(gemm_planes_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<1>::kSmemBytes) != cudaSuccess ||
-        cudaFuncSetAttribute(gemm_planes_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<2>::kSmemBytes) != cudaSuccess)
+    if (cudaFuncSetAttribute(gemm_planes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes) != cudaSuccess)
       return EIMS_ERR_CUDA;
     attr_done = true;
   }
-  static int ovh = -1;
-  if (ovh < 0) { const char* e = getenv("EIMS_GEMM_TMA_OVH"); ovh = e ? atoi(e) : 4; if (ovh < 0) ovh = 0; }
+  constexpr int kItemOverhead = 4;  // fixed cost of one work item in k-block units (balances the two problems)
   Group grp;
   memset(&grp, 0, sizeof(grp));
   const GemmTmaProblem* ps[2] = {p0, p1};
@@ -583,7 +494,7 @@ int launch_gemm_tma(const GemmTmaProblem* p0, const GemmTmaProblem* p1, cudaStre
     g.M = q->M; g.N = q->N; g.K = q->K; g.m_dev = q->m_dev; g.k_dev = q->k_dev;
     g.row_scale = q->row_scale; g.bias = q->bias; g.relu = q->relu; g.red = q->red;
     if (q->bn) g.bn = *q->bn;
-    if (ps[k]) items += (int64_t)((q->M + BM * pair - 1) / (BM * pair)) * (q->N / BN) * (q->red ? 148 : 1);
+    if (ps[k]) items += (int64_t)((q->M + BM * PAIR - 1) / (BM * PAIR)) * (q->N / BN) * (q->red ? 148 : 1);
     // the device-side schedule works in 32-bit integers (k-block units times CTAs)
     if (ps[k] && (int64_t)((q->M + BM - 1) / BM) * (q->N / BN) * ((q->K + BK - 1) / BK) * 148 >= ((int64_t)1 << 31)) return EIMS_ERR_ARG;
   }
@@ -591,32 +502,25 @@ int launch_gemm_tma(const GemmTmaProblem* p0, const GemmTmaProblem* p1, cudaStre
   for (int k = 0; k < grp.nprob; ++k)
     if (!grp.g[k].red && (grp.g[k].K + 31) / 32 > kMaxKbPerItem) grp.deep = 1;
   grp.early = dims_early_ref();
-  grp.ovh = ovh;
-  const int units = 148 / pair;
-  int grid = (int)(items < units ? items : units) * pair;
-  if (grid < pair) grid = pair;
+  grp.ovh = kItemOverhead;
+  const int units = 148 / PAIR;
+  int grid = (int)(items < units ? items : units) * PAIR;
+  if (grid < PAIR) grid = PAIR;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = pair == 2 ? Cfg<2>::kSmemBytes : Cfg<1>::kSmemBytes;
+  cfg.dynamicSmemBytes = kSmemBytes;
   cfg.stream = st;
   cudaLaunchAttribute attr[2];
-  int na = 0;
-  if (pdl_enabled()) {
-    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[na].val.programmaticStreamSerializationAllowed = 1;
-    ++na;
-  }
-  if (pair == 2) {
-    attr[na].id = cudaLaunchAttributeClusterDimension;
-    attr[na].val.clusterDim.x = 2;
-    attr[na].val.clusterDim.y = 1;
-    attr[na].val.clusterDim.z = 1;
-    ++na;
-  }
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  attr[1].id = cudaLaunchAttributeClusterDimension;
+  attr[1].val.clusterDim.x = PAIR;
+  attr[1].val.clusterDim.y = 1;
+  attr[1].val.clusterDim.z = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = na;
-  cudaError_t e = pair == 2 ? cudaLaunchKernelEx(&cfg, gemm_planes_kernel<2>, grp) : cudaLaunchKernelEx(&cfg, gemm_planes_kernel<1>, grp);
+  cfg.numAttrs = 2;
+  cudaError_t e = cudaLaunchKernelEx(&cfg, gemm_planes_kernel, grp);
   return e == cudaSuccess ? 0 : EIMS_ERR_CUDA;
 }
 

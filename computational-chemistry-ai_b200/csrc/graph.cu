@@ -17,7 +17,7 @@ namespace eims {
 // aggregate a0 = A (x * c) of GraphConv (GCN:359, i = 0), which only needs the molecule itself.
 // dims[DIM_ZERO_DEG] holds the sequence number of the last batch that had an isolated atom and
 // dims[5] the current sequence number (no reset race between blocks).
-constexpr int kK1Warps = 4;  // upper bound (shared-memory arrays); the launch picks 2 or 4 warps per block
+constexpr int kK1Warps = 4;  // upper bound (shared-memory arrays); launch_csr_build uses 2 warps per block
 constexpr int kMaxF0 = 8;
 
 // Large batches (inference, thousands of molecules): the per-block batch reduction of the fused
@@ -312,9 +312,9 @@ int launch_csr_build(const eims_dataset* ds, const int32_t* ids, int B, int F, i
                      int* gptr, int* eptr, int* gid, int* src, int* dst, int* rowptr, int* col, float* norm,
                      float* x, int* dims, cudaStream_t st, float* a0, int seq, const StepBlock* blk, int* bids) {
   if (F > kMaxF0) return EIMS_ERR_ARG;
-  // molecules (warps) per block: 2 gives 256 blocks for a batch of 512, 4 is round 1's shape (EIMS_K1_WARPS for A/B)
-  static int k1w = 0;
-  if (!k1w) { const char* e = getenv("EIMS_K1_WARPS"); k1w = e ? atoi(e) : 2; if (k1w < 1 || k1w > kK1Warps) k1w = 2; }
+  // molecules (warps) per block: 2 gives 256 blocks for a batch of 512, 4 is round 1's shape
+  constexpr int k1w = 2;
+  static_assert(k1w <= kK1Warps, "k1_build_kernel is sized for at most kK1Warps warps");
   const int blocks = B > 0 ? (B + k1w - 1) / k1w : 1;
   const int prescanned = B > 1024;
   if (prescanned)
@@ -403,9 +403,8 @@ int launch_layer0_fwd(const int* dims, const float* norm, const float* a0, int F
   const int slabs = (H + 63) / 64;
   // one wave: the kernel needs 104 registers, so two blocks are resident per SM (measured at cfg 2: 13.7 us with
   // 2 blocks per SM, 16.7-17.5 us with 3 or 4, i.e. a second wave)
-  static int per_sm = 0;
-  if (!per_sm) { const char* e = getenv("EIMS_L0_BLOCKS_PER_SM"); per_sm = e ? atoi(e) : 2; if (per_sm < 1) per_sm = 1; }
-  int rg = (148 * per_sm + slabs - 1) / slabs;
+  constexpr int kBlocksPerSm = 2;
+  int rg = (148 * kBlocksPerSm + slabs - 1) / slabs;
   const int need = (max_nodes + kL0Rows - 1) / kL0Rows;  // a block stages at most kL0Rows rows
   if (rg < need) rg = need;
   if (rg < 1) rg = 1;
@@ -855,13 +854,9 @@ __global__ void __launch_bounds__(THREADS) spmm_mol_kernel(const int* __restrict
 int launch_spmm_mol(const int* dims, const int* gptr, const int* rowptr, const int* col, const float* norm, const float* h,
                            int H, const float* bn_scale, const float* bn_shift, DropCfg drop, int out_mode, float* out,
                            int max_graphs, int tile_rows, cudaStream_t st, const BnBwdFuse* bf, int64_t lo_off) {
-  // Shape: a block owns HC = 128 columns (4 warps) or 256 columns (8 warps) of one molecule at a time.  The narrow
-  // shape keeps the tile at tile_rows x 512 bytes (32 KB at 64 rows), so ~7 blocks are resident per SM and the
-  // (molecules x column chunks) grid of a training batch - 512 x 2 at cfg 2 - fits in ONE wave; with 256-column
-  // blocks the same batch took 1.15 waves of 3 blocks per SM, i.e. twice the time (EIMS_SPMM_MOL_WIDE=1 for A/B).
-  static int wide = -1;
-  if (wide < 0) { const char* e = getenv("EIMS_SPMM_MOL_WIDE"); wide = (e && e[0] == '0') ? 0 : 1; }
-  const int NV = (wide && H % 256 == 0 && (size_t)tile_rows * 256 * 4 <= 64 * 1024) ? 2 : 1;
+  // Shape: a block owns HC = 256 columns (8 warps) of one molecule at a time where H is a multiple of 256 and the
+  // tile_rows x 1 KB tile fits in 64 KB (up to 64 rows), else HC = 128 columns (4 warps).
+  const int NV = (H % 256 == 0 && (size_t)tile_rows * 256 * 4 <= 64 * 1024) ? 2 : 1;
   const int HC = 128 * NV, threads = 128 * NV;
   if (H % HC) return EIMS_ERR_ARG;
   const int cap_edges = 4 * tile_rows + 64;
@@ -891,7 +886,7 @@ int launch_spmm_norm(const int* dims, const int* rowptr, const int* col, const f
                      int max_nodes, cudaStream_t st, const BnBwdFuse* bf, const int* gptr, int max_graphs, int tile_rows,
                      int64_t lo_off) {
   if (H % 4) return EIMS_ERR_ARG;
-  if (bf && out_mode != 1) return EIMS_ERR_ARG;
+  if (bf && (out_mode != 1 || H > 256)) return EIMS_ERR_ARG;  // the statistics form exists up to 256 columns (see plan.cu)
   if (lo_off && (bf || (lo_off & 3))) return EIMS_ERR_ARG;
   // Molecule-tile kernel (neighbour rows staged in shared memory by the bulk-copy engine) when the caller knows the
   // batch's graph offsets AND the batch is large.  Measured on a B200 (profiles/r2_spmm_ab.md): with >= ~8 molecules
@@ -899,35 +894,35 @@ int launch_spmm_norm(const int* dims, const int* rowptr, const int* col, const f
   // vs 59 % of the measured copy bandwidth); at a training batch of 512 molecules a block sees one molecule, its
   // phases (offsets -> bulk copy lands -> transform -> sum) cannot overlap, and the gather kernel - 9.5 k warps with
   // independent rows in flight - is faster (17 vs 18-26 us per launch for three staged variants, software-pipelined
-  // producer/consumer ring included).  EIMS_SPMM_MOL=0 / 1 forces one or the other (A/B timing, tests).
-  static int mol_on = -2;
-  if (mol_on == -2) { const char* e = getenv("EIMS_SPMM_MOL"); mol_on = e ? (e[0] == '0' ? 0 : 1) : -1; }
+  // producer/consumer ring included).
   const bool big_batch = max_graphs >= 2048 && !bf;
-  if ((mol_on == 1 || (mol_on == -1 && big_batch)) && gptr && tile_rows > 0 && H % 128 == 0)
+  if (big_batch && gptr && tile_rows > 0 && H % 128 == 0)
     return launch_spmm_mol(dims, gptr, rowptr, col, norm, h, H, bn_scale, bn_shift, drop, out_mode, out, max_graphs, tile_rows, st, bf, lo_off);
   const int parts = H <= 512 ? 1 : (H + 511) / 512;
   if (parts > 8 || (8 % parts)) return EIMS_ERR_ARG;  // 8 warps per block must split evenly over a row
-  static int per_sm = 0;  // resident blocks per SM the grid is sized for (tuning knob)
-  if (!per_sm) { const char* e = getenv("EIMS_SPMM_BLOCKS_PER_SM"); per_sm = e ? atoi(e) : 8; if (per_sm < 1) per_sm = 1; }
+  constexpr int kBlocksPerSm = 8;  // resident blocks per SM the grid is sized for
   int blocks = (max_nodes * parts + 7) / 8;
-  if (blocks > 148 * per_sm) blocks = 148 * per_sm;
+  if (blocks > 148 * kBlocksPerSm) blocks = 148 * kBlocksPerSm;
   if (blocks < 1) blocks = 1;
-  const BnBwdFuse none{};
   // STATS: one wave of three blocks per SM (77 registers with one neighbour in flight per trip; measured at cfg 2:
   // 20 us with 444 blocks, 25 with 296 or 592)
-  static int sblocks = 0;
-  if (!sblocks) { const char* e = getenv("EIMS_SPMM_STATS_BLOCKS"); sblocks = e ? atoi(e) : 148 * 3; if (sblocks < 1) sblocks = 1; }
-  const int blocks_s = blocks < sblocks ? blocks : sblocks;
+  constexpr int kStatsBlocks = 148 * 3;
+  const int blocks_s = blocks < kStatsBlocks ? blocks : kStatsBlocks;
+#define EIMS_SPMM_STATS(NV)                                                                                            \
+  launch_pdl(spmm_norm_kernel<NV, 1, true>, dim3(blocks_s), dim3(256), (size_t)8 * 2 * 128 * NV * sizeof(float), st, dims, rowptr, \
+             col, norm, h, H, bn_scale, bn_shift, drop, out_mode, out, parts, *bf, dims_early_ref(), (int64_t)0)
 #define EIMS_SPMM(NV, UE)                                                                                              \
-  do {                                                                                                                 \
-    if (bf) launch_pdl(spmm_norm_kernel<NV, 1, true>, dim3(blocks_s), dim3(256), (size_t)8 * 2 * 128 * NV * sizeof(float), st, dims, rowptr, col, norm, \
-                       h, H, bn_scale, bn_shift, drop, out_mode, out, parts, *bf, dims_early_ref(), (int64_t)0);         \
-    else launch_pdl(spmm_norm_kernel<NV, UE, false>, dim3(blocks), dim3(256), 0, st, dims, rowptr, col, norm, h, H, bn_scale,   \
-                    bn_shift, drop, out_mode, out, parts, none, dims_early_ref(), lo_off);                               \
-  } while (0)
-  if (H <= 128) EIMS_SPMM(1, 4);
-  else if (H <= 256) EIMS_SPMM(2, 2);
-  else EIMS_SPMM(4, 1);
+  launch_pdl(spmm_norm_kernel<NV, UE, false>, dim3(blocks), dim3(256), 0, st, dims, rowptr, col, norm, h, H, bn_scale,  \
+             bn_shift, drop, out_mode, out, parts, BnBwdFuse{}, dims_early_ref(), lo_off)
+  if (bf) {
+    if (H <= 128) EIMS_SPMM_STATS(1);
+    else EIMS_SPMM_STATS(2);
+  } else {
+    if (H <= 128) EIMS_SPMM(1, 4);
+    else if (H <= 256) EIMS_SPMM(2, 2);
+    else EIMS_SPMM(4, 1);
+  }
+#undef EIMS_SPMM_STATS
 #undef EIMS_SPMM
   return 0;
 }
@@ -1049,10 +1044,9 @@ int launch_readout(const int* dims, const int* gptr, const float* z, int H, cons
                    const float* bn_mean) {
   if (H % 4 || H < 4 || (zstat && !bn_mean)) return EIMS_ERR_ARG;
   // shared-memory tile for the graph's rows (bulk async copy): 64 KB holds 64 atoms at H = 256; graphs that do not
-  // fit read their rows from global memory as before.  EIMS_READOUT_TILE_KB=0 turns the staging off (A/B timing).
-  static int tile_kb = -1;
-  if (tile_kb < 0) { const char* e = getenv("EIMS_READOUT_TILE_KB"); tile_kb = e ? atoi(e) : 64; if (tile_kb < 0 || tile_kb > 200) tile_kb = 64; }
-  const int tile_bytes = (H * 4) % 16 == 0 ? tile_kb * 1024 : 0;
+  // fit read their rows from global memory
+  constexpr int kTileBytes = 64 * 1024;
+  const int tile_bytes = (H * 4) % 16 == 0 ? kTileBytes : 0;
   static bool attr = false;
   if (!attr) { cudaFuncSetAttribute(readout_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024); attr = true; }
   launch_pdl(readout_kernel, dim3(max_graphs < 1 ? 1 : max_graphs), dim3(256), (size_t)tile_bytes, st, dims, gptr, z, H, bn_scale, bn_shift,

@@ -48,12 +48,8 @@ int launch_bn_stats(const int* dims, const float* z, int H, const float* gamma, 
                     int max_nodes, cudaStream_t st);
 int launch_bn_eval_coeffs(const float* gamma, const float* beta, const float* rmean, const float* rvar, int H,
                           float* scale, float* shift, cudaStream_t st);
-// dh computed on the fly from the layer above (see DhSrc in dense.cu)
-struct GatherSrc { const float* da; const int* rowptr; const int* col; const float* norm; DropCfg drop; };
-int launch_bn_bwd_stats(const int* dims, const float* dh, const float* dG, const int* gid, const int* gptr,
-                        const int* argmax, int pooling, const float* z, int H, const float* mean, const float* invstd,
-                        float* dgamma, float* dbeta, float* means, float* partials, int max_nodes, cudaStream_t st,
-                        const GatherSrc* gs = nullptr);
+int launch_bn_bwd_stats(const int* dims, const float* dh, const float* z, int H, const float* mean, const float* invstd,
+                        float* dgamma, float* dbeta, float* means, float* partials, int max_nodes, cudaStream_t st);
 // statistics of the TOP layer's BatchNorm backward from per-graph quantities (O(B*H) instead of O(N*H))
 int launch_bn_bwd_stats_top(const int* dims, const float* dG, const float* zstat, const int* gptr, int pooling, int H,
                             const float* mean, const float* invstd, float* dgamma, float* dbeta, float* means,
@@ -62,7 +58,7 @@ int launch_bn_bwd_apply(const int* dims, const float* dh, const float* dG, const
                         const int* argmax, int pooling, const float* z, int H, const float* mean, const float* invstd,
                         const float* gamma, const float* norm, float* dbias, const float* means, float* q, int max_nodes,
                         cudaStream_t st, const float* a0 = nullptr, int F = 0, float* dW0 = nullptr,
-                        const GatherSrc* gs = nullptr, int64_t q_lo_off = 0);  // != 0: q as stacked tf32 hi / lo planes
+                        int64_t q_lo_off = 0);  // != 0: q as stacked tf32 hi / lo planes
 int launch_ln_fwd(const int* dims, const float* u, int W, const float* gamma, const float* beta, DropCfg drop, float* y,
                   float* stats, int max_graphs, cudaStream_t st);
 int launch_ln_bwd(const int* dims, const float* u, const float* y, const float* dy, int W, const float* gamma,
@@ -100,10 +96,8 @@ struct alignas(64) TmaMap { uint8_t bytes[128]; };  // a CUtensorMap (driver typ
 // map over the stacked planes [2][rows][ld] (plane_stride floats apart) of a row-major operand with `cols` columns:
 // mn_major = 0 -> the rows are the operand's M / N index (box_rows of them per tile), 1 -> the rows are its K index
 int tma_make_map(TmaMap* out, const float* planes, int64_t plane_stride, int rows, int cols, int ld, int box_rows, int mn_major);
-bool gemm_tma_enabled();  // EIMS_GEMM_TMA=0 turns the planes path off (A/B timing)
-bool gemm_tma_forced();   // EIMS_GEMM_TMA=1: use it wherever the shapes allow (default: large batches only, see plan.cu)
-int gemm_tma_pair();      // 2: CTA pairs (tcgen05.mma.cta_group::2), 1: one CTA per tile (EIMS_GEMM_PAIR=1)
-int gemm_tma_b_rows();    // box rows of a K-major B map for that mode (256 / pair)
+bool gemm_tma_enabled();  // the driver offers cuTensorMapEncodeTiled
+constexpr int kTmaBRows = 128;  // box rows of a K-major B map: each CTA of a pair stages half of a 256-column tile
 struct GemmTmaProblem {
   const TmaMap* ta; const TmaMap* tb; float* C; int ldc, a_mn, b_mn, M, N, K;
   const int* m_dev; const int* k_dev; const float* row_scale; const float* bias; int relu, red; const BnFuse* bn;

@@ -85,10 +85,10 @@ struct eims_plan {
   int last_training;
   // per-stage CUDA-event profiling (bench.py's roofline pass) and launch accounting
   eims_peaks peak_targets{};  // targets as peak lists (eims_plan_set_peak_targets); peak_ptr == NULL: unset
-  bool pair_gemms = true;     // wgrad + dgrad of a layer share one launch (EIMS_PAIR_GEMMS=0: two launches)
-  bool top_stats_per_graph = true;  // BatchNorm-backward statistics of the top layer from per-graph quantities (EIMS_TOP_STATS_PER_GRAPH=0: node pass)
-  bool fuse_bn_bwd_stats = true;  // BatchNorm-backward statistics come out of the SpMM that writes dh (EIMS_FUSE_BN_BWD_STATS=0: own pass)
-  bool fuse_spmm_bwd = false;  // measured slower at cfg 2 (0.405 vs 0.386 ms/step): the slab-layout gather costs more than K2 saves
+  // BatchNorm-backward statistics of the layers below the top come out of the SpMM that writes their dh.  Beyond 256
+  // columns the statistics variant of K2 needs 172 registers - one block per SM - and measured slower than K2 plus the
+  // separate statistics pass: cfg 5, 0.99 + 0.02 ms against 0.38 + 0.43 ms per step.
+  bool fuse_bn_bwd_stats = false;
   int batch_seq = 0;  // K1 sequence number (tags the zero-degree flag, see k1_build_kernel)
   bool prof = false;
   struct ProfRec { int stage; cudaEvent_t a, b; };
@@ -99,7 +99,7 @@ struct eims_plan {
   // Planes path of the GraphConv products (csrc/gemm_tma.cu): a_l, q and the GraphConv weights exist as stacked tf32
   // hi / lo planes [2][rows][H] and the GEMMs are fed by the tensor-map copy engine.  planes_cap: the shapes allow it
   // (H a multiple of 256, <= 1024) and the workspace was sized for it; planes_on(): ... and the tensor-core backend is
-  // selected and the path is not switched off (EIMS_GEMM_TMA=0).
+  // selected.
   bool planes_cap = false;
   int64_t act_plane = 0;   // floats between the hi and the lo plane of a_l / q ( = rows_alloc * H )
   int64_t w_plane = 0;     // floats between the hi and the lo plane of the weight range [W_1 .. W_{L-1}]
@@ -118,11 +118,11 @@ struct eims_plan {
   // outweighs the faster main loop: 0.363 against 0.342 ms per step.  At hidden 1024 (cfg 5: 14 tiles per SM, K = 1024) the
   // planes kernel needs ~12 TB/s of operand bytes out of L2 to keep the tensor cores fed and gets ~7: 7.48 against 7.03 ms
   // per step - fp32 operands split in the kernel are half the bytes.  So: large batches at hidden <= 512 only, unless
-  // EIMS_GEMM_TMA=1 / eims_plan_set_gemm_planes(EIMS_PLANES_ON).
+  // eims_plan_set_gemm_planes(EIMS_PLANES_ON).
   bool planes_on() const {
     if (!(planes_cap && gemm_backend == EIMS_GEMM_TCGEN05 && gemm_tma_enabled() && !maps.empty())) return false;
     if (planes_mode >= 0) return planes_mode != 0;
-    return gemm_tma_forced() || (d.hidden_dim <= 512 && (int64_t)((Nc + 127) / 128) * (d.hidden_dim / 256) >= 4 * 148);
+    return d.hidden_dim <= 512 && (int64_t)((Nc + 127) / 128) * (d.hidden_dim / 256) >= 4 * 148;
   }
   int planes_mode = -1;  // eims_plan_set_gemm_planes
   int pool_dim() const { return d.pooling == EIMS_POOL_COMBINED ? 2 * d.hidden_dim : d.hidden_dim; }
@@ -186,7 +186,7 @@ int gemm(eims_plan* p, const float* A, int lda, int a_mn, const float* B, int ld
 
 // weight gradient + data gradient of one layer (both consume the same dy) in one launch
 int gemm_pair(eims_plan* p, const GemmProblem& a, const GemmProblem& b, cudaStream_t st) {
-  if (p->gemm_backend == EIMS_GEMM_FP32_SIMT || !p->pair_gemms) {
+  if (p->gemm_backend == EIMS_GEMM_FP32_SIMT) {
     for (const GemmProblem* q : {&a, &b})
       if (int rc = gemm(p, q->A, q->lda, q->a_mn, q->B, q->ldb, q->b_mn, q->C, q->ldc, q->M, q->N, q->K, q->m_dev, q->k_dev,
                         q->row_scale, q->bias, q->relu, q->accumulate, st, q->bn)) return rc;
@@ -238,11 +238,6 @@ struct EarlyDimsScope {
   explicit EarlyDimsScope(int v) { dims_early_ref() = v; }
   ~EarlyDimsScope() { dims_early_ref() = 0; }
 };
-bool early_dims_enabled() {
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("EIMS_EARLY_DIMS"); on = (e && e[0] == '0') ? 0 : 1; }
-  return on != 0;
-}
 
 #define STAGE(id, nk, expr)          \
   do {                               \
@@ -359,7 +354,7 @@ int eims_gemm_planes(const eims_gemm_problem* p0, const eims_gemm_problem* p1, v
   if (!p0 || !scratch) return fail(EIMS_ERR_ARG, "problem / scratch is NULL");
   if (scratch_bytes < eims_gemm_planes_scratch_bytes(p0, p1)) return fail(EIMS_ERR_ARG, "scratch too small");
   if (reinterpret_cast<uintptr_t>(scratch) & 255) return fail(EIMS_ERR_ARG, "scratch must be 256-byte aligned");
-  if (!gemm_tma_enabled()) return fail(EIMS_ERR_STATE, "the planes GEMM is unavailable (EIMS_GEMM_TMA=0 or no cuTensorMapEncodeTiled)");
+  if (!gemm_tma_enabled()) return fail(EIMS_ERR_STATE, "the planes GEMM is unavailable (no cuTensorMapEncodeTiled)");
   cudaStream_t st = (cudaStream_t)stream;
   TmaMap maps[4];
   GemmTmaProblem gp[2];
@@ -375,9 +370,8 @@ int eims_gemm_planes(const eims_gemm_problem* p0, const eims_gemm_problem* p1, v
     for (int o = 0; o < 2; ++o) {
       const int64_t plane = rows[o] * ld[o];
       float* hi = reinterpret_cast<float*>(c);
-      // EIMS_PLANES_SKIP_SPLIT (diagnostic timing only): reuse the planes the previous call left in scratch
-      if (!getenv("EIMS_PLANES_SKIP_SPLIT")) EIMS_TRY(launch_split_planes(src[o], hi, hi + plane, plane, st, false));
-      EIMS_TRY(tma_make_map(&maps[2 * n + o], hi, plane, (int)rows[o], cols[o], ld[o], o ? gemm_tma_b_rows() : 128, mn[o]));
+      EIMS_TRY(launch_split_planes(src[o], hi, hi + plane, plane, st, false));
+      EIMS_TRY(tma_make_map(&maps[2 * n + o], hi, plane, (int)rows[o], cols[o], ld[o], o ? kTmaBRows : 128, mn[o]));
       c += ((2 * 4 * plane + 255) & ~(int64_t)255);
     }
     gp[n] = GemmTmaProblem{&maps[2 * n], &maps[2 * n + 1], q->C, q->ldc, q->a_mn_major, q->b_mn_major, q->M, q->N, q->K, q->m_dev,
@@ -449,13 +443,7 @@ int eims_plan_create(const eims_dims* d, int32_t max_graphs, int32_t max_nodes, 
   p->d = *d;
   p->Bc = max_graphs; p->Nc = max_nodes; p->Ec = max_edges > 0 ? max_edges : 1;
   p->gemm_backend = EIMS_GEMM_TCGEN05;
-  if (const char* e = getenv("EIMS_FUSE_SPMM_BWD")) p->fuse_spmm_bwd = e[0] != '0';
-  if (const char* e = getenv("EIMS_PAIR_GEMMS")) p->pair_gemms = e[0] != '0';
-  if (const char* e = getenv("EIMS_TOP_STATS_PER_GRAPH")) p->top_stats_per_graph = e[0] != '0';
-  // (beyond 256 columns the statistics variant of K2 needs 172 registers - one block per SM - and measured slower
-  // than K2 plus the separate statistics pass: cfg 5, 0.99 + 0.02 ms against 0.38 + 0.43 ms per step)
   p->fuse_bn_bwd_stats = d->hidden_dim <= 256;
-  if (const char* e = getenv("EIMS_FUSE_BN_BWD_STATS")) p->fuse_bn_bwd_stats = e[0] != '0';
   p->ws_bytes = 0; p->bound = false; p->state = 0; p->last_training = 0;
   memset(&p->last_step, 0, sizeof(p->last_step));
   auto s = param_sizes(d);
@@ -532,8 +520,8 @@ int eims_plan_bind(eims_plan* p, void* workspace, int64_t bytes) {
       float* w = wpl + (p->off_gcn_w(l) - p->off_gcn_w(1));
       rc = tma_make_map(&p->maps[4 * (l - 1) + 0], a, p->act_plane, rows, H, H, 128, 0);
       if (!rc) rc = tma_make_map(&p->maps[4 * (l - 1) + 1], a, p->act_plane, rows, H, H, 128, 1);
-      if (!rc) rc = tma_make_map(&p->maps[4 * (l - 1) + 2], w, p->w_plane, H, H, H, gemm_tma_b_rows(), 1);
-      if (!rc) rc = tma_make_map(&p->maps[4 * (l - 1) + 3], w, p->w_plane, H, H, H, gemm_tma_b_rows(), 0);
+      if (!rc) rc = tma_make_map(&p->maps[4 * (l - 1) + 2], w, p->w_plane, H, H, H, kTmaBRows, 1);
+      if (!rc) rc = tma_make_map(&p->maps[4 * (l - 1) + 3], w, p->w_plane, H, H, H, kTmaBRows, 0);
     }
     float* q = reinterpret_cast<float*>(p->buf["q"].ptr);
     if (!rc) rc = tma_make_map(&p->maps[4 * (L - 1) + 0], q, p->act_plane, rows, H, H, 128, 0);
@@ -690,7 +678,7 @@ int eims_forward(eims_plan* p, const float* params, float* bn_running, int32_t t
     if (!training) STAGE(ST_BN_STATS, 1, bn(0));
   }
   // every launch from here on is at least two kernels after the batch build: sizes before the grid-dependency wait
-  EarlyDimsScope early_scope(early_dims_enabled() ? 1 : 0);
+  EarlyDimsScope early_scope(1);
   const bool planes = p->planes_on();
   if (planes)  // hi / lo planes of the GraphConv weights W_1 .. W_{L-1} (one pass over the range that holds them)
     STAGE(ST_ELEMENTWISE, 1, launch_split_planes(params + p->off_gcn_w(1), p->f("wplanes"), p->f("wplanes") + p->w_plane, p->w_plane, st, true));
@@ -755,7 +743,7 @@ static int loss_impl(eims_plan* p, const float* targets, const int32_t* target_r
   if (!targets && !peaks && p->peak_targets.peak_ptr) peaks = &p->peak_targets;
   if (!targets && !peaks) return fail(EIMS_ERR_ARG, "targets is NULL (and no peak-list targets are set)");
   cudaStream_t st = (cudaStream_t)stream;
-  EarlyDimsScope early_scope(early_dims_enabled() && p->state >= 2 ? 1 : 0);  // after a forward, never right after a batch build
+  EarlyDimsScope early_scope(p->state >= 2 ? 1 : 0);  // after a forward, never right after a batch build
   // metrics != NULL: the last block of the loss kernel also folds the row terms into the running
   // metrics (flags[0] is its ticket), which saves the separate one-block launch
   STAGE(ST_LOSS, 1, launch_loss(p->i("dims"), p->f("logits"), targets, target_rows, p->d.max_mz, loss_kind, p->f("prob"),
@@ -782,7 +770,7 @@ int eims_backward_part(eims_plan* p, const float* params, const float* dprob, fl
   }
   if (!params || !grads) return fail(EIMS_ERR_ARG, "params / grads is NULL");
   cudaStream_t st = (cudaStream_t)stream;
-  EarlyDimsScope early_scope(early_dims_enabled() ? 1 : 0);  // backward always follows a forward (state >= 2)
+  EarlyDimsScope early_scope(1);  // backward always follows a forward (state >= 2)
   const eims_dims& d = p->d;
   const int H = d.hidden_dim, F = d.node_feat_dim, L = d.num_gcn_layers, M = d.max_mz, P = p->pool_dim();
   const int* dims = p->i("dims");
@@ -806,18 +794,18 @@ int eims_backward_part(eims_plan* p, const float* params, const float* dprob, fl
   } else {
     STAGE(ST_COLSUM, 1, launch_colsum(dims, DIM_B, dl, M, M, grads + p->off_head(9), p->Bc, st));
   }
-  STAGE(ST_GEMM_HEAD_BWD, (p->pair_gemms && p->gemm_backend == EIMS_GEMM_TCGEN05) ? 1 : 2, gemm_pair(p,
+  STAGE(ST_GEMM_HEAD_BWD, p->gemm_backend == EIMS_GEMM_TCGEN05 ? 1 : 2, gemm_pair(p,
         GemmProblem{dl, M, 1, p->f("y2"), H, 1, grads + p->off_head(8), H, M, H, p->Bc, nullptr, dB, nullptr, nullptr, 0, 1, nullptr},
         GemmProblem{dl, M, 0, params + p->off_head(8), H, 1, p->f("dy2"), H, p->Bc, H, M, dB, nullptr, nullptr, nullptr, 0, 3, nullptr}, st));
   // LayerNorm backward also leaves the bias gradient of the Linear in front of it (column sums of du)
   STAGE(ST_LN_BWD, 1, launch_ln_bwd(dims, p->f("u2"), p->f("y2"), p->f("dy2"), H, params + p->off_head(6), p->f("ln2"), drop_scale,
                          p->f("dy2"), grads + p->off_head(6), grads + p->off_head(7), grads + p->off_head(5), p->Bc, st));
-  STAGE(ST_GEMM_HEAD_BWD, (p->pair_gemms && p->gemm_backend == EIMS_GEMM_TCGEN05) ? 1 : 2, gemm_pair(p,
+  STAGE(ST_GEMM_HEAD_BWD, p->gemm_backend == EIMS_GEMM_TCGEN05 ? 1 : 2, gemm_pair(p,
         GemmProblem{p->f("dy2"), H, 1, p->f("y1"), 2 * H, 1, grads + p->off_head(4), 2 * H, H, 2 * H, p->Bc, nullptr, dB, nullptr, nullptr, 0, 1, nullptr},
         GemmProblem{p->f("dy2"), H, 0, params + p->off_head(4), 2 * H, 1, p->f("dy1"), 2 * H, p->Bc, 2 * H, H, dB, nullptr, nullptr, nullptr, 0, 3, nullptr}, st));
   STAGE(ST_LN_BWD, 1, launch_ln_bwd(dims, p->f("u1"), p->f("y1"), p->f("dy1"), 2 * H, params + p->off_head(2), p->f("ln1"),
                          drop_scale, p->f("dy1"), grads + p->off_head(2), grads + p->off_head(3), grads + p->off_head(1), p->Bc, st));
-  STAGE(ST_GEMM_HEAD_BWD, (p->pair_gemms && p->gemm_backend == EIMS_GEMM_TCGEN05) ? 1 : 2, gemm_pair(p,
+  STAGE(ST_GEMM_HEAD_BWD, p->gemm_backend == EIMS_GEMM_TCGEN05 ? 1 : 2, gemm_pair(p,
         GemmProblem{p->f("dy1"), 2 * H, 1, p->f("readout"), P, 1, grads + p->off_head(0), P, 2 * H, P, p->Bc, nullptr, dB, nullptr, nullptr, 0, 1, nullptr},
         GemmProblem{p->f("dy1"), 2 * H, 0, params + p->off_head(0), P, 1, p->f("dG"), P, p->Bc, P, 2 * H, dB, nullptr, nullptr, nullptr, 0, 3, nullptr}, st));
   p->state = 4;  // head gradients final (the data-parallel reducer may start on that bucket)
@@ -825,26 +813,22 @@ int eims_backward_part(eims_plan* p, const float* params, const float* dprob, fl
   if (part == EIMS_BWD_HEAD) return check_launch("eims_backward_part");
   // ---- GCN layers, last to first (GCN:358-363 backwards)
   for (int l = L - 1; l >= 0; --l) {
+    // the top layer's dh is the readout backward of dG, computed on the fly, and its BatchNorm-backward statistics come
+    // from per-graph quantities; the layers below read the dh that the backward SpMM of the layer above wrote, and their
+    // statistics pass rides on that SpMM when fuse_bn_bwd_stats (see below)
     const bool from_readout = (l == L - 1);
-    // layers below the last get their dh = (A da) * c * dropmask from the layer above, gathered on
-    // the fly inside both BatchNorm-backward passes when EIMS_FUSE_SPMM_BWD=1; by default K2 materialises it
-    const bool gather = !from_readout && p->fuse_spmm_bwd;
-    const float* dh_in = (from_readout || gather) ? nullptr : p->f("dh");
-    GatherSrc gsrc{p->f("da"), p->i("rowptr"), p->i("col"), p->f("norm"), p->drop(drop_p, seed, step, l)};
-    const GatherSrc* gs = gather ? &gsrc : nullptr;
-    // the statistics pass of layer l < L-1 rides on the SpMM that wrote its dh (see below)
-    if (from_readout && p->top_stats_per_graph)
+    const float* dh_in = from_readout ? nullptr : p->f("dh");
+    if (from_readout)
       STAGE(ST_BN_BWD_STATS, 1, launch_bn_bwd_stats_top(dims, p->f("dG"), p->f("zstat"), p->i("gptr"), d.pooling, H, p->f(L_("bn_mean", l)),
                                    p->f(L_("bn_invstd", l)), grads + p->off_bn_g(l), grads + p->off_bn_b(l), p->f("bn_means2"),
                                    p->f("bn_partials"), p->Bc, st));
-    else if (from_readout || gather || !p->fuse_bn_bwd_stats)
-    STAGE(ST_BN_BWD_STATS, 1, launch_bn_bwd_stats(dims, dh_in, p->f("dG"), p->i("gid"), p->i("gptr"), p->i("argmax"), d.pooling,
-                                 p->f(L_("z", l)), H, p->f(L_("bn_mean", l)), p->f(L_("bn_invstd", l)), grads + p->off_bn_g(l),
-                                 grads + p->off_bn_b(l), p->f("bn_means2"), p->f("bn_partials"), p->Nc, st, gs));
+    else if (!p->fuse_bn_bwd_stats)
+      STAGE(ST_BN_BWD_STATS, 1, launch_bn_bwd_stats(dims, dh_in, p->f(L_("z", l)), H, p->f(L_("bn_mean", l)), p->f(L_("bn_invstd", l)),
+                                   grads + p->off_bn_g(l), grads + p->off_bn_b(l), p->f("bn_means2"), p->f("bn_partials"), p->Nc, st));
     STAGE(ST_BN_BWD_APPLY, 1, launch_bn_bwd_apply(dims, dh_in, p->f("dG"), p->i("gid"), p->i("gptr"), p->i("argmax"), d.pooling,
                                  p->f(L_("z", l)), H, p->f(L_("bn_mean", l)), p->f(L_("bn_invstd", l)), params + p->off_bn_g(l),
                                  p->f("norm"), grads + p->off_gcn_b(l), p->f("bn_means2"), p->f("q"), p->Nc, st,
-                                 l == 0 ? p->f("a0") : nullptr, F, l == 0 ? grads + p->off_gcn_w(0) : nullptr, gs,
+                                 l == 0 ? p->f("a0") : nullptr, F, l == 0 ? grads + p->off_gcn_w(0) : nullptr,
                                  (planes && l > 0) ? p->act_plane : 0));
     if (l > 0 && planes) {
       // one persistent launch: data gradient tiles (stores) + weight gradient k-slices (red.add), balanced on the device
@@ -852,20 +836,18 @@ int eims_backward_part(eims_plan* p, const float* params, const float* dprob, fl
       GemmTmaProblem wg{p->map_a_mn(l), p->map_q_mn(), grads + p->off_gcn_w(l), H, 1, 1, H, H, p->Nc, nullptr, dims + DIM_N, nullptr, nullptr, 0, 1, nullptr};
       STAGE(ST_GEMM_GCN_BWD, 1, launch_gemm_tma(&dg, &wg, st));
     } else if (l > 0) {
-      STAGE(ST_GEMM_GCN_BWD, (p->pair_gemms && p->gemm_backend == EIMS_GEMM_TCGEN05) ? 1 : 2, gemm_pair(p,
+      STAGE(ST_GEMM_GCN_BWD, p->gemm_backend == EIMS_GEMM_TCGEN05 ? 1 : 2, gemm_pair(p,
             GemmProblem{p->f(L_("a", l)), H, 1, p->f("q"), H, 1, grads + p->off_gcn_w(l), H, H, H, p->Nc, nullptr, dims + DIM_N, nullptr, nullptr, 0, 1, nullptr},
             GemmProblem{p->f("q"), H, 0, params + p->off_gcn_w(l), H, 0, p->f("da"), H, p->Nc, H, H, dims + DIM_N, nullptr, nullptr, nullptr, 0, 0, nullptr}, st));
     }
     if (l > 0) {
-      if (!p->fuse_spmm_bwd) {
-        float* scratch = p->f("bn_partials");
-        BnBwdFuse bf{p->f(L_("z", l - 1)), p->f(L_("bn_mean", l - 1)), p->f(L_("bn_invstd", l - 1)),
-                     reinterpret_cast<double*>(scratch + 16), reinterpret_cast<unsigned int*>(scratch),
-                     grads + p->off_bn_g(l - 1), grads + p->off_bn_b(l - 1), p->f("bn_means2")};
-        STAGE(ST_SPMM_BWD, 1, launch_spmm_norm(dims, p->i("rowptr"), p->i("col"), p->f("norm"), p->f("da"), H, nullptr, nullptr,
-                                  p->drop(drop_p, seed, step, l - 1), 1, p->f("dh"), p->Nc, st,
-                                  p->fuse_bn_bwd_stats ? &bf : nullptr, p->i("gptr"), p->Bc, p->tile_rows()));
-      }
+      float* scratch = p->f("bn_partials");
+      BnBwdFuse bf{p->f(L_("z", l - 1)), p->f(L_("bn_mean", l - 1)), p->f(L_("bn_invstd", l - 1)),
+                   reinterpret_cast<double*>(scratch + 16), reinterpret_cast<unsigned int*>(scratch),
+                   grads + p->off_bn_g(l - 1), grads + p->off_bn_b(l - 1), p->f("bn_means2")};
+      STAGE(ST_SPMM_BWD, 1, launch_spmm_norm(dims, p->i("rowptr"), p->i("col"), p->f("norm"), p->f("da"), H, nullptr, nullptr,
+                                p->drop(drop_p, seed, step, l - 1), 1, p->f("dh"), p->Nc, st,
+                                p->fuse_bn_bwd_stats ? &bf : nullptr, p->i("gptr"), p->Bc, p->tile_rows()));
     }  // l == 0: dW0 came out of the BatchNorm-backward apply pass above (q_0 is never materialised)
   }
   p->state = 1;
@@ -995,7 +977,7 @@ int eims_infer_batch(eims_plan* p, const eims_dataset* ds, const int32_t* mol_id
   EIMS_TRY(eims_batch_build(p, ds, mol_ids, num_graphs, stream));
   EIMS_TRY(eims_forward(p, params, const_cast<float*>(bn_running), 0, nullptr, stream));
   cudaStream_t st = (cudaStream_t)stream;
-  EarlyDimsScope early_scope(early_dims_enabled() ? 1 : 0);
+  EarlyDimsScope early_scope(1);
   STAGE(ST_ELEMENTWISE, 1, launch_sigmoid(p->i("dims"), p->f("logits"), p->d.max_mz, prob_out ? prob_out : p->f("prob"), p->Bc,
                           (cudaStream_t)stream));
   return check_launch("eims_infer_batch");

@@ -583,8 +583,8 @@ class GraphedTrainStep:
         self.hold_next, self.held = False, None
         self.side = torch.cuda.Stream(plan.device)
         # second side branch: the bias gradient of the output layer and the head's AdamW run off the chain (single GPU;
-        # in data-parallel runs the fused exchange kernel is the optimiser).  EIMS_STEP_SIDE_BRANCH=0 keeps one chain.
-        self.side2 = torch.cuda.Stream(plan.device) if (fused is None and os.environ.get("EIMS_STEP_SIDE_BRANCH", "1") != "0") else None
+        # in data-parallel runs the fused exchange kernel is the optimiser)
+        self.side2 = torch.cuda.Stream(plan.device) if fused is None else None
         plan.enable_step_block(max(self.group, 1))
         if fused is None:
             fp.ensure_adam()

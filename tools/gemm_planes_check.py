@@ -59,6 +59,19 @@ def timeit(fn, n=200):
     return e0.elapsed_time(e1) / n * 1e3
 
 
+def planes_kernel_us(fn, n=200):
+    """Mean time of the gemm_planes_kernel launches of one call of fn, from the profiler's kernel records: the GEMM alone,
+    without the split kernels eims_gemm_planes launches in front of it."""
+    for _ in range(20):
+        fn()
+    torch.cuda.synchronize()
+    with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+        for _ in range(n):
+            fn()
+        torch.cuda.synchronize()
+    return sum(e.device_time_total for e in prof.key_averages() if "gemm_planes_kernel" in e.key) / n
+
+
 def sweep(R, Nl, Nc, H):
     dev = "cuda"
     nd = torch.tensor([Nl], dtype=torch.int32, device=dev)
@@ -67,11 +80,7 @@ def sweep(R, Nl, Nc, H):
         W = torch.randn(K, H, device=dev)
         Z = torch.zeros(Nc, H, device=dev)
         p = problem(X, 0, W, 1, Z, Nc, H, K, m_dev=nd)
-        R.run(p)
-        torch.cuda.synchronize()
-        os.environ["EIMS_PLANES_SKIP_SPLIT"] = "1"
-        us = timeit(lambda: R.run(p))
-        del os.environ["EIMS_PLANES_SKIP_SPLIT"]
+        us = planes_kernel_us(lambda: R.run(p))
         old = timeit(lambda: R.old(p))
         print(f"K={K:4d}  planes {us:7.2f} us   in-kernel split {old:7.2f} us")
     return 0
@@ -148,15 +157,12 @@ def main():
         return 0 if ok else 1
 
     lib, st = R.lib, R.st
-    # time the GEMM launches alone (planes left in scratch by the previous call) and with the two split kernels
+    # time the GEMM launch alone (profiler kernel time) and back to back with the split kernels in front of it
     for name, p0, p1, flops in (("forward", pf, None, 2.0 * Nl * H * H), ("dgrad", pd, None, 2.0 * Nl * H * H),
                                 ("wgrad", pw, None, 2.0 * Nl * H * H), ("dgrad+wgrad", pd, pw, 4.0 * Nl * H * H)):
-        R.run(p0, p1)
-        torch.cuda.synchronize()
-        split = timeit(lambda: [check(lib.eims_gemm_planes(C.byref(p0), C.byref(p1) if p1 is not None else None, ptr(R.scratch), R.scratch.numel(), st))], 50)
-        os.environ["EIMS_PLANES_SKIP_SPLIT"] = "1"
-        us = timeit(lambda: check(lib.eims_gemm_planes(C.byref(p0), C.byref(p1) if p1 is not None else None, ptr(R.scratch), R.scratch.numel(), st)))
-        del os.environ["EIMS_PLANES_SKIP_SPLIT"]
+        call = lambda: check(lib.eims_gemm_planes(C.byref(p0), C.byref(p1) if p1 is not None else None, ptr(R.scratch), R.scratch.numel(), st))  # noqa: E731
+        split = timeit(call, 50)
+        us = planes_kernel_us(call)
         if p1 is None:
             old = timeit(lambda: R.old(p0))
         else:

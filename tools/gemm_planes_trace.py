@@ -48,10 +48,8 @@ def main():
             R.run(p0, p1)
             torch.cuda.synchronize()
         assert rd(buf, 512) == 0   # reset
-        os.environ["EIMS_PLANES_SKIP_SPLIT"] = "1"
         R.run(p0, p1)
         torch.cuda.synchronize()
-        del os.environ["EIMS_PLANES_SKIP_SPLIT"]
         assert rd(buf, 512) == 0
         t = np.array(buf[:], dtype=np.int64).reshape(8, 64)
         print(f"==== {title}")
