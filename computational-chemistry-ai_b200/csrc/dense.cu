@@ -977,16 +977,7 @@ int launch_adamw(float* p, float* g, float* m, float* v, int64_t n, const eims_s
   return 0;
 }
 
-// ---- step block upload: one block stores the by-value struct (see StepBlock in common.cuh)
-__global__ void step_block_store_kernel(StepBlock v, StepBlock* __restrict__ dst) {
-  pdl_sync();
-  if (threadIdx.x == 0) *dst = v;
-}
-int launch_step_block_store(const StepBlock& v, StepBlock* dst, cudaStream_t st) {
-  launch_pdl(step_block_store_kernel, dim3(1), dim3(32), 0, st, v, dst);
-  return 0;
-}
-// several consecutive blocks at once (a graph that holds several steps): still one launch, the blocks by value
+// ---- step block upload: consecutive blocks (see StepBlock in common.cuh) by value, one launch for up to kStepPack
 __global__ void step_blocks_store_kernel(StepBlockPack v, StepBlock* __restrict__ dst, int n) {
   pdl_sync();
   if ((int)threadIdx.x < n) dst[threadIdx.x] = v.b[threadIdx.x];

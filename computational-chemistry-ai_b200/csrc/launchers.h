@@ -77,7 +77,6 @@ int launch_metrics(const int* dims, const float* row_loss, const float* row_cos,
 int launch_colsum(const int* dims, int dim_slot, const float* in, int C, int ld, float* out, int max_rows, cudaStream_t st);
 int launch_adamw(float* p, float* g, float* m, float* v, int64_t n, const eims_step* s, cudaStream_t st,
                  const StepBlock* blk = nullptr);  // blk: the scalars are read from the device step block
-int launch_step_block_store(const StepBlock& v, StepBlock* dst, cudaStream_t st);
 int launch_step_blocks_store(const StepBlockPack& v, StepBlock* dst, int n, cudaStream_t st);
 int launch_dropout_mask(DropCfg d, int rows, int W, float* out, cudaStream_t st);
 

@@ -632,9 +632,7 @@ int eims_step_blocks_upload(eims_plan* p, const eims_step* steps, const int32_t*
 int eims_step_block_upload(eims_plan* p, const eims_step* s, const int32_t* mol_ids, uint32_t dp_seq, eims_stream_t stream) {
   if (!p || !p->blk) return fail(EIMS_ERR_STATE, "no step block set (eims_plan_set_step_block)");
   if (!s || s->step < 1) return fail(EIMS_ERR_ARG, "step scalars are NULL / step < 1");
-  const StepBlock v = make_step_block(p, s, mol_ids, dp_seq);
-  EIMS_TRY(launch_step_block_store(v, p->blk, (cudaStream_t)stream));
-  return check_launch("eims_step_block_upload");
+  return eims_step_blocks_upload(p, s, &mol_ids, &dp_seq, (int32_t)(p->blk - p->blk_base), 1, stream);
 }
 
 int eims_forward(eims_plan* p, const float* params, float* bn_running, int32_t training, const eims_step* s,
@@ -865,64 +863,46 @@ int eims_metrics_accumulate(eims_plan* p, float* metrics, eims_stream_t stream) 
   return check_launch("eims_metrics_accumulate");
 }
 
-int eims_train_step(eims_plan* p, const eims_dataset* ds, const int32_t* mol_ids, int32_t num_graphs, float* params,
-                    float* grads, float* adam_m, float* adam_v, float* bn_running, int32_t loss_kind,
-                    const eims_step* s, float* metrics, eims_stream_t stream) {
-  if (!s) return fail(EIMS_ERR_ARG, "step scalars are NULL");
-  if (!ds || (!ds->targets && !ds->peaks)) return fail(EIMS_ERR_ARG, "training needs dataset targets (dense rows or peak lists)");
-  EIMS_TRY(eims_batch_build(p, ds, mol_ids, num_graphs, stream));
-  EIMS_TRY(eims_forward(p, params, bn_running, 1, s, stream));
-  EIMS_TRY(loss_impl(p, ds->targets, mol_ids, loss_kind, 1, metrics, stream, ds->targets ? nullptr : ds->peaks));
-  EIMS_TRY(eims_backward(p, params, nullptr, grads, stream));
-  if (adam_m && adam_v) {
-    cudaStream_t st = (cudaStream_t)stream;
-    STAGE(ST_ADAMW, 1, launch_adamw(params, grads, adam_m, adam_v, p->poff.back(), s, st));
-  }
-  return 0;
-}
+// One training step on the batch built last, as every eims_train_step* entry point enqueues it.
+struct StepCall {
+  const float* targets;         // dense target rows; NULL: `peaks`, else the plan's peak-list targets
+  const eims_peaks* peaks;
+  const int32_t* target_rows;   // direct calls only: an indirect step reads the rows K1 took from the step block
+  float *params, *grads, *adam_m, *adam_v, *bn_running;  // AdamW runs when adam_m and adam_v are both set
+  int32_t loss_kind;
+  const eims_step* s;           // direct: the step's scalars; NULL: indirect, scalars and dropout keys from the step block
+  float* metrics;
+  int32_t part;                 // EIMS_BWD_ALL; EIMS_BWD_HEAD: forward, loss, head backward; EIMS_BWD_GCN: the rest
+  cudaStream_t st, side;        // side (indirect only): output-layer bias gradient and the head's AdamW
+};
 
-int eims_train_step_built(eims_plan* p, const float* targets, const int32_t* target_rows, float* params, float* grads,
-                          float* adam_m, float* adam_v, float* bn_running, int32_t loss_kind, const eims_step* s,
-                          float* metrics, eims_stream_t stream) {
-  if (!s) return fail(EIMS_ERR_ARG, "step scalars are NULL");
-  if (!targets && !(p && p->peak_targets.peak_ptr)) return fail(EIMS_ERR_ARG, "training needs target spectra");
-  EIMS_TRY(eims_forward(p, params, bn_running, 1, s, stream));
-  EIMS_TRY(loss_impl(p, targets, target_rows, loss_kind, 1, metrics, stream));
-  EIMS_TRY(eims_backward(p, params, nullptr, grads, stream));
-  if (adam_m && adam_v) {
-    cudaStream_t st = (cudaStream_t)stream;
-    STAGE(ST_ADAMW, 1, launch_adamw(params, grads, adam_m, adam_v, p->poff.back(), s, st));
-  }
-  return 0;
-}
-
-int eims_train_step_built_indirect(eims_plan* p, const float* targets, float* params, float* grads, float* adam_m,
-                                   float* adam_v, float* bn_running, int32_t loss_kind, float* metrics, eims_stream_t stream,
-                                   eims_stream_t side_stream) {
-  if (!p || !p->blk) return fail(EIMS_ERR_STATE, "no step block set (eims_plan_set_step_block)");
-  if (!targets && !p->peak_targets.peak_ptr) return fail(EIMS_ERR_ARG, "training needs target spectra");
-  cudaStream_t st = (cudaStream_t)stream, side = (cudaStream_t)side_stream;
-  if (side && side != st && p->ensure_events()) return fail(EIMS_ERR_CUDA, "cudaEventCreate failed");
-  if (side == st) side = nullptr;
-  eims_step dummy{};  // seed / step are not used: the dropout keys come from the step block
-  struct Scope {  // the plan's per-call mode must not leak out of this function
+// forward -> loss (+ metrics) -> backward [-> AdamW].  The plan's per-call mode (indirect, side) is set here only and
+// must not leak out of this function.
+static int enqueue_step(eims_plan* p, const StepCall& c) {
+  if (!p || !p->bound) return fail(EIMS_ERR_STATE, "plan not bound");
+  const cudaStream_t st = c.st, side = c.side == c.st ? nullptr : c.side;
+  if (side && p->ensure_events()) return fail(EIMS_ERR_CUDA, "cudaEventCreate failed");
+  const eims_stream_t stream = (eims_stream_t)st;
+  const bool indirect = !c.s;
+  struct Mode {
     eims_plan* p;
-    ~Scope() { p->indirect = false; p->side = nullptr; }
-  } scope{p};
-  p->indirect = true;
+    ~Mode() { p->indirect = false; p->side = nullptr; }
+  } mode{p};
+  p->indirect = indirect;
   p->side = side;
-  EIMS_TRY(eims_forward(p, params, bn_running, 1, &dummy, stream));
-  EIMS_TRY(loss_impl(p, targets, p->i("bids"), loss_kind, 1, metrics, stream));
-  const bool adam = adam_m && adam_v;
+  if (c.part != EIMS_BWD_GCN) {
+    const eims_step dummy{};  // indirect: seed / step are not used, the dropout keys come from the step block
+    EIMS_TRY(eims_forward(p, c.params, c.bn_running, 1, indirect ? &dummy : c.s, stream));
+    EIMS_TRY(loss_impl(p, c.targets, indirect ? p->i("bids") : c.target_rows, c.loss_kind, 1, c.metrics, stream,
+                       c.targets ? nullptr : c.peaks));
+  }
+  if (c.part != EIMS_BWD_ALL) return eims_backward_part(p, c.params, nullptr, c.grads, c.part, stream);
+  const bool adam = c.adam_m && c.adam_v;
+  const StepBlock* blk = indirect ? p->blk : nullptr;
   const int64_t P = p->poff.back();
-  int64_t split = p->off_head(0) & ~(int64_t)3;   // [0, split) GraphConv + BatchNorm tensors, [split, P) the head
   if (!side || !adam) {
-    EIMS_TRY(eims_backward(p, params, nullptr, grads, stream));
-    if (adam) {
-      prof_begin(p, ST_ADAMW, 1, st);
-      EIMS_TRY(launch_adamw(params, grads, adam_m, adam_v, P, nullptr, st, p->blk));
-      prof_end(p, st);
-    }
+    EIMS_TRY(eims_backward(p, c.params, nullptr, c.grads, stream));
+    if (adam) STAGE(ST_ADAMW, 1, launch_adamw(c.params, c.grads, c.adam_m, c.adam_v, P, c.s, st, blk));
     if (side) {  // join the colsum branch
       if (cudaEventRecord(p->ev[1], side) != cudaSuccess || cudaStreamWaitEvent(st, p->ev[1], 0) != cudaSuccess)
         return fail(EIMS_ERR_CUDA, "side-branch join failed");
@@ -931,22 +911,47 @@ int eims_train_step_built_indirect(eims_plan* p, const float* targets, float* pa
   }
   // head part on the main stream (its bias-gradient colsum on the side branch), then
   //   side: AdamW of the head range, as soon as the head gradients are final   ||   main: GCN layers backward
-  EIMS_TRY(eims_backward_part(p, params, nullptr, grads, EIMS_BWD_HEAD, stream));
+  const int64_t split = p->off_head(0) & ~(int64_t)3;   // [0, split) GraphConv + BatchNorm tensors, [split, P) the head
+  EIMS_TRY(eims_backward_part(p, c.params, nullptr, c.grads, EIMS_BWD_HEAD, stream));
   if (cudaEventRecord(p->ev[2], st) != cudaSuccess || cudaStreamWaitEvent(side, p->ev[2], 0) != cudaSuccess)
     return fail(EIMS_ERR_CUDA, "side-branch fork failed");
   prof_begin(p, ST_ADAMW, 1, side);
-  EIMS_TRY(launch_adamw(params + split, grads + split, adam_m + split, adam_v + split, P - split, nullptr, side, p->blk));
+  EIMS_TRY(launch_adamw(c.params + split, c.grads + split, c.adam_m + split, c.adam_v + split, P - split, c.s, side, blk));
   prof_end(p, side);
   if (cudaEventRecord(p->ev[1], side) != cudaSuccess) return fail(EIMS_ERR_CUDA, "cudaEventRecord failed");
   p->side = nullptr;  // the GCN part has nothing for the side branch
-  EIMS_TRY(eims_backward_part(p, params, nullptr, grads, EIMS_BWD_GCN, stream));
-  if (split > 0) {
-    prof_begin(p, ST_ADAMW, 1, st);
-    EIMS_TRY(launch_adamw(params, grads, adam_m, adam_v, split, nullptr, st, p->blk));
-    prof_end(p, st);
-  }
+  EIMS_TRY(eims_backward_part(p, c.params, nullptr, c.grads, EIMS_BWD_GCN, stream));
+  if (split > 0) STAGE(ST_ADAMW, 1, launch_adamw(c.params, c.grads, c.adam_m, c.adam_v, split, c.s, st, blk));
   if (cudaStreamWaitEvent(st, p->ev[1], 0) != cudaSuccess) return fail(EIMS_ERR_CUDA, "side-branch join failed");
   return 0;
+}
+
+int eims_train_step(eims_plan* p, const eims_dataset* ds, const int32_t* mol_ids, int32_t num_graphs, float* params,
+                    float* grads, float* adam_m, float* adam_v, float* bn_running, int32_t loss_kind,
+                    const eims_step* s, float* metrics, eims_stream_t stream) {
+  if (!s) return fail(EIMS_ERR_ARG, "step scalars are NULL");
+  if (!ds || (!ds->targets && !ds->peaks)) return fail(EIMS_ERR_ARG, "training needs dataset targets (dense rows or peak lists)");
+  EIMS_TRY(eims_batch_build(p, ds, mol_ids, num_graphs, stream));
+  return enqueue_step(p, {ds->targets, ds->peaks, mol_ids, params, grads, adam_m, adam_v, bn_running, loss_kind, s, metrics,
+                          EIMS_BWD_ALL, (cudaStream_t)stream, nullptr});
+}
+
+int eims_train_step_built(eims_plan* p, const float* targets, const int32_t* target_rows, float* params, float* grads,
+                          float* adam_m, float* adam_v, float* bn_running, int32_t loss_kind, const eims_step* s,
+                          float* metrics, eims_stream_t stream) {
+  if (!s) return fail(EIMS_ERR_ARG, "step scalars are NULL");
+  if (!targets && !(p && p->peak_targets.peak_ptr)) return fail(EIMS_ERR_ARG, "training needs target spectra");
+  return enqueue_step(p, {targets, nullptr, target_rows, params, grads, adam_m, adam_v, bn_running, loss_kind, s, metrics,
+                          EIMS_BWD_ALL, (cudaStream_t)stream, nullptr});
+}
+
+int eims_train_step_built_indirect(eims_plan* p, const float* targets, float* params, float* grads, float* adam_m,
+                                   float* adam_v, float* bn_running, int32_t loss_kind, float* metrics, eims_stream_t stream,
+                                   eims_stream_t side_stream) {
+  if (!p || !p->blk) return fail(EIMS_ERR_STATE, "no step block set (eims_plan_set_step_block)");
+  if (!targets && !p->peak_targets.peak_ptr) return fail(EIMS_ERR_ARG, "training needs target spectra");
+  return enqueue_step(p, {targets, nullptr, nullptr, params, grads, adam_m, adam_v, bn_running, loss_kind, nullptr, metrics,
+                          EIMS_BWD_ALL, (cudaStream_t)stream, (cudaStream_t)side_stream});
 }
 
 // The same step in two parts for a caller that runs its own optimiser between them (data-parallel training: the head
@@ -956,20 +961,9 @@ int eims_train_step_built_indirect_part(eims_plan* p, const float* targets, floa
                                         int32_t loss_kind, float* metrics, int32_t part, eims_stream_t stream) {
   if (!p || !p->blk) return fail(EIMS_ERR_STATE, "no step block set (eims_plan_set_step_block)");
   if (part != 1 && part != 2) return fail(EIMS_ERR_ARG, "part must be 1 (forward, loss, head backward) or 2 (GraphConv backward)");
-  struct Scope {
-    eims_plan* p;
-    ~Scope() { p->indirect = false; p->side = nullptr; }
-  } scope{p};
-  p->indirect = true;
-  p->side = nullptr;
-  if (part == 1) {
-    if (!targets && !p->peak_targets.peak_ptr) return fail(EIMS_ERR_ARG, "training needs target spectra");
-    eims_step dummy{};  // seed / step are not used: the dropout keys come from the step block
-    EIMS_TRY(eims_forward(p, params, bn_running, 1, &dummy, stream));
-    EIMS_TRY(loss_impl(p, targets, p->i("bids"), loss_kind, 1, metrics, stream));
-    return eims_backward_part(p, params, nullptr, grads, EIMS_BWD_HEAD, stream);
-  }
-  return eims_backward_part(p, params, nullptr, grads, EIMS_BWD_GCN, stream);
+  if (part == 1 && !targets && !p->peak_targets.peak_ptr) return fail(EIMS_ERR_ARG, "training needs target spectra");
+  return enqueue_step(p, {targets, nullptr, nullptr, params, grads, nullptr, nullptr, bn_running, loss_kind, nullptr, metrics,
+                          part == 1 ? EIMS_BWD_HEAD : EIMS_BWD_GCN, (cudaStream_t)stream, nullptr});
 }
 
 int eims_infer_batch(eims_plan* p, const eims_dataset* ds, const int32_t* mol_ids, int32_t num_graphs,

@@ -158,5 +158,5 @@ def check(rc: int) -> None:
 
 
 def ptr(t):
-    """Device / host pointer of a torch tensor (None -> NULL)."""
-    return None if t is None else C.c_void_p(t.data_ptr())
+    """Device / host pointer of a torch tensor or an address (None -> NULL)."""
+    return None if t is None else C.c_void_p(t if isinstance(t, int) else t.data_ptr())

@@ -223,6 +223,12 @@ class FusedP2PAdamW:
         self.fp.grads = self.sym_grads[self.seq % 2][: self.fp.numel]
         self.seq += 1
 
+    def next_seqs(self, n: int):
+        """Sequence numbers of the next n steps run from captured graphs, which read theirs from the step blocks (the
+        gradient buffer each one uses was fixed by begin_step at capture)."""
+        self.seq += n
+        return list(range(self.seq - n + 1, self.seq + 1))
+
     def _launch(self, bucket, step, stream, step_block=None):
         from ._lib import check, ptr
         C = self.C

@@ -97,6 +97,19 @@ class FlatParams:
             self.adam_m = torch.zeros_like(self.params)
             self.adam_v = torch.zeros_like(self.params)
 
+    def step_ptrs(self, optimizer=True):
+        """params, grads, adam_m, adam_v, bn_running as arguments of a training step; without the optimiser the Adam
+        state is NULL (the step runs no AdamW)."""
+        if optimizer:
+            self.ensure_adam()
+        return (ptr(self.params), ptr(self.grads), ptr(self.adam_m) if optimizer else None,
+                ptr(self.adam_v) if optimizer else None, ptr(self.bn_running))
+
+    def count_steps(self, n=1):
+        """n more training-mode forwards: what BatchNorm's num_batches_tracked counts."""
+        for l in range(len(self.num_batches_tracked)):
+            self.num_batches_tracked[l] += n
+
     def views(self, flat):
         out = OrderedDict()
         for (name, shape), o in zip(self.spec, self.offsets):
@@ -277,6 +290,22 @@ class DeviceDataset:
         return int(self.host_num_atoms[ids].sum()), int(2 * self.host_num_bonds[ids].sum())
 
 
+class PackedDataset:
+    """One packed batch (the layout of eims_host_pack_batch / PackedHostBatch) at device address `base`, as the data set
+    of its `num_graphs` molecules.  offsets: section name -> byte offset from base; a section that is absent has no
+    entry.  Duck-types DeviceDataset for the plan: struct, targets (an address), peaks (a Peaks struct)."""
+
+    def __init__(self, base: int, offsets, num_graphs: int, mz_is_f64: int = 0):
+        o = offsets
+        self.num_mols = int(num_graphs)
+        self.targets = base + o["targets"] if "targets" in o else None
+        self.peaks = (_lib.Peaks(base + o["peak_ptr"], base + o["peak_mz"], base + o["peak_inten"], mz_is_f64, self.num_mols)
+                      if "peak_ptr" in o else None)
+        self.struct = Dataset(base + o["node_ptr"], base + o["bond_ptr"], base + o["feat"], base + o["bond_begin"],
+                              base + o["bond_end"], self.targets, self.num_mols,
+                              C.pointer(self.peaks) if self.peaks is not None else None)
+
+
 def make_step(lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-8, weight_decay=1e-4, grad_scale=1.0, step=1, seed=0) -> Step:
     return Step(lr, beta1, beta2, eps, weight_decay, grad_scale, int(step), int(seed))
 
@@ -320,6 +349,7 @@ class Plan:
         cd = d.c()
         check(self.lib.eims_plan_create(C.byref(cd), self.max_graphs, self.max_nodes, self.max_edges, C.byref(h)))
         self.h = h
+        self._peak_targets = None  # what eims_plan_set_peak_targets was last given (keeps the arrays alive)
         nbytes = self.lib.eims_plan_workspace_bytes(self.h)
         self.workspace = torch.empty(nbytes + 256, dtype=torch.uint8, device=self.device)
         self._base = (self.workspace.data_ptr() + 255) // 256 * 256
@@ -377,15 +407,18 @@ class Plan:
     def sigmoid(self):
         check(self.lib.eims_sigmoid(self.h, self.stream))
 
-    def set_peak_targets(self, peaks: "DevicePeaks"):
-        """Targets as peak lists, binned inside the loss kernel (eims_plan_set_peak_targets)."""
-        check(self.lib.eims_plan_set_peak_targets(self.h, C.byref(peaks.struct) if peaks is not None else None))
-        self._peak_targets = peaks  # keeps the arrays alive
+    def set_peak_targets(self, peaks):
+        """Targets as peak lists, binned inside the loss kernel (eims_plan_set_peak_targets): a DevicePeaks, the Peaks
+        struct of a PackedDataset, or None."""
+        s = peaks if peaks is None or isinstance(peaks, _lib.Peaks) else peaks.struct
+        check(self.lib.eims_plan_set_peak_targets(self.h, C.byref(s) if s is not None else None))
+        self._peak_targets = peaks
 
-    def _targets(self, ds: "DeviceDataset"):
-        """Dense target pointer of a dataset, or None after pointing the plan at its peak lists."""
-        if ds.targets is None and ds.peaks is not None and getattr(self, "_peak_targets", None) is not ds.peaks:
-            self.set_peak_targets(ds.peaks)
+    def _targets(self, ds):
+        """Dense targets of a DeviceDataset or PackedDataset; without them (None) the plan is pointed at its peak lists."""
+        peaks = ds.peaks if ds.targets is None else None
+        if peaks is not self._peak_targets:
+            self.set_peak_targets(peaks)
         return ds.targets
 
     def loss(self, targets, target_rows=None, loss_kind="mse", want_grad=True):
@@ -404,15 +437,18 @@ class Plan:
 
     def train_step(self, ds: DeviceDataset, ids, fp: FlatParams, step: Step, metrics=None, loss_kind="mse",
                    optimizer=True, num_graphs=None):
+        """K1 + forward + loss + backward [+ AdamW] of one batch of `ds` (a DeviceDataset or a PackedDataset)."""
         n = int(num_graphs if num_graphs is not None else (len(ids) if ids is not None else ds.num_mols))
-        if optimizer:
-            fp.ensure_adam()
-        check(self.lib.eims_train_step(self.h, C.byref(ds.struct), ptr(ids), n, ptr(fp.params), ptr(fp.grads),
-                                       ptr(fp.adam_m) if optimizer else None, ptr(fp.adam_v) if optimizer else None,
-                                       ptr(fp.bn_running), _lib.LOSS[loss_kind], C.byref(step), ptr(metrics), self.stream))
+        check(self.lib.eims_train_step(self.h, C.byref(ds.struct), ptr(ids), n, *fp.step_ptrs(optimizer),
+                                       _lib.LOSS[loss_kind], C.byref(step), ptr(metrics), self.stream))
         self.num_graphs = n
-        for l in range(self.d.num_gcn_layers):
-            fp.num_batches_tracked[l] += 1
+        fp.count_steps()
+
+    def train_step_built(self, ds, ids, fp: FlatParams, step: Step, metrics=None, loss_kind="mse", optimizer=True):
+        """Forward + loss + backward [+ AdamW] on the batch built last; ids: its target rows in `ds` (None: in order)."""
+        check(self.lib.eims_train_step_built(self.h, ptr(self._targets(ds)), ptr(ids), *fp.step_ptrs(optimizer),
+                                             _lib.LOSS[loss_kind], C.byref(step), ptr(metrics), self.stream))
+        fp.count_steps()
 
     def train_step_prefetch(self, ds: DeviceDataset, ids, next_ids, fp: FlatParams, step: Step, metrics=None, loss_kind="mse",
                             optimizer=True, on_head_grads=None):
@@ -429,26 +465,13 @@ class Plan:
             self.batch_build(ds, ids, n)             # cold start: build on the compute stream
         else:
             cur.wait_event(self._built[0])
-        if optimizer:
-            fp.ensure_adam()
         if on_head_grads is None:
-            check(self.lib.eims_train_step_built(self.h, ptr(self._targets(ds)), ptr(ids), ptr(fp.params), ptr(fp.grads),
-                                                 ptr(fp.adam_m) if optimizer else None, ptr(fp.adam_v) if optimizer else None,
-                                                 ptr(fp.bn_running), _lib.LOSS[loss_kind], C.byref(step), ptr(metrics), self.stream))
+            self.train_step_built(ds, ids, fp, step, metrics, loss_kind, optimizer)
+        elif optimizer:
+            raise ValueError("on_head_grads is for the data-parallel path, which runs its own optimiser kernel")
         else:
-            # backward in two parts with a host callback in between (data-parallel bucket overlap)
-            if optimizer:
-                raise ValueError("on_head_grads is for the data-parallel path, which runs its own optimiser kernel")
-            self.forward(fp, True, step)
-            self.loss(self._targets(ds), ids, loss_kind, True)
-            if metrics is not None:
-                self.metrics_accumulate(metrics)
-            check(self.lib.eims_backward_part(self.h, ptr(fp.params), None, ptr(fp.grads), _lib.BWD_HEAD, self.stream))
-            on_head_grads()
-            check(self.lib.eims_backward_part(self.h, ptr(fp.params), None, ptr(fp.grads), _lib.BWD_GCN, self.stream))
+            self._train_split(ds, ids, fp, step, metrics, loss_kind, on_head_grads)
         self.num_graphs = n
-        for l in range(self.d.num_gcn_layers):
-            fp.num_batches_tracked[l] += 1
         end = torch.cuda.Event()
         end.record(cur)
         prev_end, self._step_end = self._step_end[1], [self._step_end[1], end]
@@ -470,6 +493,10 @@ class Plan:
         head and the GCN part of the backward pass (data-parallel bucket overlap, dist.py)."""
         n = int(num_graphs if num_graphs is not None else (len(ids) if ids is not None else ds.num_mols))
         self.batch_build(ds, ids, n)
+        self._train_split(ds, ids, fp, step, metrics, loss_kind, on_head_grads)
+
+    def _train_split(self, ds, ids, fp, step, metrics, loss_kind, on_head_grads):
+        """train_step_split on the batch built last."""
         self.forward(fp, True, step)
         self.loss(self._targets(ds), ids, loss_kind, True)
         if metrics is not None:
@@ -478,8 +505,7 @@ class Plan:
         if on_head_grads is not None:
             on_head_grads()
         check(self.lib.eims_backward_part(self.h, ptr(fp.params), None, ptr(fp.grads), _lib.BWD_GCN, self.stream))
-        for l in range(self.d.num_gcn_layers):
-            fp.num_batches_tracked[l] += 1
+        fp.count_steps()
 
     # -- device step block / CUDA-graph replay (include/eims_b200.h, "one optimiser step as a replayable CUDA graph")
     def enable_step_block(self, count: int = 1):
@@ -513,7 +539,8 @@ class Plan:
 
     def step_block_upload(self, step: Step, ids, dp_seq: int = 0):
         """Rewrite the device step block: AdamW scalars + dropout keys of `step`, the ids the next indirect batch
-        build reads, the data-parallel sequence number.  One 1-block kernel on the current stream."""
+        build reads, the data-parallel sequence number.  One 1-block kernel on the current stream, the one
+        step_blocks_upload launches."""
         check(self.lib.eims_step_block_upload(self.h, C.byref(step), ptr(ids), C.c_uint32(int(dp_seq) & 0xffffffff), self.stream))
 
     def batch_build_indirect(self, ds: DeviceDataset, num_graphs: int):
@@ -522,11 +549,8 @@ class Plan:
 
     def train_step_built_indirect(self, ds: DeviceDataset, fp: FlatParams, metrics=None, loss_kind="mse", optimizer=True, side=None):
         """side: a torch stream for the step's side branch (output-layer bias gradient, AdamW of the head tensors)."""
-        if optimizer:
-            fp.ensure_adam()
-        check(self.lib.eims_train_step_built_indirect(self.h, ptr(self._targets(ds)), ptr(fp.params), ptr(fp.grads),
-                                                      ptr(fp.adam_m) if optimizer else None, ptr(fp.adam_v) if optimizer else None,
-                                                      ptr(fp.bn_running), _lib.LOSS[loss_kind], ptr(metrics), self.stream,
+        check(self.lib.eims_train_step_built_indirect(self.h, ptr(self._targets(ds)), *fp.step_ptrs(optimizer),
+                                                      _lib.LOSS[loss_kind], ptr(metrics), self.stream,
                                                       C.c_void_p(side.cuda_stream) if side is not None else None))
 
     def train_step_built_indirect_part(self, ds: DeviceDataset, fp: FlatParams, part: int, metrics=None, loss_kind="mse"):
@@ -554,7 +578,51 @@ class Plan:
         return out if out is not None else self.buffer("prob", torch.float32, (n, self.d.max_mz))
 
 
-class GraphedTrainStep:
+class StepReplay:
+    """What the replayed training loops (GraphedTrainStep, hostpath.GraphedHostTrainer) share: the enqueue of one step
+    that reads its scalars from a device step block, the capture bracket and the exchange's sequence numbers.
+    Subclasses set plan, fp, metrics, loss_kind, fused (a dist.FusedP2PAdamW or None) and side2."""
+
+    def _enqueue_step(self, ds, block: int, step):
+        """One step on the batch built last, with the scalars of step block `block`: forward, loss, backward and AdamW
+        (the output layer's bias gradient and the head's AdamW on side2), or the fused exchange as the optimiser."""
+        plan, fused = self.plan, self.fused
+        plan.select_step_block(block)
+        if fused is None:
+            plan.train_step_built_indirect(ds, self.fp, self.metrics, self.loss_kind, side=self.side2)
+            return
+        fused.begin_step()
+        blk = plan.step_block_ptr(block)
+        if fused.side is not None:
+            # two buckets: the head's exchange + AdamW (84 % of the parameters) runs on the exchange's side stream under
+            # the GraphConv backward, only the GraphConv bucket is left for the end of the step
+            plan.train_step_built_indirect_part(ds, self.fp, 1, self.metrics, self.loss_kind)
+            fused.head_ready(step, step_block=blk)
+            plan.train_step_built_indirect_part(ds, self.fp, 2, self.metrics, self.loss_kind)
+        else:
+            plan.train_step_built_indirect(ds, self.fp, self.metrics, self.loss_kind, optimizer=False)
+        fused.finish(step, plan.stream, step_block=blk)
+
+    def _capture(self, *bodies):
+        """One CUDA graph per callable, captured in turn.  Capture runs nothing, so the exchange's sequence number is
+        restored at the end: each graph kept the gradient buffer its place in that sequence selected."""
+        seq0 = self.fused.seq if self.fused is not None else 0
+        graphs = []
+        for body in bodies:
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g):
+                body()
+            graphs.append(g)
+        if self.fused is not None:
+            self.fused.seq = seq0
+        return graphs
+
+    def _seqs(self, n: int):
+        """Exchange sequence numbers of the next n replayed steps (0 without the exchange)."""
+        return self.fused.next_seqs(n) if self.fused is not None else [0] * n
+
+
+class GraphedTrainStep(StepReplay):
     """Optimiser steps (GCN:410-431) as replayed CUDA graphs: the host issues one tiny kernel (the step-block upload)
     and one cudaGraphLaunch per GROUP of steps instead of ~30 kernel launches per step, so a descheduled Python thread
     no longer stalls the GPU - which matters most in data-parallel runs, where every rank waits for the slowest one at
@@ -589,26 +657,12 @@ class GraphedTrainStep:
         if fused is None:
             fp.ensure_adam()
 
-    def _enqueue(self, block: int, step_for_fused=None):
-        plan, cur = self.plan, torch.cuda.current_stream(self.plan.device)
-        plan.select_step_block(block)
+    def _enqueue(self, block: int, step):
+        cur = torch.cuda.current_stream(self.plan.device)
         self.side.wait_stream(cur)                       # fork: the build may start with the step
-        if self.fused is not None:
-            self.fused.begin_step()
-        if self.fused is not None and self.fused.side is not None:
-            # two buckets: the head's exchange + AdamW (84 % of the parameters) runs on the exchange's side stream under
-            # the GraphConv backward, only the GraphConv bucket is left for the end of the step
-            blk = plan.step_block_ptr(block)
-            plan.train_step_built_indirect_part(self.ds, self.fp, 1, self.metrics, self.loss_kind)
-            self.fused.head_ready(step_for_fused, step_block=blk)
-            plan.train_step_built_indirect_part(self.ds, self.fp, 2, self.metrics, self.loss_kind)
-            self.fused.finish(step_for_fused, plan.stream, step_block=blk)
-        else:
-            plan.train_step_built_indirect(self.ds, self.fp, self.metrics, self.loss_kind, optimizer=self.fused is None, side=self.side2)
-            if self.fused is not None:
-                self.fused.finish(step_for_fused, plan.stream, step_block=plan.step_block_ptr(block))
+        self._enqueue_step(self.ds, block, step)
         with torch.cuda.stream(self.side):
-            plan.batch_build_indirect(self.ds, self.batch)
+            self.plan.batch_build_indirect(self.ds, self.batch)
         cur.wait_stream(self.side)                       # join
 
     def capture(self, first_ids, step: Step):
@@ -616,44 +670,20 @@ class GraphedTrainStep:
         warm-up steps (module loading and one-time attribute calls must not happen under capture)."""
         plan = self.plan
         plan.select_step_block(0)
-        plan.step_block_upload(step, first_ids, 0)       # also loads the upload kernel before capture
         plan.step_blocks_upload([step], [first_ids], [0], 0)
         plan.batch_build(self.ds, first_ids, self.batch)
         torch.cuda.synchronize(plan.device)
-        seq0 = self.fused.seq if self.fused is not None else 0
-        for _ in range(2):                               # the pair of single-step graphs (block 0)
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                self._enqueue(0, step)
-            self.singles.append(g)
-        if self.fused is not None:
-            self.fused.seq = seq0                        # capture enqueued nothing
+        self.singles = self._capture(lambda: self._enqueue(0, step), lambda: self._enqueue(0, step))   # block 0
         if self.group >= 2:
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                for j in range(self.group):
-                    self._enqueue(j, step)
-            self.multi = g
-            if self.fused is not None:
-                self.fused.seq = seq0
+            self.multi, = self._capture(lambda: [self._enqueue(j, step) for j in range(self.group)])
         plan.select_step_block(0)
         self._keep = [first_ids]
         self.k, self.primed = 0, True
 
-    def _bump(self, n):
-        for l in range(self.plan.d.num_gcn_layers):
-            self.fp.num_batches_tracked[l] += n
-
     def _launch(self, items):
         """items: queued (Step, next_ids); a full group goes out as the multi-step graph (only from table parity 0,
         the one it was captured at), anything else step by step through the single-step graphs."""
-        seqs = []
-        for _ in items:
-            if self.fused is not None:
-                self.fused.seq += 1
-                seqs.append(self.fused.seq)
-            else:
-                seqs.append(0)
+        seqs = self._seqs(len(items))
         self._keep = [ids for _, ids in items]
         if self.multi is not None and len(items) == self.group and self.k == 0:
             prep = self.plan.step_blocks_args([st for st, _ in items], [ids for _, ids in items], seqs)
@@ -667,7 +697,7 @@ class GraphedTrainStep:
                 self.plan.step_blocks_upload([st], [ids], [q], 0)
                 self.singles[self.k].replay()
                 self.k ^= 1
-        self._bump(len(items))
+        self.fp.count_steps(len(items))
 
     def can_hold(self, n_steps: int) -> bool:
         """A full group can be prepared now and launched later with release() (see hold_next)."""

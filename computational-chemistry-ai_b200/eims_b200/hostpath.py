@@ -16,11 +16,18 @@ import torch
 
 from . import _lib
 from ._lib import Dataset, check
+from .engine import PackedDataset, StepReplay
 from .synth import MolTable
 
 
 def _align(n, a=256):
     return (n + a - 1) // a * a
+
+
+def _offsets(lay) -> dict:
+    """Section offsets of an eims_host_batch_layout (a section at -1 is absent)."""
+    return {n: getattr(lay, n) for n in ("node_ptr", "bond_ptr", "bond_begin", "bond_end", "feat", "targets", "peak_ptr",
+                                         "peak_mz", "peak_inten") if getattr(lay, n) >= 0}
 
 
 class PackedHostBatch:
@@ -129,8 +136,7 @@ class HostPacker:
         check(self.lib.eims_host_pack_batch(C.byref(self.hds.struct), C.c_void_p(ids.ctypes.data), len(ids), self.hds.feat_dim,
                                             self.max_mz, C.c_void_p(buf.data_ptr()), buf.numel(), C.byref(lay)))
         hb = PackedHostBatch.__new__(PackedHostBatch)
-        hb.offsets = {n: getattr(lay, n) for n in ("node_ptr", "bond_ptr", "bond_begin", "bond_end", "feat", "targets", "peak_ptr",
-                                                   "peak_mz", "peak_inten") if getattr(lay, n) >= 0}
+        hb.offsets = _offsets(lay)
         hb.nbytes, hb.buf, hb.mz_is_f64 = int(lay.nbytes), buf, int(lay.mz_is_f64)
         hb.num_graphs, hb.num_nodes, hb.num_edges, hb.feat_dim = lay.num_graphs, lay.num_nodes, lay.num_edges, lay.feat_dim
         hb.has_targets, hb.has_peaks = lay.targets >= 0, lay.peak_ptr >= 0
@@ -164,17 +170,8 @@ class HostBatchRunner:
         self.d2h_bytes = 0
         self._i = 0
 
-    def _dataset(self, slot, hb: PackedHostBatch) -> Dataset:
-        base = self.slots[slot].data_ptr()
-        o = hb.offsets
-        pk = None
-        if hb.has_peaks:
-            pk = _lib.Peaks(base + o["peak_ptr"], base + o["peak_mz"], base + o["peak_inten"], hb.mz_is_f64, hb.num_graphs)
-        ds = Dataset(base + o["node_ptr"], base + o["bond_ptr"], base + o["feat"], base + o["bond_begin"],
-                     base + o["bond_end"], (base + o["targets"]) if hb.has_targets else None, hb.num_graphs,
-                     C.pointer(pk) if pk is not None else None)
-        ds._peaks_keepalive = pk
-        return ds
+    def _dataset(self, slot, hb: PackedHostBatch) -> PackedDataset:
+        return PackedDataset(self.slots[slot].data_ptr(), hb.offsets, hb.num_graphs, hb.mz_is_f64)
 
     def upload(self, hb: PackedHostBatch, build: bool = False):
         """Enqueue the H2D copy of `hb` (and, with build=True, its K1 batch build) on the copy
@@ -192,9 +189,7 @@ class HostBatchRunner:
             if build:
                 # K1 on the copy stream: the table set it overwrites was last read by the step that
                 # consumed this slot, which the wait above already covers
-                ds = self._dataset(slot, hb)
-                check(self.plan.lib.eims_batch_build(self.plan.h, C.byref(ds), None, hb.num_graphs,
-                                                     C.c_void_p(self.copy_stream.cuda_stream)))
+                self.plan.batch_build(self._dataset(slot, hb), None, hb.num_graphs)
             self.built[slot] = build
             self.copied[slot].record(self.copy_stream)
             if getattr(hb, "_ring_event", None) is not None:
@@ -212,23 +207,10 @@ class HostBatchRunner:
         cur = torch.cuda.current_stream(self.plan.device)
         cur.wait_event(self.copied[slot])
         ds = self._dataset(slot, hb)
-        self.fp.ensure_adam()
-        fp = self.fp
         if self.built[slot]:
-            # targets as peak lists: point the plan at this slot's arrays (the struct is copied)
-            check(self.plan.lib.eims_plan_set_peak_targets(self.plan.h, ds.peaks if hb.has_peaks else None))
-            self.plan._peak_targets = None
-            check(self.plan.lib.eims_train_step_built(self.plan.h, C.c_void_p(ds.targets), None, _lib.ptr(fp.params),
-                                                      _lib.ptr(fp.grads), _lib.ptr(fp.adam_m) if optimizer else None,
-                                                      _lib.ptr(fp.adam_v) if optimizer else None, _lib.ptr(fp.bn_running),
-                                                      _lib.LOSS[loss_kind], C.byref(step), _lib.ptr(self.metrics),
-                                                      self.plan.stream))
+            self.plan.train_step_built(ds, None, self.fp, step, self.metrics, loss_kind, optimizer)
         else:
-            check(self.plan.lib.eims_train_step(self.plan.h, C.byref(ds), None, hb.num_graphs, _lib.ptr(fp.params),
-                                                _lib.ptr(fp.grads), _lib.ptr(fp.adam_m) if optimizer else None,
-                                                _lib.ptr(fp.adam_v) if optimizer else None,
-                                                _lib.ptr(fp.bn_running), _lib.LOSS[loss_kind], C.byref(step),
-                                                _lib.ptr(self.metrics), self.plan.stream))
+            self.plan.train_step(ds, None, self.fp, step, self.metrics, loss_kind, optimizer, num_graphs=hb.num_graphs)
         ev = torch.cuda.Event()
         ev.record(cur)
         self.consumed[slot] = ev
@@ -237,20 +219,14 @@ class HostBatchRunner:
         self.d2h_done[k].record(cur)
         self._n += 1
         self.d2h_bytes += self.metrics.numel() * 4
-        for l in range(self.plan.d.num_gcn_layers):
-            fp.num_batches_tracked[l] += 1
 
     def infer(self, slot, hb: PackedHostBatch, out_host: torch.Tensor):
         cur = torch.cuda.current_stream(self.plan.device)
         cur.wait_event(self.copied[slot])
-        ds = self._dataset(slot, hb)
-        fp = self.fp
-        check(self.plan.lib.eims_infer_batch(self.plan.h, C.byref(ds), None, hb.num_graphs, _lib.ptr(fp.params),
-                                             _lib.ptr(fp.bn_running), None, self.plan.stream))
+        prob = self.plan.infer_batch(self._dataset(slot, hb), None, self.fp, num_graphs=hb.num_graphs)
         ev = torch.cuda.Event()
         ev.record(cur)
         self.consumed[slot] = ev
-        prob = self.plan.buffer("prob", torch.float32, (hb.num_graphs, self.plan.d.max_mz))
         out_host[:hb.num_graphs].copy_(prob, non_blocking=True)
         self.d2h_bytes += prob.numel() * 4
 
@@ -268,7 +244,7 @@ class HostBatchRunner:
         return self.read(0)
 
 
-class GraphedHostTrainer:
+class GraphedHostTrainer(StepReplay):
     """Training steps fed from HOST-resident data, replayed as CUDA graphs: per step the graph holds the H2D copy of
     the NEXT batch from a pinned ring buffer into one of two device slots + its K1 batch build (copy stream), the step
     itself on the batch built one step earlier (forward, loss, backward, AdamW or the fused data-parallel exchange),
@@ -308,15 +284,7 @@ class GraphedHostTrainer:
         self.pool = ThreadPoolExecutor(max(1, int(workers)))
         self.h2d_bytes = self.d2h_bytes = 0
         self.graphs, self.done, self.launches = [], {}, 0
-        self._ds, self._pk = [], []
-        for s in range(2):
-            base = self.slots[s].data_ptr()
-            pk = None
-            if lay.peak_ptr >= 0:
-                pk = _lib.Peaks(base + lay.peak_ptr, base + lay.peak_mz, base + lay.peak_inten, lay.mz_is_f64, self.batch)
-            self._pk.append(pk)
-            self._ds.append(Dataset(base + lay.node_ptr, base + lay.bond_ptr, base + lay.feat, base + lay.bond_begin, base + lay.bond_end,
-                                    (base + lay.targets) if lay.targets >= 0 else None, self.batch, C.pointer(pk) if pk is not None else None))
+        self._ds = [PackedDataset(s.data_ptr(), _offsets(lay), self.batch, lay.mz_is_f64) for s in self.slots]
         plan.enable_step_block(self.G)
         if fused is None:
             fp.ensure_adam()
@@ -342,43 +310,20 @@ class GraphedHostTrainer:
         """Batch 0 (already submitted with pack_async) is uploaded and built eagerly on the current stream."""
         fut0.result()
         self.slots[0].copy_(self.pinned[0], non_blocking=True)
-        check(self.lib.eims_batch_build(self.plan.h, C.byref(self._ds[0]), None, self.batch, self.plan.stream))
+        self.plan.batch_build(self._ds[0], None, self.batch)
         self.h2d_bytes += self.nbytes
 
     def _enqueue(self, n_local: int, block: int, step):
-        plan, cur = self.plan, torch.cuda.current_stream(self.plan.device)
+        cur = torch.cuda.current_stream(self.plan.device)
         slot, nxt = n_local % 2, (n_local + 1) % 2
-        plan.select_step_block(block)
         self.copy_stream.wait_stream(cur)            # the next batch's slot was last read by the previous step: fork here
-        if self.fused is not None:
-            self.fused.begin_step()
-        check(self.lib.eims_plan_set_peak_targets(plan.h, C.byref(self._pk[slot]) if self._pk[slot] is not None else None))
-        plan._peak_targets = None
-        fp, opt = self.fp, self.fused is None
-        tgt = self._ds[slot].targets
-        if self.fused is not None and self.fused.side is not None:
-            # data-parallel, two buckets: the head's exchange runs on the exchange's side stream under the GraphConv backward
-            blk = plan.step_block_ptr(block)
-            for part in (1, 2):
-                check(self.lib.eims_train_step_built_indirect_part(plan.h, C.c_void_p(tgt) if tgt else None, _lib.ptr(fp.params),
-                                                                   _lib.ptr(fp.grads), _lib.ptr(fp.bn_running), _lib.LOSS[self.loss_kind],
-                                                                   _lib.ptr(self.metrics), part, plan.stream))
-                if part == 1:
-                    self.fused.head_ready(step, step_block=blk)
-            self.fused.finish(step, plan.stream, step_block=blk)
-        else:
-            check(self.lib.eims_train_step_built_indirect(plan.h, C.c_void_p(tgt) if tgt else None, _lib.ptr(fp.params), _lib.ptr(fp.grads),
-                                                          _lib.ptr(fp.adam_m) if opt else None, _lib.ptr(fp.adam_v) if opt else None,
-                                                          _lib.ptr(fp.bn_running), _lib.LOSS[self.loss_kind], _lib.ptr(self.metrics), plan.stream,
-                                                          C.c_void_p(self.side2.cuda_stream) if self.side2 is not None else None))
-            if self.fused is not None:
-                self.fused.finish(step, plan.stream, step_block=plan.step_block_ptr(block))
+        self._enqueue_step(self._ds[slot], block, step)
         self.out_host[n_local].copy_(self.metrics, non_blocking=True)      # the step's loss / cosine back to the host
         with torch.cuda.stream(self.copy_stream):
             self.slots[nxt].copy_(self.pinned[(n_local + 1) % (2 * self.G)], non_blocking=True)
             # indirect: K1 takes its sequence number (the zero-degree tag) from the step block, so every replay tags its
             # batches anew; a number baked in at capture would repeat every other launch
-            check(self.lib.eims_batch_build_indirect(plan.h, C.byref(self._ds[nxt]), self.batch, C.c_void_p(self.copy_stream.cuda_stream)))
+            self.plan.batch_build_indirect(self._ds[nxt], self.batch)
         cur.wait_stream(self.copy_stream)            # join
 
     def capture(self, step):
@@ -387,15 +332,11 @@ class GraphedHostTrainer:
         plan.select_step_block(0)
         plan.step_blocks_upload([step], [None], [0], 0)   # loads the upload kernel; ids None: K1 reads the slot in order
         torch.cuda.synchronize(plan.device)
-        seq0 = self.fused.seq if self.fused is not None else 0
-        for s in range(2):
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                for j in range(self.G):
-                    self._enqueue(s * self.G + j, j, step)
-            self.graphs.append(g)
-        if self.fused is not None:
-            self.fused.seq = seq0
+
+        def group(s):
+            for j in range(self.G):
+                self._enqueue(s * self.G + j, j, step)
+        self.graphs = self._capture(lambda: group(0), lambda: group(1))
         plan.select_step_block(0)
 
     def launch(self, steps, futures):
@@ -405,14 +346,7 @@ class GraphedHostTrainer:
         for f in futures:
             f.result()
         l = self.launches
-        seqs = []
-        for _ in steps:
-            if self.fused is not None:
-                self.fused.seq += 1
-                seqs.append(self.fused.seq)
-            else:
-                seqs.append(0)
-        self.plan.step_blocks_upload(list(steps), [None] * self.G, seqs, 0)
+        self.plan.step_blocks_upload(list(steps), [None] * self.G, self._seqs(self.G), 0)
         self.graphs[l % 2].replay()
         ev = torch.cuda.Event()
         ev.record(torch.cuda.current_stream(self.plan.device))
@@ -421,8 +355,7 @@ class GraphedHostTrainer:
         self.launches += 1
         self.h2d_bytes += self.G * self.nbytes
         self.d2h_bytes += self.G * 32
-        for k in range(self.plan.d.num_gcn_layers):
-            self.fp.num_batches_tracked[k] += self.G
+        self.fp.count_steps(self.G)
         return l
 
     def results(self, l: int):

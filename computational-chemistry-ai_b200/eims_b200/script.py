@@ -420,24 +420,18 @@ class GCNSpectrum(nn.Module):
         return self._plan, self._fp
 
     def _run_forward(self, g, training, targets=None):
-        from .engine import Dataset
+        from .engine import PackedDataset
         if isinstance(g, MolGraph):
             g = g.to(self.flat.device)
         if g._dev_buf is None:
             g = g.to(self.flat.device)
         plan, fp = self._engine(g.batch_size, g.num_nodes(), g.num_edges())
-        hb, base = g._packed, g._dev_buf.data_ptr()
-        o = hb.offsets
-        ds = Dataset(base + o["node_ptr"], base + o["bond_ptr"], base + o["feat"], base + o["bond_begin"],
-                     base + o["bond_end"], None, hb.num_graphs)
+        hb = g._packed
         self._keep = g  # the packed batch must outlive the asynchronous kernels
-        import ctypes as C
-        _lib.check(plan.lib.eims_batch_build(plan.h, C.byref(ds), None, hb.num_graphs, plan.stream))
-        plan.num_graphs = hb.num_graphs
+        plan.batch_build(PackedDataset(g._dev_buf.data_ptr(), hb.offsets, hb.num_graphs), None, hb.num_graphs)
         if training:
             self._step += 1
-            for l in range(self.dims.num_gcn_layers):
-                self.num_batches_tracked[l] += 1
+            fp.count_steps()
         plan.forward(fp, training, make_step(step=self._step, seed=self._seed))
         plan.sigmoid()
         plan.check()  # raises ZeroInDegreeError like DGL's GraphConv
