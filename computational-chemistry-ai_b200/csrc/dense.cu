@@ -174,21 +174,25 @@ int launch_bn_stats(const int* dims, const float* z, int H, const float* gamma, 
   return 0;
 }
 
-// eval-mode coefficients from the running buffers (GCN:442, model.eval()):
+// eval-mode coefficients from the running buffers (GCN:442, model.eval()); mean / invstd (optional): the running
+// mean and 1/sqrt(running_var + eps), which the eval-mode BatchNorm backward uses as its statistics
 __global__ void bn_eval_coeffs_kernel(const float* __restrict__ gamma, const float* __restrict__ beta,
                                       const float* __restrict__ rmean, const float* __restrict__ rvar, int H,
-                                      float* __restrict__ scale, float* __restrict__ shift) {
+                                      float* __restrict__ scale, float* __restrict__ shift, float* __restrict__ mean,
+                                      float* __restrict__ invstd_out) {
   pdl_sync();
   for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < H; c += gridDim.x * blockDim.x) {
     float invstd = 1.f / sqrtf(rvar[c] + kBnEps);
     float sc = gamma[c] * invstd;
     scale[c] = sc;
     shift[c] = fmaf(-rmean[c], sc, beta[c]);
+    if (mean) { mean[c] = rmean[c]; invstd_out[c] = invstd; }
   }
 }
 int launch_bn_eval_coeffs(const float* gamma, const float* beta, const float* rmean, const float* rvar, int H,
-                          float* scale, float* shift, cudaStream_t st) {
-  launch_pdl(bn_eval_coeffs_kernel, dim3((H + 255) / 256), dim3(256), 0, st, gamma, beta, rmean, rvar, H, scale, shift);
+                          float* scale, float* shift, cudaStream_t st, float* mean, float* invstd) {
+  if (!mean != !invstd) return EIMS_ERR_ARG;
+  launch_pdl(bn_eval_coeffs_kernel, dim3((H + 255) / 256), dim3(256), 0, st, gamma, beta, rmean, rvar, H, scale, shift, mean, invstd);
   return 0;
 }
 
@@ -227,7 +231,9 @@ __device__ __forceinline__ float4 load_dh(const DhSrc& s, int i, int c, int H) {
   return v;
 }
 
-// pass 1: column sums of dh and dh*xhat (fp64) -> dgamma, dbeta (into grads) and the two column means.
+// pass 1: column sums of dh and dh*xhat (fp64) -> dgamma, dbeta (into grads) and the two column means (means == NULL:
+// not written - eval mode, where BatchNorm's output does not depend on the batch statistics and the apply pass takes
+// zero means).
 __global__ void __launch_bounds__(256, 4) bn_bwd_stats_kernel(const int* __restrict__ dims, const float* __restrict__ dh,
                                                            const float* __restrict__ z, int H,
                                                            const float* __restrict__ mean, const float* __restrict__ invstd,
@@ -262,8 +268,10 @@ __global__ void __launch_bounds__(256, 4) bn_bwd_stats_kernel(const int* __restr
     const double sa = bn_acc_take(acc, H, 0, k), sb = bn_acc_take(acc, H, 1, k);
     dbeta[k] += (float)sa;
     dgamma[k] += (float)sb;
-    means[k] = N > 0 ? (float)(sa / N) : 0.f;
-    means[H + k] = N > 0 ? (float)(sb / N) : 0.f;
+    if (means) {
+      means[k] = N > 0 ? (float)(sa / N) : 0.f;
+      means[H + k] = N > 0 ? (float)(sb / N) : 0.f;
+    }
   }
 }
 
@@ -314,9 +322,50 @@ __global__ void __launch_bounds__(256) bn_bwd_stats_top_kernel(const int* __rest
     const double sa = bn_acc_take(acc, H, 0, k), sb = bn_acc_take(acc, H, 1, k);
     dbeta[k] += (float)sa;
     dgamma[k] += (float)sb;
-    means[k] = N > 0 ? (float)(sa / N) : 0.f;
-    means[H + k] = N > 0 ? (float)(sb / N) : 0.f;
+    if (means) {
+      means[k] = N > 0 ? (float)(sa / N) : 0.f;
+      means[H + k] = N > 0 ? (float)(sb / N) : 0.f;
+    }
   }
+}
+
+// zstat of an eval-mode forward, whose readout writes none: per graph, the column sums of z - mean (sum / mean
+// pooling) and z - mean at the arg-max node (max pooling), mean = the running mean.  Thread = (graph, column quad).
+__global__ void __launch_bounds__(256) bn_eval_zstat_kernel(const int* __restrict__ dims, const int* __restrict__ gptr,
+                                                            const float* __restrict__ z, int H, const float* __restrict__ mean,
+                                                            const int* __restrict__ argmax, int pooling,
+                                                            float* __restrict__ zstat, int early) {
+  const int B = pdl_sync_dims(dims, early).B;
+  const int q4 = H >> 2;
+  for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < (int64_t)B * q4; t += (int64_t)gridDim.x * blockDim.x) {
+    const int g = (int)(t / q4), c = (int)(t % q4) * 4;
+    const int r0 = __ldg(gptr + g), r1 = __ldg(gptr + g + 1);
+    const float4 mu = ldg4(mean + c);
+    float* zo = zstat + (int64_t)g * 2 * H;
+    if (pooling != EIMS_POOL_MAX) {
+      float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
+      for (int i = r0; i < r1; ++i) {
+        const float4 v = ldg4(z + (int64_t)i * H + c);
+        s.x += v.x - mu.x; s.y += v.y - mu.y; s.z += v.z - mu.z; s.w += v.w - mu.w;
+      }
+      st4(zo + c, s);
+    }
+    if ((pooling == EIMS_POOL_MAX || pooling == EIMS_POOL_COMBINED) && r1 > r0) {
+      const int4 a = *reinterpret_cast<const int4*>(argmax + (int64_t)g * H + c);
+      st4(zo + H + c, make_float4(__ldg(z + (int64_t)a.x * H + c) - mu.x, __ldg(z + (int64_t)a.y * H + c + 1) - mu.y,
+                                  __ldg(z + (int64_t)a.z * H + c + 2) - mu.z, __ldg(z + (int64_t)a.w * H + c + 3) - mu.w));
+    }
+  }
+}
+
+int launch_bn_eval_zstat(const int* dims, const int* gptr, const float* z, int H, const float* mean, const int* argmax,
+                         int pooling, float* zstat, int max_graphs, cudaStream_t st) {
+  if (H % 4 || H > 4096) return EIMS_ERR_ARG;
+  int64_t blocks = ((int64_t)max_graphs * (H / 4) + 255) / 256;
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  launch_pdl(bn_eval_zstat_kernel, dim3(blocks < 1 ? 1 : (int)blocks), dim3(256), 0, st, dims, gptr, z, H, mean,
+             argmax, pooling, zstat, dims_early_ref());
+  return 0;
 }
 
 int launch_bn_bwd_stats_top(const int* dims, const float* dG, const float* zstat, const int* gptr, int pooling, int H,
@@ -337,13 +386,14 @@ int launch_bn_bwd_stats_top(const int* dims, const float* dG, const float* zstat
 }
 
 // pass 2: q = gamma*invstd*(dh - mean(dh) - xhat*mean(dh*xhat)) * [z>0] * c_i ;  dbias += colsum(dr)
-// LAYER0: the first GraphConv has no input gradient, so q is consumed on the spot by its weight
-// gradient dW0[f,k] += sum_i a0[i,f] * q[i,k] (F <= 8 rows) and never written.
+// LAYER0: q is consumed on the spot by the first GraphConv's weight gradient dW0[f,k] += sum_i a0[i,f] * q[i,k]
+// (F <= 8 rows); it is written (plain fp32) only when STORE_Q0, i.e. when the gradient w.r.t. the atom features is
+// wanted (bn_bwd_apply_q0_kernel), and never by bn_bwd_apply_kernel<true>.
 constexpr int kMaxF0d = 8;
 
-template <bool LAYER0>
-__global__ void __launch_bounds__(256, LAYER0 ? 2 : 4) bn_bwd_apply_kernel(
-    const int* __restrict__ dims, DhSrc src, const float* __restrict__ z, int H, const float* __restrict__ mean,
+template <bool LAYER0, bool STORE_Q0>
+__device__ __forceinline__ void bn_bwd_apply_body(
+    const int* __restrict__ dims, const DhSrc& src, const float* __restrict__ z, int H, const float* __restrict__ mean,
     const float* __restrict__ invstd, const float* __restrict__ gamma, const float* __restrict__ means,
     const float* __restrict__ norm, float* __restrict__ q, float* __restrict__ dbias, const float* __restrict__ a0,
     int F, float* __restrict__ dW0, int early, int64_t q_lo_off) {
@@ -379,6 +429,7 @@ __global__ void __launch_bounds__(256, LAYER0 ? 2 : 4) bn_bwd_apply_kernel(
             w[f].x = fmaf(a, o.x, w[f].x); w[f].y = fmaf(a, o.y, w[f].y);
             w[f].z = fmaf(a, o.z, w[f].z); w[f].w = fmaf(a, o.w, w[f].w);
           }
+        if (STORE_Q0) st4(q + (int64_t)r * H + c, o);
       } else if (q_lo_off) {  // q as stacked tf32 hi / lo planes: the operand layout of gemm_tma.cu
         float4 hi4, lo4;
         split_tf32_planes4(o, hi4, lo4);
@@ -422,6 +473,24 @@ __global__ void __launch_bounds__(256, LAYER0 ? 2 : 4) bn_bwd_apply_kernel(
   }
 }
 
+template <bool LAYER0>
+__global__ void __launch_bounds__(256, LAYER0 ? 2 : 4) bn_bwd_apply_kernel(
+    const int* __restrict__ dims, DhSrc src, const float* __restrict__ z, int H, const float* __restrict__ mean,
+    const float* __restrict__ invstd, const float* __restrict__ gamma, const float* __restrict__ means,
+    const float* __restrict__ norm, float* __restrict__ q, float* __restrict__ dbias, const float* __restrict__ a0,
+    int F, float* __restrict__ dW0, int early, int64_t q_lo_off) {
+  bn_bwd_apply_body<LAYER0, false>(dims, src, z, H, mean, invstd, gamma, means, norm, q, dbias, a0, F, dW0, early, q_lo_off);
+}
+
+// layer 0 when the gradient w.r.t. the atom features is wanted: the same pass, and q_0 = c * (dz_0 * relu') stored
+__global__ void __launch_bounds__(256, 2) bn_bwd_apply_q0_kernel(
+    const int* __restrict__ dims, DhSrc src, const float* __restrict__ z, int H, const float* __restrict__ mean,
+    const float* __restrict__ invstd, const float* __restrict__ gamma, const float* __restrict__ means,
+    const float* __restrict__ norm, float* __restrict__ q, float* __restrict__ dbias, const float* __restrict__ a0,
+    int F, float* __restrict__ dW0, int early) {
+  bn_bwd_apply_body<true, true>(dims, src, z, H, mean, invstd, gamma, means, norm, q, dbias, a0, F, dW0, early, 0);
+}
+
 int launch_bn_bwd_stats(const int* dims, const float* dh, const float* z, int H, const float* mean, const float* invstd,
                         float* dgamma, float* dbeta, float* means, float* partials, int max_nodes, cudaStream_t st) {
   if (H % 4 || H > 4096) return EIMS_ERR_ARG;
@@ -433,13 +502,16 @@ int launch_bn_bwd_stats(const int* dims, const float* dh, const float* z, int H,
 int launch_bn_bwd_apply(const int* dims, const float* dh, const float* dG, const int* gid, const int* gptr,
                         const int* argmax, int pooling, const float* z, int H, const float* mean, const float* invstd,
                         const float* gamma, const float* norm, float* dbias, const float* means, float* q, int max_nodes,
-                        cudaStream_t st, const float* a0, int F, float* dW0, int64_t q_lo_off) {
-  if (H % 4 || H > 4096 || (dW0 && (F < 1 || F > kMaxF0d)) || (q_lo_off & 3) || (dW0 && q_lo_off)) return EIMS_ERR_ARG;
+                        cudaStream_t st, const float* a0, int F, float* dW0, int64_t q_lo_off, bool store_q0) {
+  if (H % 4 || H > 4096 || (dW0 && (F < 1 || F > kMaxF0d)) || (q_lo_off & 3) || (dW0 && q_lo_off) || (store_q0 && !dW0))
+    return EIMS_ERR_ARG;
   const DhSrc src{dh, dG, gid, gptr, argmax, pooling};
   const dim3 grid = bn_grid(H, max_nodes);
   // the layer-0 variant (104 registers: two resident blocks per SM) is launched as one wave: 12.7 us against 16.3
   constexpr int kL0BlocksPerSm = 2;
-  if (dW0)
+  if (store_q0)
+    launch_pdl(bn_bwd_apply_q0_kernel, bn_grid(H, max_nodes, kL0BlocksPerSm), dim3(256), 0, st, dims, src, z, H, mean, invstd, gamma, means, norm, q, dbias, a0, F, dW0, dims_early_ref());
+  else if (dW0)
     launch_pdl(bn_bwd_apply_kernel<true>, bn_grid(H, max_nodes, kL0BlocksPerSm), dim3(256), 0, st, dims, src, z, H, mean, invstd, gamma, means, norm, q, dbias, a0, F, dW0, dims_early_ref(), (int64_t)0);
   else
     launch_pdl(bn_bwd_apply_kernel<false>, grid, dim3(256), 0, st, dims, src, z, H, mean, invstd, gamma, means, norm, q, dbias, nullptr, 0, nullptr, dims_early_ref(), q_lo_off);

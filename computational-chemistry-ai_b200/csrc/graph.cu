@@ -413,6 +413,88 @@ int launch_layer0_fwd(const int* dims, const float* norm, const float* a0, int F
   return 0;
 }
 
+// --------------------------------------------------------------------------- layer 0 backward to the atom features
+// a0 = A D x and z0 = relu(D a0 W0 + b0), so with q0 = D (dz0 * relu') (the BatchNorm-backward apply pass stores it):
+//   da0 = q0 W0^T   [N, F]                      (layer0_dgrad_kernel: warp per row, W0 staged in shared memory)
+//   dx  = D A^T da0 = D A da0                  (feat_grad_kernel: every bond gives both directed edges, so A^T = A
+//                                               and K1's CSR by destination is also the CSR by source)
+__global__ void __launch_bounds__(256) layer0_dgrad_kernel(const int* __restrict__ dims, const float* __restrict__ q, int H,
+                                                           const float* __restrict__ W0, int F, float* __restrict__ da0,
+                                                           int early) {
+  extern __shared__ __align__(16) float sw[];  // W0 [F][H]
+  const int N = pdl_sync_dims(dims, early).N;
+  for (int t = threadIdx.x; t < F * H; t += blockDim.x) sw[t] = __ldg(W0 + t);
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int nwarps = (gridDim.x * blockDim.x) >> 5;
+  for (int i = warp; i < N; i += nwarps) {
+    float acc[kMaxF0];
+#pragma unroll
+    for (int f = 0; f < kMaxF0; ++f) acc[f] = 0.f;
+    for (int c = lane * 4; c < H; c += 128) {
+      const float4 v = ldg4(q + (int64_t)i * H + c);
+#pragma unroll
+      for (int f = 0; f < kMaxF0; ++f)
+        if (f < F) {
+          const float4 w = *reinterpret_cast<const float4*>(sw + f * H + c);
+          acc[f] = fmaf(v.x, w.x, fmaf(v.y, w.y, fmaf(v.z, w.z, fmaf(v.w, w.w, acc[f]))));
+        }
+    }
+    float mine = 0.f;
+#pragma unroll
+    for (int f = 0; f < kMaxF0; ++f)
+      if (f < F) {
+        const float s = warp_sum(acc[f]);
+        if (lane == f) mine = s;
+      }
+    if (lane < F) da0[(int64_t)i * F + lane] = mine;
+  }
+}
+
+__global__ void __launch_bounds__(256) feat_grad_kernel(const int* __restrict__ dims, const int* __restrict__ rowptr,
+                                                        const int* __restrict__ col, const float* __restrict__ norm,
+                                                        const float* __restrict__ da0, int F, float* __restrict__ dx,
+                                                        int early) {
+  const int N = pdl_sync_dims(dims, early).N;
+  for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < N; j += gridDim.x * blockDim.x) {
+    float acc[kMaxF0];
+#pragma unroll
+    for (int f = 0; f < kMaxF0; ++f) acc[f] = 0.f;
+    const int e0 = __ldg(rowptr + j), e1 = __ldg(rowptr + j + 1);
+    for (int e = e0; e < e1; ++e) {
+      const int i = __ldg(col + e);
+#pragma unroll
+      for (int f = 0; f < kMaxF0; ++f)
+        if (f < F) acc[f] += __ldg(da0 + (int64_t)i * F + f);
+    }
+    const float cj = __ldg(norm + j);
+#pragma unroll
+    for (int f = 0; f < kMaxF0; ++f)
+      if (f < F) dx[(int64_t)j * F + f] = acc[f] * cj;
+  }
+}
+
+int launch_layer0_dgrad(const int* dims, const float* q0, int H, const float* W0, int F, float* da0, int max_nodes,
+                        cudaStream_t st) {
+  if (F < 1 || F > kMaxF0 || H % 4 || H > 1024) return EIMS_ERR_ARG;
+  int blocks = (max_nodes + 7) / 8;  // 8 warps, one row each
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  launch_pdl(layer0_dgrad_kernel, dim3(blocks < 1 ? 1 : blocks), dim3(256), (size_t)F * H * sizeof(float), st, dims, q0, H,
+             W0, F, da0, dims_early_ref());
+  return 0;
+}
+
+int launch_feat_grad(const int* dims, const int* rowptr, const int* col, const float* norm, const float* da0, int F,
+                     float* dx, int max_nodes, cudaStream_t st) {
+  if (F < 1 || F > kMaxF0) return EIMS_ERR_ARG;
+  int blocks = (max_nodes + 255) / 256;
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  launch_pdl(feat_grad_kernel, dim3(blocks < 1 ? 1 : blocks), dim3(256), 0, st, dims, rowptr, col, norm, da0, F, dx,
+             dims_early_ref());
+  return 0;
+}
+
 // ------------------------------------------------------------------------------------ K2
 // Warp per destination row; lane owns NV float4 column groups (columns (i*32+lane)*4), so a
 // whole row of H <= 128*NV floats is gathered by one warp-wide 128-bit load per neighbour and
@@ -589,8 +671,10 @@ __global__ void __launch_bounds__(256) spmm_norm_kernel(const int* __restrict__ 
       }
       bf.dbeta[k] += (float)sa;
       bf.dgamma[k] += (float)sb;
-      bf.means[k] = N > 0 ? (float)(sa / N) : 0.f;
-      bf.means[H + k] = N > 0 ? (float)(sb / N) : 0.f;
+      if (bf.means) {  // NULL in eval mode (see bn_bwd_stats_kernel)
+        bf.means[k] = N > 0 ? (float)(sa / N) : 0.f;
+        bf.means[H + k] = N > 0 ? (float)(sb / N) : 0.f;
+      }
     }
   }
 }
@@ -845,8 +929,10 @@ __global__ void __launch_bounds__(THREADS) spmm_mol_kernel(const int* __restrict
       }
       bf.dbeta[k] += (float)sa;
       bf.dgamma[k] += (float)sb;
-      bf.means[k] = N > 0 ? (float)(sa / N) : 0.f;
-      bf.means[H + k] = N > 0 ? (float)(sb / N) : 0.f;
+      if (bf.means) {  // NULL in eval mode (see bn_bwd_stats_kernel)
+        bf.means[k] = N > 0 ? (float)(sa / N) : 0.f;
+        bf.means[H + k] = N > 0 ? (float)(sb / N) : 0.f;
+      }
     }
   }
 }

@@ -33,6 +33,11 @@ int launch_spmm_norm(const int* dims, const int* rowptr, const int* col, const f
 int launch_spmm_mol(const int* dims, const int* gptr, const int* rowptr, const int* col, const float* norm, const float* h, int H,
                     const float* bn_scale, const float* bn_shift, DropCfg drop, int out_mode, float* out, int max_graphs,
                     int tile_rows, cudaStream_t st, const BnBwdFuse* bf, int64_t lo_off = 0);
+// gradient w.r.t. the atom features: da0 = q0 W0^T ([N, F], q0 from launch_bn_bwd_apply(store_q0)), then dx = D A da0
+int launch_layer0_dgrad(const int* dims, const float* q0, int H, const float* W0, int F, float* da0, int max_nodes,
+                        cudaStream_t st);
+int launch_feat_grad(const int* dims, const int* rowptr, const int* col, const float* norm, const float* da0, int F,
+                     float* dx, int max_nodes, cudaStream_t st);
 int launch_readout(const int* dims, const int* gptr, const float* z, int H, const float* bn_scale,
                    const float* bn_shift, int pooling, float* out, int* argmax, int max_graphs, cudaStream_t st,
                    float* zstat = nullptr, const float* bn_mean = nullptr);  // zstat [B][2H]: per graph, column sums of
@@ -47,18 +52,24 @@ int launch_bn_stats(const int* dims, const float* z, int H, const float* gamma, 
                     float* rvar, float* mean, float* invstd, float* scale, float* shift, float* partials,
                     int max_nodes, cudaStream_t st);
 int launch_bn_eval_coeffs(const float* gamma, const float* beta, const float* rmean, const float* rvar, int H,
-                          float* scale, float* shift, cudaStream_t st);
+                          float* scale, float* shift, cudaStream_t st,
+                          float* mean = nullptr, float* invstd = nullptr);  // also: running mean, 1/sqrt(running_var + eps)
+// means (the two column means the apply pass subtracts) may be NULL in the statistics passes below: eval mode
 int launch_bn_bwd_stats(const int* dims, const float* dh, const float* z, int H, const float* mean, const float* invstd,
                         float* dgamma, float* dbeta, float* means, float* partials, int max_nodes, cudaStream_t st);
 // statistics of the TOP layer's BatchNorm backward from per-graph quantities (O(B*H) instead of O(N*H))
 int launch_bn_bwd_stats_top(const int* dims, const float* dG, const float* zstat, const int* gptr, int pooling, int H,
                             const float* mean, const float* invstd, float* dgamma, float* dbeta, float* means,
                             float* partials, int max_graphs, cudaStream_t st);
+// the zstat [B][2H] that launch_bn_bwd_stats_top reads, for an eval-mode forward (mean: the running mean)
+int launch_bn_eval_zstat(const int* dims, const int* gptr, const float* z, int H, const float* mean, const int* argmax,
+                         int pooling, float* zstat, int max_graphs, cudaStream_t st);
 int launch_bn_bwd_apply(const int* dims, const float* dh, const float* dG, const int* gid, const int* gptr,
                         const int* argmax, int pooling, const float* z, int H, const float* mean, const float* invstd,
                         const float* gamma, const float* norm, float* dbias, const float* means, float* q, int max_nodes,
                         cudaStream_t st, const float* a0 = nullptr, int F = 0, float* dW0 = nullptr,
-                        int64_t q_lo_off = 0);  // != 0: q as stacked tf32 hi / lo planes
+                        int64_t q_lo_off = 0,     // != 0: q as stacked tf32 hi / lo planes
+                        bool store_q0 = false);   // layer 0 (dW0 set): also store q_0 into q as plain fp32
 int launch_ln_fwd(const int* dims, const float* u, int W, const float* gamma, const float* beta, DropCfg drop, float* y,
                   float* stats, int max_graphs, cudaStream_t st);
 int launch_ln_bwd(const int* dims, const float* u, const float* y, const float* dy, int W, const float* gamma,

@@ -83,6 +83,7 @@ struct eims_plan {
   std::map<std::string, Buf> buf;
   int state;  // 0 none, 1 batch built, 2 forward(train) done, 3 loss grad ready, 4 head backward done
   int last_training;
+  bool eval_fwd = false;  // the last forward of the batch built last was an eval-mode one (eims_backward_feat may follow)
   // per-stage CUDA-event profiling (bench.py's roofline pass) and launch accounting
   eims_peaks peak_targets{};  // targets as peak lists (eims_plan_set_peak_targets); peak_ptr == NULL: unset
   // BatchNorm-backward statistics of the layers below the top come out of the SpMM that writes their dh.  Beyond 256
@@ -571,6 +572,7 @@ static int batch_build_impl(eims_plan* p, const eims_dataset* ds, const int32_t*
     p->batch_seq = 0;
   }
   ++p->batch_seq;
+  p->eval_fwd = false;
   STAGE(ST_K1, num_graphs > 1024 ? 2 : 1, launch_csr_build(ds, mol_ids, num_graphs, p->d.node_feat_dim, p->Nc, p->Ec, p->i("gptr"), p->i("eptr"),
                             p->i("gid"), p->i("src"), p->i("dst"), p->i("rowptr"), p->i("col"), p->f("norm"),
                             p->f("x"), p->i("dims"), st, p->f("a0"), p->batch_seq, indirect ? p->blk : nullptr, p->i("bids")));
@@ -657,7 +659,7 @@ int eims_forward(eims_plan* p, const float* params, float* bn_running, int32_t t
                              p->f(L_("bn_mean", l)), p->f(L_("bn_invstd", l)), p->f(L_("bn_scale", l)),
                              p->f(L_("bn_shift", l)), p->f("bn_partials"), p->Nc, st);
     return launch_bn_eval_coeffs(params + p->off_bn_g(l), params + p->off_bn_b(l), rm, rv, H, p->f(L_("bn_scale", l)),
-                                 p->f(L_("bn_shift", l)), st);
+                                 p->f(L_("bn_shift", l)), st, p->f(L_("bn_mean", l)), p->f(L_("bn_invstd", l)));
   };
   auto fuse = [&](int l) {
     float* rm = bn_running + (int64_t)l * 2 * H;
@@ -718,6 +720,7 @@ int eims_forward(eims_plan* p, const float* params, float* bn_running, int32_t t
                 nullptr, nullptr, params + p->off_head(9), 0, head_acc, st));
   p->state = training ? 2 : 1;
   p->last_training = training;
+  p->eval_fwd = !training;
   return check_launch("eims_forward");
 }
 
@@ -756,28 +759,34 @@ int eims_loss(eims_plan* p, const float* targets, const int32_t* target_rows, in
   return loss_impl(p, targets, target_rows, loss_kind, want_grad, nullptr, stream);
 }
 
-int eims_backward_part(eims_plan* p, const float* params, const float* dprob, float* grads, int32_t part,
-                       eims_stream_t stream) {
-  if (!p || !p->bound) return fail(EIMS_ERR_STATE, "plan not bound");
-  if (part < EIMS_BWD_ALL || part > EIMS_BWD_GCN) return fail(EIMS_ERR_ARG, "part must be one of EIMS_BWD_*");
-  if (p->state < 2 || !p->last_training) return fail(EIMS_ERR_STATE, "eims_backward needs a training-mode eims_forward first");
-  if (part == EIMS_BWD_GCN) {
-    if (p->state != 4) return fail(EIMS_ERR_STATE, "EIMS_BWD_GCN needs EIMS_BWD_HEAD first");
-  } else if (!dprob && p->state != 3) {
-    return fail(EIMS_ERR_STATE, "eims_backward without dprob needs eims_loss(want_grad=1) first");
-  }
-  if (!params || !grads) return fail(EIMS_ERR_ARG, "params / grads is NULL");
-  cudaStream_t st = (cudaStream_t)stream;
-  EarlyDimsScope early_scope(1);  // backward always follows a forward (state >= 2)
+// The backward of the forward enqueued last, for every public entry point: the training step's (eval = false, dfeat
+// NULL: eims_backward, eims_backward_part) and eims_backward_feat's (either mode, optionally down to the atom features).
+// The callers have checked the plan's state.
+static int backward_impl(eims_plan* p, const float* params, const float* dprob, float* grads, int32_t part, float* dfeat,
+                         bool eval, cudaStream_t st) {
+  EarlyDimsScope early_scope(1);  // backward always follows a forward (state >= 2, or an eval forward)
   const eims_dims& d = p->d;
   const int H = d.hidden_dim, F = d.node_feat_dim, L = d.num_gcn_layers, M = d.max_mz, P = p->pool_dim();
   const int* dims = p->i("dims");
-  const float drop_p = d.dropout > 0.f ? d.dropout : 0.f;
+  // eval mode: no dropout, BatchNorm is the affine map of the running statistics (bn_mean<l> / bn_invstd<l> hold them,
+  // written by the eval forward), so its backward has no batch-statistics terms: the two column means the apply pass
+  // subtracts stay zero (the statistics passes get means == NULL)
+  const float drop_p = (!eval && d.dropout > 0.f) ? d.dropout : 0.f;
   const float drop_scale = drop_p > 0.f ? 1.f / (1.f - drop_p) : 1.f;
+  float* means2 = eval ? nullptr : p->f("bn_means2");
+  // the head data gradients: a training forward's layer-0 kernel zeroed dy2 / dy1 / dG (split-K allowed); an eval
+  // forward zeroes nothing, so there they are plain stores
+  const int head_acc = eval ? 0 : 3;
   const uint64_t seed = p->last_step.seed;
   const int step = p->last_step.step;
   const bool planes = p->planes_on();  // as in the forward that produced a_l (the backend must not change in between)
   auto L_ = [&](const char* b, int l) { return std::string(b) + std::to_string(l); };
+  if (eval) {
+    if (cudaMemsetAsync(p->f("bn_means2"), 0, 2 * (size_t)H * sizeof(float), st) != cudaSuccess)
+      return fail(EIMS_ERR_CUDA, "cudaMemsetAsync failed");
+    // prob of this forward (an eval forward leaves only the logits; eims_sigmoid may not have run)
+    STAGE(ST_ELEMENTWISE, 1, launch_sigmoid(dims, p->f("logits"), M, p->f("prob"), p->Bc, st));
+  }
   if (part != EIMS_BWD_GCN) {
   if (dprob) STAGE(ST_ELEMENTWISE, 1, launch_dprob_to_dlogits(dims, p->f("prob"), dprob, M, p->f("dlogits"), p->Bc, st));
   float* dl = p->f("dlogits");
@@ -794,19 +803,19 @@ int eims_backward_part(eims_plan* p, const float* params, const float* dprob, fl
   }
   STAGE(ST_GEMM_HEAD_BWD, p->gemm_backend == EIMS_GEMM_TCGEN05 ? 1 : 2, gemm_pair(p,
         GemmProblem{dl, M, 1, p->f("y2"), H, 1, grads + p->off_head(8), H, M, H, p->Bc, nullptr, dB, nullptr, nullptr, 0, 1, nullptr},
-        GemmProblem{dl, M, 0, params + p->off_head(8), H, 1, p->f("dy2"), H, p->Bc, H, M, dB, nullptr, nullptr, nullptr, 0, 3, nullptr}, st));
+        GemmProblem{dl, M, 0, params + p->off_head(8), H, 1, p->f("dy2"), H, p->Bc, H, M, dB, nullptr, nullptr, nullptr, 0, head_acc, nullptr}, st));
   // LayerNorm backward also leaves the bias gradient of the Linear in front of it (column sums of du)
   STAGE(ST_LN_BWD, 1, launch_ln_bwd(dims, p->f("u2"), p->f("y2"), p->f("dy2"), H, params + p->off_head(6), p->f("ln2"), drop_scale,
                          p->f("dy2"), grads + p->off_head(6), grads + p->off_head(7), grads + p->off_head(5), p->Bc, st));
   STAGE(ST_GEMM_HEAD_BWD, p->gemm_backend == EIMS_GEMM_TCGEN05 ? 1 : 2, gemm_pair(p,
         GemmProblem{p->f("dy2"), H, 1, p->f("y1"), 2 * H, 1, grads + p->off_head(4), 2 * H, H, 2 * H, p->Bc, nullptr, dB, nullptr, nullptr, 0, 1, nullptr},
-        GemmProblem{p->f("dy2"), H, 0, params + p->off_head(4), 2 * H, 1, p->f("dy1"), 2 * H, p->Bc, 2 * H, H, dB, nullptr, nullptr, nullptr, 0, 3, nullptr}, st));
+        GemmProblem{p->f("dy2"), H, 0, params + p->off_head(4), 2 * H, 1, p->f("dy1"), 2 * H, p->Bc, 2 * H, H, dB, nullptr, nullptr, nullptr, 0, head_acc, nullptr}, st));
   STAGE(ST_LN_BWD, 1, launch_ln_bwd(dims, p->f("u1"), p->f("y1"), p->f("dy1"), 2 * H, params + p->off_head(2), p->f("ln1"),
                          drop_scale, p->f("dy1"), grads + p->off_head(2), grads + p->off_head(3), grads + p->off_head(1), p->Bc, st));
   STAGE(ST_GEMM_HEAD_BWD, p->gemm_backend == EIMS_GEMM_TCGEN05 ? 1 : 2, gemm_pair(p,
         GemmProblem{p->f("dy1"), 2 * H, 1, p->f("readout"), P, 1, grads + p->off_head(0), P, 2 * H, P, p->Bc, nullptr, dB, nullptr, nullptr, 0, 1, nullptr},
-        GemmProblem{p->f("dy1"), 2 * H, 0, params + p->off_head(0), P, 1, p->f("dG"), P, p->Bc, P, 2 * H, dB, nullptr, nullptr, nullptr, 0, 3, nullptr}, st));
-  p->state = 4;  // head gradients final (the data-parallel reducer may start on that bucket)
+        GemmProblem{p->f("dy1"), 2 * H, 0, params + p->off_head(0), P, 1, p->f("dG"), P, p->Bc, P, 2 * H, dB, nullptr, nullptr, nullptr, 0, head_acc, nullptr}, st));
+  if (!eval) p->state = 4;  // head gradients final (the data-parallel reducer may start on that bucket)
   }
   if (part == EIMS_BWD_HEAD) return check_launch("eims_backward_part");
   // ---- GCN layers, last to first (GCN:358-363 backwards)
@@ -816,18 +825,22 @@ int eims_backward_part(eims_plan* p, const float* params, const float* dprob, fl
     // statistics pass rides on that SpMM when fuse_bn_bwd_stats (see below)
     const bool from_readout = (l == L - 1);
     const float* dh_in = from_readout ? nullptr : p->f("dh");
-    if (from_readout)
+    if (from_readout) {
+      if (eval)  // the per-graph sums a training readout leaves in zstat, about the running mean
+        STAGE(ST_BN_BWD_STATS, 1, launch_bn_eval_zstat(dims, p->i("gptr"), p->f(L_("z", l)), H, p->f(L_("bn_mean", l)), p->i("argmax"),
+                                     d.pooling, p->f("zstat"), p->Bc, st));
       STAGE(ST_BN_BWD_STATS, 1, launch_bn_bwd_stats_top(dims, p->f("dG"), p->f("zstat"), p->i("gptr"), d.pooling, H, p->f(L_("bn_mean", l)),
-                                   p->f(L_("bn_invstd", l)), grads + p->off_bn_g(l), grads + p->off_bn_b(l), p->f("bn_means2"),
+                                   p->f(L_("bn_invstd", l)), grads + p->off_bn_g(l), grads + p->off_bn_b(l), means2,
                                    p->f("bn_partials"), p->Bc, st));
-    else if (!p->fuse_bn_bwd_stats)
+    } else if (!p->fuse_bn_bwd_stats) {
       STAGE(ST_BN_BWD_STATS, 1, launch_bn_bwd_stats(dims, dh_in, p->f(L_("z", l)), H, p->f(L_("bn_mean", l)), p->f(L_("bn_invstd", l)),
-                                   grads + p->off_bn_g(l), grads + p->off_bn_b(l), p->f("bn_means2"), p->f("bn_partials"), p->Nc, st));
+                                   grads + p->off_bn_g(l), grads + p->off_bn_b(l), means2, p->f("bn_partials"), p->Nc, st));
+    }
     STAGE(ST_BN_BWD_APPLY, 1, launch_bn_bwd_apply(dims, dh_in, p->f("dG"), p->i("gid"), p->i("gptr"), p->i("argmax"), d.pooling,
                                  p->f(L_("z", l)), H, p->f(L_("bn_mean", l)), p->f(L_("bn_invstd", l)), params + p->off_bn_g(l),
                                  p->f("norm"), grads + p->off_gcn_b(l), p->f("bn_means2"), p->f("q"), p->Nc, st,
                                  l == 0 ? p->f("a0") : nullptr, F, l == 0 ? grads + p->off_gcn_w(0) : nullptr,
-                                 (planes && l > 0) ? p->act_plane : 0));
+                                 (planes && l > 0) ? p->act_plane : 0, l == 0 && dfeat));
     if (l > 0 && planes) {
       // one persistent launch: data gradient tiles (stores) + weight gradient k-slices (red.add), balanced on the device
       GemmTmaProblem dg{p->map_q_k(), p->map_w_k(l), p->f("da"), H, 0, 0, p->Nc, H, H, dims + DIM_N, nullptr, nullptr, nullptr, 0, 0, nullptr};
@@ -842,18 +855,52 @@ int eims_backward_part(eims_plan* p, const float* params, const float* dprob, fl
       float* scratch = p->f("bn_partials");
       BnBwdFuse bf{p->f(L_("z", l - 1)), p->f(L_("bn_mean", l - 1)), p->f(L_("bn_invstd", l - 1)),
                    reinterpret_cast<double*>(scratch + 16), reinterpret_cast<unsigned int*>(scratch),
-                   grads + p->off_bn_g(l - 1), grads + p->off_bn_b(l - 1), p->f("bn_means2")};
+                   grads + p->off_bn_g(l - 1), grads + p->off_bn_b(l - 1), means2};
       STAGE(ST_SPMM_BWD, 1, launch_spmm_norm(dims, p->i("rowptr"), p->i("col"), p->f("norm"), p->f("da"), H, nullptr, nullptr,
                                 p->drop(drop_p, seed, step, l - 1), 1, p->f("dh"), p->Nc, st,
                                 p->fuse_bn_bwd_stats ? &bf : nullptr, p->i("gptr"), p->Bc, p->tile_rows()));
-    }  // l == 0: dW0 came out of the BatchNorm-backward apply pass above (q_0 is never materialised)
+    } else if (dfeat) {
+      // layer 0: dW0 came out of the apply pass above, which also left q_0 in q; da and dh are free here
+      STAGE(ST_GEMM_GCN_DGRAD, 1, launch_layer0_dgrad(dims, p->f("q"), H, params + p->off_gcn_w(0), F, p->f("da"), p->Nc, st));
+      STAGE(ST_SPMM_BWD, 1, launch_feat_grad(dims, p->i("rowptr"), p->i("col"), p->f("norm"), p->f("da"), F, dfeat, p->Nc, st));
+    }  // l == 0 without dfeat: q_0 is never materialised
   }
-  p->state = 1;
-  return check_launch("eims_backward_part");
+  if (!eval) p->state = 1;
+  return check_launch("eims_backward");
+}
+
+int eims_backward_part(eims_plan* p, const float* params, const float* dprob, float* grads, int32_t part,
+                       eims_stream_t stream) {
+  if (!p || !p->bound) return fail(EIMS_ERR_STATE, "plan not bound");
+  if (part < EIMS_BWD_ALL || part > EIMS_BWD_GCN) return fail(EIMS_ERR_ARG, "part must be one of EIMS_BWD_*");
+  if (p->state < 2 || !p->last_training) return fail(EIMS_ERR_STATE, "eims_backward needs a training-mode eims_forward first");
+  if (part == EIMS_BWD_GCN) {
+    if (p->state != 4) return fail(EIMS_ERR_STATE, "EIMS_BWD_GCN needs EIMS_BWD_HEAD first");
+  } else if (!dprob && p->state != 3) {
+    return fail(EIMS_ERR_STATE, "eims_backward without dprob needs eims_loss(want_grad=1) first");
+  }
+  if (!params || !grads) return fail(EIMS_ERR_ARG, "params / grads is NULL");
+  return backward_impl(p, params, dprob, grads, part, nullptr, false, (cudaStream_t)stream);
 }
 
 int eims_backward(eims_plan* p, const float* params, const float* dprob, float* grads, eims_stream_t stream) {
   return eims_backward_part(p, params, dprob, grads, EIMS_BWD_ALL, stream);
+}
+
+int eims_backward_feat(eims_plan* p, const float* params, const float* dprob, float* grads, float* dfeat,
+                       eims_stream_t stream) {
+  if (!p || !p->bound) return fail(EIMS_ERR_STATE, "plan not bound");
+  const bool eval = p->eval_fwd;
+  if (!eval) {
+    if (p->state < 2 || !p->last_training)
+      return fail(EIMS_ERR_STATE, "eims_backward_feat needs an eims_forward of the batch built last (and no backward since)");
+    if (p->state == 4) return fail(EIMS_ERR_STATE, "eims_backward_feat after EIMS_BWD_HEAD");
+    if (!dprob && p->state != 3) return fail(EIMS_ERR_STATE, "eims_backward_feat without dprob needs eims_loss(want_grad=1) first");
+  } else if (!dprob) {
+    return fail(EIMS_ERR_ARG, "dprob is NULL: an eval-mode backward needs the gradient w.r.t. the spectrum");
+  }
+  if (!params || !grads) return fail(EIMS_ERR_ARG, "params / grads is NULL");
+  return backward_impl(p, params, dprob, grads, EIMS_BWD_ALL, dfeat, eval, (cudaStream_t)stream);
 }
 
 int eims_metrics_accumulate(eims_plan* p, float* metrics, eims_stream_t stream) {

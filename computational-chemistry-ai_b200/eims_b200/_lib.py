@@ -103,6 +103,7 @@ _SIGS = {
     "eims_loss": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _vp]),
     "eims_backward": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
     "eims_backward_part": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _vp]),
+    "eims_backward_feat": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "eims_metrics_accumulate": (C.c_int, [_vp, _vp, _vp]),
     "eims_train_step": (C.c_int, [_vp, C.POINTER(Dataset), _vp, _i32, _vp, _vp, _vp, _vp, _vp, _i32, C.POINTER(Step), _vp, _vp]),
     "eims_train_step_built": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, C.POINTER(Step), _vp, _vp]),

@@ -293,15 +293,16 @@ class DeviceDataset:
 class PackedDataset:
     """One packed batch (the layout of eims_host_pack_batch / PackedHostBatch) at device address `base`, as the data set
     of its `num_graphs` molecules.  offsets: section name -> byte offset from base; a section that is absent has no
-    entry.  Duck-types DeviceDataset for the plan: struct, targets (an address), peaks (a Peaks struct)."""
+    entry.  Duck-types DeviceDataset for the plan: struct, targets (an address), peaks (a Peaks struct).  feat: the
+    address of other atom features [N, F] in the batch's order, read instead of the packed ones."""
 
-    def __init__(self, base: int, offsets, num_graphs: int, mz_is_f64: int = 0):
+    def __init__(self, base: int, offsets, num_graphs: int, mz_is_f64: int = 0, feat: int | None = None):
         o = offsets
         self.num_mols = int(num_graphs)
         self.targets = base + o["targets"] if "targets" in o else None
         self.peaks = (_lib.Peaks(base + o["peak_ptr"], base + o["peak_mz"], base + o["peak_inten"], mz_is_f64, self.num_mols)
                       if "peak_ptr" in o else None)
-        self.struct = Dataset(base + o["node_ptr"], base + o["bond_ptr"], base + o["feat"], base + o["bond_begin"],
+        self.struct = Dataset(base + o["node_ptr"], base + o["bond_ptr"], base + o["feat"] if feat is None else feat, base + o["bond_begin"],
                               base + o["bond_end"], self.targets, self.num_mols,
                               C.pointer(self.peaks) if self.peaks is not None else None)
 
@@ -426,6 +427,12 @@ class Plan:
 
     def backward(self, fp: FlatParams, dprob=None):
         check(self.lib.eims_backward(self.h, ptr(fp.params), ptr(dprob), ptr(fp.grads), self.stream))
+
+    def backward_feat(self, fp: FlatParams, dprob=None, dfeat=None):
+        """The backward of the forward enqueued last, training or eval mode (eims_backward_feat): parameter gradients
+        added into fp.grads and, when `dfeat` (a float32 [N, F] device tensor) is given, the gradient w.r.t. the
+        batch's atom features written into it.  dprob may be None only after loss(want_grad=True) in training mode."""
+        check(self.lib.eims_backward_feat(self.h, ptr(fp.params), ptr(dprob), ptr(fp.grads), ptr(dfeat), self.stream))
 
     def metrics_accumulate(self, metrics):
         check(self.lib.eims_metrics_accumulate(self.h, ptr(metrics), self.stream))

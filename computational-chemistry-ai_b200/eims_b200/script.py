@@ -21,6 +21,7 @@ from dataclasses import dataclass
 import numpy as np
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from . import _lib
 from .engine import FlatParams, ModelDims, Plan, make_step, onecycle_schedule, state_dict_order
@@ -165,17 +166,12 @@ class BatchedGraph:
         g._packed = self.packed()
         g._dev_buf = g._packed.buf.to(dev, non_blocking=True)
         g.device = dev
-        g.ndata = {"feat": _DeviceFeatHandle(g)}
+        # the features section of the uploaded batch, as a tensor (no copy): what K1 reads when forward() is given
+        # this tensor or no features
+        hb, n = g._packed, g.num_nodes()
+        o = hb.offsets["feat"]
+        g.ndata = {"feat": g._dev_buf[o:o + 4 * n * hb.feat_dim].view(torch.float32).view(n, hb.feat_dim)}
         return g
-
-
-class _DeviceFeatHandle:
-    """`batch_graph.ndata['feat']` after `.to(device)`: the model reads the features from the
-    uploaded packed batch, so this is only a handle naming it (GCN:419)."""
-
-    def __init__(self, g):
-        self.graph = g
-        self.shape = (g.num_nodes(), 6)
 
 
 def batch(graphs) -> BatchedGraph:
@@ -301,21 +297,33 @@ class OptimizedEIMSDataset(torch.utils.data.Dataset):
 
 # ------------------------------------------------------------------------------ model (GCN:303-376)
 class _ForwardFn(torch.autograd.Function):
-    """Differentiable GCNSpectrum.forward for callers that drive their own loop
-    (`loss.backward()` as in GCN:428): backward goes through eims_backward."""
+    """Differentiable GCNSpectrum.forward for callers that drive their own loop (`loss.backward()` as in GCN:428, or
+    per-atom attribution in eval mode): backward goes through eims_backward_feat, to the parameters (flat) and to the
+    atom features x (None: the graph's own, not differentiated).  The parameter gradients are always computed into the
+    model's scratch buffer and returned only when flat requires them."""
 
     @staticmethod
-    def forward(ctx, flat, model, g):
-        prob = model._run_forward(g, training=model.training)
-        ctx.model = model
+    def forward(ctx, flat, x, model, g):
+        prob = model._run_forward(g, training=model.training, feat=x)
+        ctx.model, ctx.seq, ctx.done = model, model._fwd_seq, False
+        ctx.x_shape = None if x is None else tuple(x.shape)
         return prob
 
     @staticmethod
+    @once_differentiable
     def backward(ctx, dprob):
         m = ctx.model
+        if ctx.done:
+            raise RuntimeError("GCNSpectrum: this forward was differentiated already")
+        if m._fwd_seq != ctx.seq:
+            raise RuntimeError("GCNSpectrum: the model ran another forward since this one; its activations are gone "
+                               "(call backward before the next forward)")
+        ctx.done = True
+        want_x = ctx.x_shape is not None and ctx.needs_input_grad[1]
+        dfeat = torch.empty(ctx.x_shape, dtype=torch.float32, device=dprob.device) if want_x else None
         m._fp.grads.zero_()
-        m._plan.backward(m._fp, dprob.contiguous())
-        return m._fp.grads.clone(), None, None
+        m._plan.backward_feat(m._fp, dprob.contiguous(), dfeat)
+        return (m._fp.grads.clone() if ctx.needs_input_grad[0] else None), dfeat, None, None
 
 
 class GCNSpectrum(nn.Module):
@@ -331,6 +339,7 @@ class GCNSpectrum(nn.Module):
         self._fp = None
         self._plan = None
         self._step = 0
+        self._fwd_seq = 0  # forwards run so far: a backward must belong to the last one (_ForwardFn)
         self._seed = int(np.random.SeedSequence().entropy % (1 << 62))
         self._init_host()
 
@@ -419,7 +428,8 @@ class GCNSpectrum(nn.Module):
             self._plan = Plan(self.dims, up(n_graphs, 16), up(n_nodes, 256), up(n_edges, 512), dev)
         return self._plan, self._fp
 
-    def _run_forward(self, g, training, targets=None):
+    def _run_forward(self, g, training, targets=None, feat=None):
+        """feat: atom features [N, F] (validated by _node_features) read instead of the graph's own."""
         from .engine import PackedDataset
         if isinstance(g, MolGraph):
             g = g.to(self.flat.device)
@@ -427,8 +437,11 @@ class GCNSpectrum(nn.Module):
             g = g.to(self.flat.device)
         plan, fp = self._engine(g.batch_size, g.num_nodes(), g.num_edges())
         hb = g._packed
-        self._keep = g  # the packed batch must outlive the asynchronous kernels
-        plan.batch_build(PackedDataset(g._dev_buf.data_ptr(), hb.offsets, hb.num_graphs), None, hb.num_graphs)
+        feat = None if feat is None else feat.detach().contiguous()
+        self._keep = (g, feat)  # the packed batch and the features must outlive the asynchronous kernels
+        self._fwd_seq += 1
+        plan.batch_build(PackedDataset(g._dev_buf.data_ptr(), hb.offsets, hb.num_graphs,
+                                       feat=None if feat is None else feat.data_ptr()), None, hb.num_graphs)
         if training:
             self._step += 1
             fp.count_steps()
@@ -437,10 +450,31 @@ class GCNSpectrum(nn.Module):
         plan.check()  # raises ZeroInDegreeError like DGL's GraphConv
         return plan.buffer("prob", torch.float32, (hb.num_graphs, self.dims.max_mz)).clone()
 
+    def _node_features(self, g, node_features):
+        """None when the graph's own features are to be read (no features given, or the graph's own tensor that needs
+        no gradient); otherwise the tensor, checked as the reference's first GraphConv would check its input."""
+        own = getattr(g, "ndata", {}).get("feat")
+        if node_features is None or (node_features is own and not node_features.requires_grad):
+            return None
+        x = node_features
+        if not isinstance(x, torch.Tensor):
+            raise TypeError(f"node_features must be a tensor, not {type(x).__name__}")
+        want = (g.num_nodes(), self.dims.node_feat_dim)
+        if tuple(x.shape) != want:
+            raise RuntimeError(f"node_features has shape {tuple(x.shape)}; this graph and model need {want}")
+        if x.dtype != torch.float32:
+            raise RuntimeError(f"node_features must be float32 (the model's dtype), got {x.dtype}")
+        if x.device != self.flat.device:
+            raise RuntimeError(f"node_features is on {x.device}, the model on {self.flat.device}")
+        return x
+
     def forward(self, g, node_features=None):
-        if torch.is_grad_enabled() and self.training:
-            return _ForwardFn.apply(self.flat, self, g)
-        return self._run_forward(g, training=self.training)
+        if self.flat.device.type != "cuda":
+            self._engine(0, 0, 0)  # raises: no CPU path
+        x = self._node_features(g, node_features)
+        if torch.is_grad_enabled() and (self.flat.requires_grad or (x is not None and x.requires_grad)):
+            return _ForwardFn.apply(self.flat, x, self, g)
+        return self._run_forward(g, training=self.training, feat=x)
 
 
 # ------------------------------------------------------------------------------ training (GCN:382-488)

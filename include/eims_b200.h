@@ -286,9 +286,17 @@ int eims_loss(eims_plan* p, const float* targets, const int32_t* target_rows, in
               int32_t want_grad, eims_stream_t stream);
 /* dprob: optional [B,M] gradient w.r.t. the spectrum (autograd use); NULL = use the
  * dlogits left by eims_loss(want_grad=1).  Gradients are ADDED into grads (flat, zeroed by
- * eims_adamw_flat / the caller). */
+ * eims_adamw_flat / the caller).  Training-mode forwards only (EIMS_ERR_STATE after an eval
+ * forward); eims_backward_feat also differentiates eval-mode forwards and the atom features. */
 int eims_backward(eims_plan* p, const float* params, const float* dprob, float* grads,
                   eims_stream_t stream);
+/* The backward of the forward enqueued last, training OR eval mode, optionally down to the atom features.
+ * dprob [B,M]: gradient w.r.t. the spectrum.  It may be NULL only after eims_loss(want_grad=1) in training mode.
+ * Parameter gradients are ADDED into grads, as in eims_backward.  In eval mode BatchNorm is the affine map
+ * of the running statistics, dropout is off, and running statistics are not touched.
+ * dfeat (may be NULL): d/dx of the batch's atom features, [N, F] in batch order, rows [0, N) overwritten. */
+int eims_backward_feat(eims_plan* p, const float* params, const float* dprob, float* grads, float* dfeat,
+                       eims_stream_t stream);
 /* The same in two parts, EIMS_BWD_HEAD then EIMS_BWD_GCN: after the head part the gradients of
  * the 10 spectrum_predictor tensors (the tail of the flat buffer, 84 % of its bytes) are final,
  * so a data-parallel caller can start reducing that bucket while the GCN layers are
