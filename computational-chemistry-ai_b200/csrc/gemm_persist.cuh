@@ -44,8 +44,9 @@ __device__ __forceinline__ void red_add_v4(float* p, float4 v) {
   asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
 }
 
-// The share of one CTA (PAIR = 1) or CTA pair (PAIR = 2) of the launch: identical in every role and in both CTAs of a
-// pair, a pure function of the live sizes.  TM = rows of an output tile = 128 * PAIR.
+// The share of CTA (pair) c of G (PAIR = 1: CTAs, PAIR = 2: CTA pairs) of the launch: identical in every role and in
+// both CTAs of a pair, a pure function of the live sizes.  TM = rows of an output tile = 128 * PAIR.  Host-callable, so
+// that the deal can be checked exhaustively without a GPU (tests/native/gemm_sched_probe.cu).
 struct Sched {
   int ps, pk;                          // index of the store / the split-K problem, -1 = none
   int tiles_s, nt_s, kb_s;             // store problem: live tiles, column tiles, k-blocks per tile
@@ -60,14 +61,13 @@ struct Cursor { int j, u; };
 struct SchedIn { int nprob, ovh; int red[2], N[2]; };
 
 template <int PAIR>
-__device__ __forceinline__ Sched make_sched(const SchedIn& in, const int (&Mv)[2], const int (&Kv)[2]) {
+__host__ __device__ __forceinline__ Sched make_sched(const SchedIn& in, const int (&Mv)[2], const int (&Kv)[2], int c, int G) {
   constexpr int TM = BM * PAIR;
   Sched s;
   s.ps = s.pk = -1;
   for (int k = 0; k < in.nprob; ++k) {
     if (in.red[k]) s.pk = k; else s.ps = k;
   }
-  const int G = gridDim.x / PAIR, c = blockIdx.x / PAIR;
   s.c = c; s.G = G;
   s.tiles_s = 0; s.nt_s = 1; s.kb_s = 0; s.KB = 0; s.nt_k = 1; s.u0 = s.u1 = 0;
   if (s.ps >= 0) {
@@ -101,7 +101,7 @@ __device__ __forceinline__ Sched make_sched(const SchedIn& in, const int (&Mv)[2
 }
 
 template <int PAIR>
-__device__ __forceinline__ bool next_item(const Sched& s, Cursor& cur, Item& it) {
+__host__ __device__ __forceinline__ bool next_item(const Sched& s, Cursor& cur, Item& it) {
   constexpr int TM = BM * PAIR;
   if (s.ps >= 0) {
     const int t = s.c + cur.j * s.G;

@@ -657,7 +657,7 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_3xtf32_persistent_ker
   pg::SchedIn sin;
   sin.nprob = 1; sin.ovh = 0;   // one store problem: no split-K items to balance against
   sin.red[0] = sin.red[1] = 0; sin.N[0] = sin.N[1] = g.N;
-  const pg::Sched sch = pg::make_sched<1>(sin, Mv, Kv);
+  const pg::Sched sch = pg::make_sched<1>(sin, Mv, Kv, blockIdx.x, gridDim.x);
 
   if (warp < kPersistProducerWarps) {
     // ---------------------------------------------------------------- producers

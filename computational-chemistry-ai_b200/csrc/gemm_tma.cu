@@ -221,7 +221,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_planes_kernel(const __grid_c
   SchedIn sin;
   sin.nprob = grp.nprob; sin.ovh = grp.ovh;
   sin.red[0] = grp.g[0].red; sin.red[1] = grp.g[1].red; sin.N[0] = grp.g[0].N; sin.N[1] = grp.g[1].N;
-  const Sched sch = make_sched<PAIR>(sin, Mv, Kv);
+  const Sched sch = make_sched<PAIR>(sin, Mv, Kv, blockIdx.x / PAIR, gridDim.x / PAIR);
 
   if (warp == 0) {
     // ---------------------------------------------------------------- copy-engine producer (every CTA: its rows of A, its part of B)
