@@ -78,12 +78,12 @@ __global__ void __launch_bounds__(256) sgemm_simt_kernel(GemmArgs g) {
   }
 }
 
-int launch_gemm_simt(const float* A, int lda, int a_mn, const float* B, int ldb, int b_mn, float* C, int ldc, int M,
-                     int N, int K, const int* m_dev, const int* k_dev, const float* row_scale, const float* bias,
-                     int relu, int accumulate, cudaStream_t st) {
+int launch_gemm_simt(const GemmProblem& q, cudaStream_t st) {
+  const int M = q.M, N = q.N, K = q.K;
   if (M <= 0 || N <= 0 || K <= 0) return EIMS_ERR_ARG;
-  if (accumulate == 2 || accumulate == 3) accumulate = 0;  // split-K-allowed store: plain store on this path
-  GemmArgs g{A, B, C, lda, ldb, ldc, a_mn, b_mn, M, N, K, m_dev, k_dev, row_scale, bias, relu, accumulate};
+  // split-K-allowed store: plain store on this path
+  const int accumulate = (q.accumulate == kGemmStoreSplit || q.accumulate == kGemmStoreSplitZeroed) ? 0 : q.accumulate;
+  GemmArgs g{q.A, q.B, q.C, q.lda, q.ldb, q.ldc, q.a_mn, q.b_mn, M, N, K, q.m_dev, q.k_dev, q.row_scale, q.bias, q.relu, accumulate};
   int splits = 1;
   if (accumulate) {  // split-K for the weight gradients (K = atoms or graphs)
     int tiles = ((M + 63) / 64) * ((N + 63) / 64);

@@ -771,15 +771,15 @@ namespace {
 
 // Tile shape and split-K factor of one problem.  `budget` = CTAs this problem should aim for
 // (148 alone, 74 when it shares the launch with a second problem).
-int configure(tc::Args& g, int accumulate, int budget, bool* wide_out, bool* need_memset) {
+int configure(tc::Args& g, GemmAcc accumulate, int budget, bool* wide_out, bool* need_memset) {
   using namespace tc;
   if (g.M <= 0 || g.N <= 0 || g.K <= 0) return EIMS_ERR_ARG;
-  if (g.bn.acc && (accumulate != 0 || g.bn.H != g.N)) return EIMS_ERR_ARG;
+  if (g.bn.acc && (accumulate != kGemmStore || g.bn.H != g.N)) return EIMS_ERR_ARG;
   g.vec_a = ((reinterpret_cast<uintptr_t>(g.A) & 15) == 0) && (g.lda % 4 == 0);
   g.vec_b = ((reinterpret_cast<uintptr_t>(g.B) & 15) == 0) && (g.ldb % 4 == 0);
   // 128 x 256 tiles (A read once per row block, 2 stages) when the problem is tall enough to
   // fill the chip with them; 128 x 128 tiles (3 stages) otherwise.
-  const bool wide = (g.N % 256 == 0) && ((int64_t)((g.M + BM - 1) / BM) * (g.N / 256) >= 64 || (accumulate == 1 && g.K >= 4096));
+  const bool wide = (g.N % 256 == 0) && ((int64_t)((g.M + BM - 1) / BM) * (g.N / 256) >= 64 || (accumulate == kGemmAdd && g.K >= 4096));
   const int BN = wide ? 256 : 128;
   const int mt = (g.M + BM - 1) / BM, nt = (g.N + BN - 1) / BN;
   const int kblocks = (g.K + BK - 1) / BK;
@@ -787,22 +787,22 @@ int configure(tc::Args& g, int accumulate, int budget, bool* wide_out, bool* nee
   int splits = 1;
   g.accumulate = accumulate;
   *need_memset = false;
-  if (accumulate == 1) {  // split-K: weight gradients reduce over atoms / graphs
+  if (accumulate == kGemmAdd) {  // split-K: weight gradients reduce over atoms / graphs
     splits = (budget + mt * nt - 1) / (mt * nt);
     const int maxs = (kblocks + min_kb - 1) / min_kb;  // at least min_kb k-blocks per slice
     if (splits > maxs) splits = maxs;
     if (splits < 1) splits = 1;
-  } else if (accumulate == 2 || accumulate == 3) {
+  } else if (accumulate == kGemmStoreSplit || accumulate == kGemmStoreSplitZeroed) {
     // store semantics, but the caller tolerates atomic accumulation order (backward dgrads of the
     // 512-row head): when the tile grid cannot fill the chip, split K and add into a zeroed C.
-    g.accumulate = 0;
+    g.accumulate = kGemmStore;
     if (!g.relu && !g.row_scale && mt * nt <= budget / 4 && kblocks >= 8 && g.ldc == g.N) {
       splits = budget / (mt * nt);
       const int maxs = kblocks / min_kb;
       if (splits > maxs) splits = maxs;
       if (splits > 1) {
-        *need_memset = accumulate == 2;  // accumulate == 3: the caller has zeroed C already
-        g.accumulate = 1;
+        *need_memset = accumulate == kGemmStoreSplit;  // kGemmStoreSplitZeroed: the caller has zeroed C already
+        g.accumulate = kGemmAdd;
       } else {
         splits = 1;
       }
@@ -865,16 +865,13 @@ tc::Args make_args(const GemmProblem& q) {
 
 }  // namespace
 
-int launch_gemm_tc(const float* A, int lda, int a_mn, const float* B, int ldb, int b_mn, float* C, int ldc, int M,
-                   int N, int K, const int* m_dev, const int* k_dev, const float* row_scale, const float* bias,
-                   int relu, int accumulate, cudaStream_t st, const BnFuse* bn) {
-  GemmProblem q{A, lda, a_mn, B, ldb, b_mn, C, ldc, M, N, K, m_dev, k_dev, row_scale, bias, relu, accumulate, bn};
+int launch_gemm_tc(const GemmProblem& q, cudaStream_t st) {
   tc::Group grp{};
   grp.g[0] = make_args(q);
   bool wide = false, zero = false;
-  if (int rc = configure(grp.g[0], accumulate, 148, &wide, &zero)) return rc;
+  if (int rc = configure(grp.g[0], q.accumulate, 148, &wide, &zero)) return rc;
   if (int rc = set_attrs()) return rc;
-  if (zero && cudaMemsetAsync(C, 0, (size_t)M * ldc * sizeof(float), st) != cudaSuccess) return EIMS_ERR_CUDA;
+  if (zero && cudaMemsetAsync(q.C, 0, (size_t)q.M * q.ldc * sizeof(float), st) != cudaSuccess) return EIMS_ERR_CUDA;
   grp.g[1] = grp.g[0];
   grp.ctas0 = grp.g[0].nt * grp.g[0].mt * grp.g[0].splits;
   return launch_group(grp, grp.ctas0, wide, st, 1);
@@ -891,10 +888,8 @@ int launch_gemm_tc_pair(const GemmProblem& p0, const GemmProblem& p1, cudaStream
   if (int rc = configure(grp.g[0], p0.accumulate, 148, &w0, &z0)) return rc;
   if (int rc = configure(grp.g[1], p1.accumulate, 148, &w1, &z1)) return rc;
   if (w0 != w1 || z0 || z1 || p0.bn || p1.bn) {
-    if (int rc = launch_gemm_tc(p0.A, p0.lda, p0.a_mn, p0.B, p0.ldb, p0.b_mn, p0.C, p0.ldc, p0.M, p0.N, p0.K, p0.m_dev, p0.k_dev,
-                                p0.row_scale, p0.bias, p0.relu, p0.accumulate, st, p0.bn)) return rc;
-    return launch_gemm_tc(p1.A, p1.lda, p1.a_mn, p1.B, p1.ldb, p1.b_mn, p1.C, p1.ldc, p1.M, p1.N, p1.K, p1.m_dev, p1.k_dev,
-                          p1.row_scale, p1.bias, p1.relu, p1.accumulate, st, p1.bn);
+    if (int rc = launch_gemm_tc(p0, st)) return rc;
+    return launch_gemm_tc(p1, st);
   }
   // small problems share one wave: aim each at half the chip
   const int c0 = grp.g[0].nt * grp.g[0].mt * grp.g[0].splits, c1 = grp.g[1].nt * grp.g[1].mt * grp.g[1].splits;

@@ -43,10 +43,23 @@ int launch_readout(const int* dims, const int* gptr, const float* z, int H, cons
                    float* zstat = nullptr, const float* bn_mean = nullptr);  // zstat [B][2H]: per graph, column sums of
                                                                              // z - bn_mean and z - bn_mean at the arg-max node (training)
 
+// GEMM problems of the fp32 SIMT kernel (dense.cu) and the tcgen05 kernel (gemm_tc.cu).
+// How a GEMM writes C; the values are those of eims_gemm's `accumulate`.
+enum GemmAcc : int {
+  kGemmStore = 0,             // C = result
+  kGemmAdd = 1,               // C += result, atomically (split-K weight gradients)
+  kGemmStoreSplit = 2,        // store, but a small grid may split K and add into C, which the launch zeroes first
+  kGemmStoreSplitZeroed = 3,  // the same with C already zeroed by the caller
+};
+// C[M,N] = op(A) op(B) (* row_scale per row, + bias, ReLU); a_mn / b_mn: the operand is stored MN-major.  m_dev / k_dev
+// (may be NULL) override M / K with the live sizes on the device.
+struct GemmProblem {
+  const float* A; int lda, a_mn; const float* B; int ldb, b_mn; float* C; int ldc, M, N, K;
+  const int* m_dev; const int* k_dev; const float* row_scale; const float* bias; int relu; GemmAcc accumulate; const BnFuse* bn;
+};
+
 // dense.cu
-int launch_gemm_simt(const float* A, int lda, int a_mn, const float* B, int ldb, int b_mn, float* C, int ldc, int M,
-                     int N, int K, const int* m_dev, const int* k_dev, const float* row_scale, const float* bias,
-                     int relu, int accumulate, cudaStream_t st);
+int launch_gemm_simt(const GemmProblem& q, cudaStream_t st);
 int64_t bn_scratch_floats(int H, int max_nodes);
 int launch_bn_stats(const int* dims, const float* z, int H, const float* gamma, const float* beta, float* rmean,
                     float* rvar, float* mean, float* invstd, float* scale, float* shift, float* partials,
@@ -92,13 +105,7 @@ int launch_step_blocks_store(const StepBlockPack& v, StepBlock* dst, int n, cuda
 int launch_dropout_mask(DropCfg d, int rows, int W, float* out, cudaStream_t st);
 
 // gemm_tc.cu  (tcgen05 / TMEM, 3xTF32)
-int launch_gemm_tc(const float* A, int lda, int a_mn, const float* B, int ldb, int b_mn, float* C, int ldc, int M,
-                   int N, int K, const int* m_dev, const int* k_dev, const float* row_scale, const float* bias,
-                   int relu, int accumulate, cudaStream_t st, const BnFuse* bn = nullptr);
-struct GemmProblem {
-  const float* A; int lda, a_mn; const float* B; int ldb, b_mn; float* C; int ldc, M, N, K;
-  const int* m_dev; const int* k_dev; const float* row_scale; const float* bias; int relu, accumulate; const BnFuse* bn;
-};
+int launch_gemm_tc(const GemmProblem& q, cudaStream_t st);
 int launch_gemm_tc_pair(const GemmProblem& p0, const GemmProblem& p1, cudaStream_t st);
 
 // gemm_tma.cu  (tcgen05 / TMEM, 3xTF32 on pre-split hi / lo operand planes fed by the tensor-map copy engine, persistent)

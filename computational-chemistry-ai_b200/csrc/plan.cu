@@ -4,8 +4,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
-#include <map>
-#include <string>
+#include <type_traits>
 #include <vector>
 
 #include <nvtx3/nvToolsExt.h>  // header-only (dlopens the injection library when a profiler is attached)
@@ -19,6 +18,8 @@ using namespace eims;
 namespace {
 
 thread_local char g_err[512] = "";
+
+constexpr int kMaxLayers = 16;  // GraphConv layers a plan can hold
 
 int fail(int code, const char* fmt, ...) {
   va_list ap;
@@ -48,7 +49,7 @@ int check_dims(const eims_dims* d) {
   if (d->node_feat_dim < 1 || d->node_feat_dim > 8) return fail(EIMS_ERR_ARG, "node_feat_dim must be in [1,8]");
   if (d->hidden_dim < 64 || d->hidden_dim % 64 || d->hidden_dim > 1024)
     return fail(EIMS_ERR_ARG, "hidden_dim must be a multiple of 64 in [64,1024]");
-  if (d->num_gcn_layers < 1 || d->num_gcn_layers > 16) return fail(EIMS_ERR_ARG, "num_gcn_layers must be in [1,16]");
+  if (d->num_gcn_layers < 1 || d->num_gcn_layers > kMaxLayers) return fail(EIMS_ERR_ARG, "num_gcn_layers must be in [1,16]");
   if (d->max_mz < 4 || d->max_mz % 4 || d->max_mz > 4096) return fail(EIMS_ERR_ARG, "max_mz must be a multiple of 4 in [4,4096]");
   if (d->pooling < 0 || d->pooling > 3) return fail(EIMS_ERR_ARG, "pooling must be one of EIMS_POOL_*");
   if (!(d->dropout >= 0.f && d->dropout < 1.f)) return fail(EIMS_ERR_ARG, "dropout must be in [0,1)");
@@ -68,7 +69,33 @@ std::vector<int64_t> param_sizes(const eims_dims* d) {
   return s;
 }
 
-struct Buf { void* ptr; int64_t bytes; };
+// The tables K1 writes for one batch.  The plan holds two sets of them (eims_plan::cur).
+struct BatchTables {
+  int *dims, *gptr, *eptr, *gid, *bids, *src, *dst, *rowptr, *col;
+  float *norm, *x, *a0;
+};
+
+// The buffers of the bound workspace, carved by walk_workspace.
+struct Workspace {
+  BatchTables t[2];
+  int *flags, *argmax;
+  float* a[kMaxLayers];  // a_l for l >= 1 (layer 0 reads the batch table a0)
+  float* wplanes;        // planes-capable plans only
+  float *z[kMaxLayers], *bn_mean[kMaxLayers], *bn_invstd[kMaxLayers], *bn_scale[kMaxLayers], *bn_shift[kMaxLayers];
+  float *bn_means2, *bn_partials, *readout, *zstat;
+  float *u1, *u2, *logits, *dy2, *dy1, *dG;  // outputs of the split-K head GEMMs
+  float *y1, *ln1, *y2, *ln2, *prob, *dlogits, *row_loss, *row_cos, *dh, *q, *da;
+};
+
+// Where a plan is in the calls on the batch built last; decides which calls it accepts.
+enum class Phase {
+  unbuilt,    // bound, no batch built yet
+  built,      // batch built, or its training backward enqueued
+  train_fwd,  // training forward enqueued
+  loss_grad,  // ... and eims_loss(want_grad = 1): dlogits ready
+  head_bwd,   // ... and the head part of the backward: the head gradients are final
+  eval_fwd,   // eval-mode forward enqueued (eims_backward_feat may follow)
+};
 
 }  // namespace
 
@@ -79,11 +106,10 @@ struct eims_plan {
   int64_t ws_bytes;
   bool bound;
   std::vector<int64_t> poff;  // parameter offsets
-  std::vector<std::pair<std::string, int64_t>> order;  // name -> bytes (carve order)
-  std::map<std::string, Buf> buf;
-  int state;  // 0 none, 1 batch built, 2 forward(train) done, 3 loss grad ready, 4 head backward done
-  int last_training;
-  bool eval_fwd = false;  // the last forward of the batch built last was an eval-mode one (eims_backward_feat may follow)
+  Workspace ws{};
+  int64_t head_zero_bytes = 0;  // bytes of the range [u1, end of dG) a training forward's layer-0 kernel zeroes
+  Phase phase = Phase::unbuilt;
+  bool after_train_fwd() const { return phase == Phase::train_fwd || phase == Phase::loss_grad || phase == Phase::head_bwd; }
   // per-stage CUDA-event profiling (bench.py's roofline pass) and launch accounting
   eims_peaks peak_targets{};  // targets as peak lists (eims_plan_set_peak_targets); peak_ptr == NULL: unset
   // BatchNorm-backward statistics of the layers below the top come out of the SpMM that writes their dh.  Beyond 256
@@ -135,6 +161,7 @@ struct eims_plan {
   // set the kernels enqueued so far do NOT use and makes it current for what is enqueued next, so
   // the next batch can be built on a side stream while the current step is still running.
   int cur = 0;
+  const BatchTables& tab() const { return ws.t[cur]; }
   // Device step block (eims_plan_set_step_block) and the mode of the call being enqueued: `indirect` calls take
   // the batch's ids, the dropout keys and the AdamW scalars from it instead of from kernel parameters, so that
   // the launches can be captured into a CUDA graph once and replayed for every step.
@@ -158,15 +185,6 @@ struct eims_plan {
     if (indirect && blk && site >= 0 && site < kMaxDropSites) d.key_dev = &blk->drop_key[site];
     return d;
   }
-  static bool pingpong(const std::string& n) {
-    static const char* k[] = {"dims", "gptr", "eptr", "gid", "src", "dst", "rowptr", "col", "norm", "x", "a0", "bids"};
-    for (const char* s : k) if (n == s) return true;
-    return false;
-  }
-  std::string key(const std::string& n) const { return pingpong(n) ? n + (cur ? "#1" : "#0") : n; }
-  template <class T> T* get(const std::string& n) { return reinterpret_cast<T*>(buf[key(n)].ptr); }
-  float* f(const std::string& n) { return get<float>(n); }
-  int* i(const std::string& n) { return get<int>(n); }
   // parameter accessors (flat buffer)
   int64_t off_gcn_w(int l) const { return poff[2 * l]; }
   int64_t off_gcn_b(int l) const { return poff[2 * l + 1]; }
@@ -177,23 +195,66 @@ struct eims_plan {
 
 namespace {
 
-int gemm(eims_plan* p, const float* A, int lda, int a_mn, const float* B, int ldb, int b_mn, float* C, int ldc, int M,
-         int N, int K, const int* m_dev, const int* k_dev, const float* rs, const float* bias, int relu, int acc,
-         cudaStream_t st, const BnFuse* bn = nullptr) {
-  if (p->gemm_backend == EIMS_GEMM_FP32_SIMT)
-    return launch_gemm_simt(A, lda, a_mn, B, ldb, b_mn, C, ldc, M, N, K, m_dev, k_dev, rs, bias, relu, acc, st);
-  return launch_gemm_tc(A, lda, a_mn, B, ldb, b_mn, C, ldc, M, N, K, m_dev, k_dev, rs, bias, relu, acc, st, bn);
+int launch_gemm(int backend, const GemmProblem& q, cudaStream_t st) {
+  return backend == EIMS_GEMM_FP32_SIMT ? launch_gemm_simt(q, st) : launch_gemm_tc(q, st);
 }
 
 // weight gradient + data gradient of one layer (both consume the same dy) in one launch
 int gemm_pair(eims_plan* p, const GemmProblem& a, const GemmProblem& b, cudaStream_t st) {
   if (p->gemm_backend == EIMS_GEMM_FP32_SIMT) {
-    for (const GemmProblem* q : {&a, &b})
-      if (int rc = gemm(p, q->A, q->lda, q->a_mn, q->B, q->ldb, q->b_mn, q->C, q->ldc, q->M, q->N, q->K, q->m_dev, q->k_dev,
-                        q->row_scale, q->bias, q->relu, q->accumulate, st, q->bn)) return rc;
-    return 0;
+    if (int rc = launch_gemm_simt(a, st)) return rc;
+    return launch_gemm_simt(b, st);
   }
   return launch_gemm_tc_pair(a, b, st);
+}
+
+// How eims_plan_buffer names a buffer: `name`, `name<l>` (per GraphConv layer), `name#<set>` (per batch-table set).
+enum class Naming { plain, layer, set };
+
+// Every workspace buffer in carve order, as f(name, naming, index, bytes, slot) with `slot` the typed pointer field the
+// buffer is bound to.  Sizes are rounded up to 256 bytes, so in a 256-aligned workspace every buffer is 256-aligned.
+// eims_plan_create sizes the workspace with it, eims_plan_bind carves it, eims_plan_buffer resolves names.
+template <class Fn> void walk_workspace(eims_plan* p, Fn&& f) {
+  Workspace& w = p->ws;
+  const int64_t B = p->Bc, N = p->Nc, E = p->Ec, H = p->d.hidden_dim, F = p->d.node_feat_dim, M = p->d.max_mz;
+  const int L = p->d.num_gcn_layers;
+  const int64_t P = p->pool_dim();
+  auto r = [](int64_t bytes) { return (bytes + 255) & ~(int64_t)255; };
+  auto one = [&](const char* n, int64_t bytes, auto& slot) { f(n, Naming::plain, 0, r(bytes), slot); };
+  auto layer = [&](const char* n, int l, int64_t bytes, auto& slot) { f(n, Naming::layer, l, r(bytes), slot); };
+  auto sets = [&](const char* n, int64_t bytes, auto BatchTables::*m) {
+    for (int k = 0; k < 2; ++k) f(n, Naming::set, k, r(bytes), w.t[k].*m);
+  };
+  sets("dims", 16 * 4, &BatchTables::dims); one("flags", 16 * 4, w.flags);
+  sets("gptr", (B + 1) * 4, &BatchTables::gptr); sets("eptr", (B + 1) * 4, &BatchTables::eptr);
+  sets("gid", N * 4, &BatchTables::gid); sets("bids", B * 4, &BatchTables::bids);
+  sets("src", E * 4, &BatchTables::src); sets("dst", E * 4, &BatchTables::dst);
+  sets("rowptr", (N + 1) * 4, &BatchTables::rowptr); sets("col", E * 4, &BatchTables::col);
+  one("argmax", B * H * 4, w.argmax);
+  sets("norm", N * 4, &BatchTables::norm); sets("x", N * F * 4, &BatchTables::x); sets("a0", N * F * 4, &BatchTables::a0);
+  // a_l and q hold two planes (tf32 hi / lo) when the GraphConv GEMMs may take the planes path
+  const int64_t act_bytes = p->planes_cap ? 2 * p->act_plane * 4 : N * H * 4;
+  for (int l = 1; l < L; ++l) layer("a", l, act_bytes, w.a[l]);
+  if (p->planes_cap) one("wplanes", 2 * p->w_plane * 4, w.wplanes);
+  for (int l = 0; l < L; ++l) layer("z", l, N * H * 4, w.z[l]);
+  for (int l = 0; l < L; ++l) {
+    layer("bn_mean", l, H * 4, w.bn_mean[l]); layer("bn_invstd", l, H * 4, w.bn_invstd[l]);
+    layer("bn_scale", l, H * 4, w.bn_scale[l]); layer("bn_shift", l, H * 4, w.bn_shift[l]);
+  }
+  one("bn_means2", 2 * H * 4, w.bn_means2);
+  one("bn_partials", bn_scratch_floats(p->d.hidden_dim, p->Nc) * 4, w.bn_partials);
+  one("readout", B * P * 4, w.readout);
+  one("zstat", B * 2 * H * 4, w.zstat);  // per graph: raw column sums and raw arg-max values of the top layer (training)
+  // outputs of the split-K head GEMMs, contiguous: a training forward zeroes the whole range once
+  // (inside the layer-0 kernel) instead of one memset per GEMM, which would also break the
+  // programmatic-dependent-launch chain six times per step
+  one("u1", B * 2 * H * 4, w.u1); one("u2", B * H * 4, w.u2); one("logits", B * M * 4, w.logits);
+  one("dy2", B * H * 4, w.dy2); one("dy1", B * 2 * H * 4, w.dy1); one("dG", B * P * 4, w.dG);
+  one("y1", B * 2 * H * 4, w.y1); one("ln1", B * 2 * 4, w.ln1);
+  one("y2", B * H * 4, w.y2); one("ln2", B * 2 * 4, w.ln2);
+  one("prob", B * M * 4, w.prob); one("dlogits", B * M * 4, w.dlogits);
+  one("row_loss", B * 4, w.row_loss); one("row_cos", B * 4, w.row_cos);
+  one("dh", N * H * 4, w.dh); one("q", act_bytes, w.q); one("da", N * H * 4, w.da);
 }
 
 enum Stage {
@@ -246,19 +307,6 @@ struct EarlyDimsScope {
     EIMS_TRY(expr);                  \
     prof_end(p, st);                 \
   } while (0)
-
-void add(eims_plan* p, const std::string& name, int64_t bytes) {
-  bytes = (bytes + 255) & ~(int64_t)255;
-  if (eims_plan::pingpong(name)) {
-    for (const char* sfx : {"#0", "#1"}) {
-      p->order.emplace_back(name + sfx, bytes);
-      p->ws_bytes += bytes;
-    }
-    return;
-  }
-  p->order.emplace_back(name, bytes);
-  p->ws_bytes += bytes;
-}
 
 }  // namespace
 
@@ -331,12 +379,11 @@ int eims_gemm(int32_t backend, const float* A, int32_t lda, int32_t a_mn_major, 
               int32_t b_mn_major, float* C, int32_t ldc, int32_t M, int32_t N, int32_t K, const int32_t* m_dev,
               const int32_t* k_dev, const float* row_scale, const float* bias, int32_t relu, int32_t accumulate,
               eims_stream_t stream) {
-  if (backend == EIMS_GEMM_FP32_SIMT)
-    EIMS_TRY(launch_gemm_simt(A, lda, a_mn_major, B, ldb, b_mn_major, C, ldc, M, N, K, m_dev, k_dev, row_scale, bias,
-                              relu, accumulate, (cudaStream_t)stream));
-  else
-    EIMS_TRY(launch_gemm_tc(A, lda, a_mn_major, B, ldb, b_mn_major, C, ldc, M, N, K, m_dev, k_dev, row_scale, bias,
-                            relu, accumulate, (cudaStream_t)stream));
+  EIMS_TRY(launch_gemm(backend, GemmProblem{.A = A, .lda = lda, .a_mn = a_mn_major, .B = B, .ldb = ldb, .b_mn = b_mn_major,
+                                             .C = C, .ldc = ldc, .M = M, .N = N, .K = K, .m_dev = m_dev, .k_dev = k_dev,
+                                             .row_scale = row_scale, .bias = bias, .relu = relu,
+                                             .accumulate = static_cast<GemmAcc>(accumulate)},
+                       (cudaStream_t)stream));
   return check_launch("eims_gemm");
 }
 
@@ -375,8 +422,9 @@ int eims_gemm_planes(const eims_gemm_problem* p0, const eims_gemm_problem* p1, v
       EIMS_TRY(tma_make_map(&maps[2 * n + o], hi, plane, (int)rows[o], cols[o], ld[o], o ? kTmaBRows : 128, mn[o]));
       c += ((2 * 4 * plane + 255) & ~(int64_t)255);
     }
-    gp[n] = GemmTmaProblem{&maps[2 * n], &maps[2 * n + 1], q->C, q->ldc, q->a_mn_major, q->b_mn_major, q->M, q->N, q->K, q->m_dev,
-                           q->k_dev, q->row_scale, q->bias, q->relu, q->accumulate ? 1 : 0, nullptr};
+    gp[n] = GemmTmaProblem{.ta = &maps[2 * n], .tb = &maps[2 * n + 1], .C = q->C, .ldc = q->ldc, .a_mn = q->a_mn_major,
+                           .b_mn = q->b_mn_major, .M = q->M, .N = q->N, .K = q->K, .m_dev = q->m_dev, .k_dev = q->k_dev,
+                           .row_scale = q->row_scale, .bias = q->bias, .relu = q->relu, .red = q->accumulate ? 1 : 0};
     if (!gemm_tma_supports(gp[n])) return fail(EIMS_ERR_ARG, "shape not supported by the planes GEMM (N %% 256, ldc %% 4, K <= 512 unless split-K)");
     ++n;
   }
@@ -445,46 +493,36 @@ int eims_plan_create(const eims_dims* d, int32_t max_graphs, int32_t max_nodes, 
   p->Bc = max_graphs; p->Nc = max_nodes; p->Ec = max_edges > 0 ? max_edges : 1;
   p->gemm_backend = EIMS_GEMM_TCGEN05;
   p->fuse_bn_bwd_stats = d->hidden_dim <= 256;
-  p->ws_bytes = 0; p->bound = false; p->state = 0; p->last_training = 0;
+  p->ws_bytes = 0; p->bound = false;
   memset(&p->last_step, 0, sizeof(p->last_step));
   auto s = param_sizes(d);
   int64_t o = 0;
   for (int64_t v : s) { p->poff.push_back(o); o += v; }
   p->poff.push_back(o);
-  const int64_t B = p->Bc, N = p->Nc, E = p->Ec, H = d->hidden_dim, F = d->node_feat_dim, M = d->max_mz, L = d->num_gcn_layers;
-  const int64_t P = p->pool_dim();
-  add(p, "dims", 16 * 4); add(p, "flags", 16 * 4);
-  add(p, "gptr", (B + 1) * 4); add(p, "eptr", (B + 1) * 4); add(p, "gid", N * 4); add(p, "bids", B * 4);
-  add(p, "src", E * 4); add(p, "dst", E * 4); add(p, "rowptr", (N + 1) * 4); add(p, "col", E * 4);
-  add(p, "argmax", B * H * 4);
-  add(p, "norm", N * 4); add(p, "x", N * F * 4); add(p, "a0", N * F * 4);
+  const int64_t N = p->Nc, H = d->hidden_dim, L = d->num_gcn_layers;
   // a_l and q hold two planes (tf32 hi / lo) when the GraphConv GEMMs may take the planes path; rows padded to 32
   p->planes_cap = gemm_tma_enabled() && H % 256 == 0 && H <= 1024 && L > 1;
-  const int64_t Np = (N + 31) & ~(int64_t)31;
-  p->act_plane = Np * H;
+  p->act_plane = ((N + 31) & ~(int64_t)31) * H;
   p->w_plane = p->planes_cap ? (p->off_gcn_w(L - 1) + H * H - p->off_gcn_w(1)) : 0;
-  const int64_t act_bytes = p->planes_cap ? 2 * Np * H * 4 : N * H * 4;
-  for (int l = 1; l < L; ++l) add(p, "a" + std::to_string(l), act_bytes);
-  if (p->planes_cap) add(p, "wplanes", 2 * p->w_plane * 4);
-  for (int l = 0; l < L; ++l) add(p, "z" + std::to_string(l), N * H * 4);
-  for (int l = 0; l < L; ++l) {
-    add(p, "bn_mean" + std::to_string(l), H * 4); add(p, "bn_invstd" + std::to_string(l), H * 4);
-    add(p, "bn_scale" + std::to_string(l), H * 4); add(p, "bn_shift" + std::to_string(l), H * 4);
+  // The layer-0 kernel of a training forward zeroes [u1, end of dG) as one range: the six split-K head outputs must
+  // follow one another in the carve order, with nothing in between.
+  const Workspace& w = p->ws;
+  const void* const head[] = {&w.u1, &w.u2, &w.logits, &w.dy2, &w.dy1, &w.dG};
+  int next = 0;  // head[next] is the head output expected next
+  bool contiguous = true;
+  walk_workspace(p, [&](const char*, Naming, int, int64_t bytes, auto& slot) {
+    if (next < 6 && static_cast<const void*>(&slot) == head[next]) {
+      ++next;
+      p->head_zero_bytes += bytes;
+    } else if (next > 0 && next < 6) {
+      contiguous = false;
+    }
+    p->ws_bytes += bytes;
+  });
+  if (next != 6 || !contiguous) {
+    delete p;
+    return fail(EIMS_ERR_STATE, "workspace layout: the head outputs u1 .. dG are not contiguous");
   }
-  add(p, "bn_means2", 2 * H * 4);
-  add(p, "bn_partials", bn_scratch_floats(d->hidden_dim, p->Nc) * 4);
-  add(p, "readout", B * P * 4);
-  add(p, "zstat", B * 2 * H * 4);  // per graph: raw column sums and raw arg-max values of the top layer (training)
-  // outputs of the split-K head GEMMs, contiguous: a training forward zeroes the whole range once
-  // (inside the layer-0 kernel) instead of one memset per GEMM, which would also break the
-  // programmatic-dependent-launch chain six times per step
-  add(p, "u1", B * 2 * H * 4); add(p, "u2", B * H * 4); add(p, "logits", B * M * 4);
-  add(p, "dy2", B * H * 4); add(p, "dy1", B * 2 * H * 4); add(p, "dG", B * P * 4);
-  add(p, "y1", B * 2 * H * 4); add(p, "ln1", B * 2 * 4);
-  add(p, "y2", B * H * 4); add(p, "ln2", B * 2 * 4);
-  add(p, "prob", B * M * 4); add(p, "dlogits", B * M * 4);
-  add(p, "row_loss", B * 4); add(p, "row_cos", B * 4);
-  add(p, "dh", N * H * 4); add(p, "q", act_bytes); add(p, "da", N * H * 4);
   *out = p;
   return 0;
 }
@@ -501,36 +539,37 @@ int eims_plan_bind(eims_plan* p, void* workspace, int64_t bytes) {
   if (!p || !workspace) return fail(EIMS_ERR_ARG, "plan / workspace is NULL");
   if (bytes < p->ws_bytes) return fail(EIMS_ERR_ARG, "workspace too small: %lld < %lld", (long long)bytes, (long long)p->ws_bytes);
   if (reinterpret_cast<uintptr_t>(workspace) & 255) return fail(EIMS_ERR_ARG, "workspace must be 256-byte aligned");
-  char* c = reinterpret_cast<char*>(workspace);
-  for (auto& kv : p->order) { p->buf[kv.first] = Buf{c, kv.second}; c += kv.second; }
+  Workspace& w = p->ws;
   // counters / flags / dims start at zero (the ticket counter in bn_partials must be 0)
-  if (cudaMemset(p->buf["dims#0"].ptr, 0, p->buf["dims#0"].bytes) != cudaSuccess ||
-      cudaMemset(p->buf["dims#1"].ptr, 0, p->buf["dims#1"].bytes) != cudaSuccess ||
-      cudaMemset(p->buf["flags"].ptr, 0, p->buf["flags"].bytes) != cudaSuccess ||
-      cudaMemset(p->buf["bn_partials"].ptr, 0, p->buf["bn_partials"].bytes) != cudaSuccess)
-    return fail(EIMS_ERR_CUDA, "cudaMemset failed: %s", cudaGetErrorString(cudaGetLastError()));
+  const void* const zeroed[] = {&w.t[0].dims, &w.t[1].dims, &w.flags, &w.bn_partials};
+  char* c = reinterpret_cast<char*>(workspace);
+  cudaError_t e = cudaSuccess;
+  walk_workspace(p, [&](const char*, Naming, int, int64_t bytes, auto& slot) {
+    slot = reinterpret_cast<std::remove_reference_t<decltype(slot)>>(c);
+    for (const void* z : zeroed)
+      if (z == static_cast<const void*>(&slot) && e == cudaSuccess) e = cudaMemset(c, 0, bytes);
+    c += bytes;
+  });
+  if (e != cudaSuccess) return fail(EIMS_ERR_CUDA, "cudaMemset failed: %s", cudaGetErrorString(cudaGetLastError()));
   p->maps.clear();
   if (p->planes_cap) {
     const int L = p->d.num_gcn_layers, H = p->d.hidden_dim;
     const int rows = (int)(p->act_plane / H);
     p->maps.resize(4 * (L - 1) + 2);
     int rc = 0;
-    float* wpl = reinterpret_cast<float*>(p->buf["wplanes"].ptr);
     for (int l = 1; l < L && !rc; ++l) {
-      float* a = reinterpret_cast<float*>(p->buf["a" + std::to_string(l)].ptr);
-      float* w = wpl + (p->off_gcn_w(l) - p->off_gcn_w(1));
-      rc = tma_make_map(&p->maps[4 * (l - 1) + 0], a, p->act_plane, rows, H, H, 128, 0);
-      if (!rc) rc = tma_make_map(&p->maps[4 * (l - 1) + 1], a, p->act_plane, rows, H, H, 128, 1);
-      if (!rc) rc = tma_make_map(&p->maps[4 * (l - 1) + 2], w, p->w_plane, H, H, H, kTmaBRows, 1);
-      if (!rc) rc = tma_make_map(&p->maps[4 * (l - 1) + 3], w, p->w_plane, H, H, H, kTmaBRows, 0);
+      const float* wl = w.wplanes + (p->off_gcn_w(l) - p->off_gcn_w(1));
+      rc = tma_make_map(&p->maps[4 * (l - 1) + 0], w.a[l], p->act_plane, rows, H, H, 128, 0);
+      if (!rc) rc = tma_make_map(&p->maps[4 * (l - 1) + 1], w.a[l], p->act_plane, rows, H, H, 128, 1);
+      if (!rc) rc = tma_make_map(&p->maps[4 * (l - 1) + 2], wl, p->w_plane, H, H, H, kTmaBRows, 1);
+      if (!rc) rc = tma_make_map(&p->maps[4 * (l - 1) + 3], wl, p->w_plane, H, H, H, kTmaBRows, 0);
     }
-    float* q = reinterpret_cast<float*>(p->buf["q"].ptr);
-    if (!rc) rc = tma_make_map(&p->maps[4 * (L - 1) + 0], q, p->act_plane, rows, H, H, 128, 0);
-    if (!rc) rc = tma_make_map(&p->maps[4 * (L - 1) + 1], q, p->act_plane, rows, H, H, 128, 1);
+    if (!rc) rc = tma_make_map(&p->maps[4 * (L - 1) + 0], w.q, p->act_plane, rows, H, H, 128, 0);
+    if (!rc) rc = tma_make_map(&p->maps[4 * (L - 1) + 1], w.q, p->act_plane, rows, H, H, 128, 1);
     if (rc) p->maps.clear();  // the encoder refused: the in-kernel-split GEMMs take over (planes_on() is false)
   }
   p->bound = true;
-  p->state = 0;
+  p->phase = Phase::unbuilt;
   return 0;
 }
 
@@ -550,10 +589,19 @@ int eims_plan_set_gemm_planes(eims_plan* p, int32_t mode) {
 
 int eims_plan_buffer(eims_plan* p, const char* name, void** ptr, int64_t* bytes) {
   if (!p || !p->bound || !name) return fail(EIMS_ERR_STATE, "plan not bound");
-  auto it = p->buf.find(p->key(name));
-  if (it == p->buf.end()) return fail(EIMS_ERR_ARG, "no workspace buffer named '%s'", name);
-  if (ptr) *ptr = it->second.ptr;
-  if (bytes) *bytes = it->second.bytes;
+  bool found = false;
+  walk_workspace(p, [&](const char* base, Naming how, int k, int64_t n, auto& slot) {
+    if (found) return;
+    char full[32];
+    if (how == Naming::plain) snprintf(full, sizeof(full), "%s", base);
+    else snprintf(full, sizeof(full), how == Naming::layer ? "%s%d" : "%s#%d", base, k);
+    // a bare batch-table name means the current set
+    if (strcmp(name, full) != 0 && !(how == Naming::set && k == p->cur && strcmp(name, base) == 0)) return;
+    found = true;
+    if (ptr) *ptr = slot;
+    if (bytes) *bytes = n;
+  });
+  if (!found) return fail(EIMS_ERR_ARG, "no workspace buffer named '%s'", name);
   return 0;
 }
 
@@ -566,17 +614,17 @@ static int batch_build_impl(eims_plan* p, const eims_dataset* ds, const int32_t*
   cudaStream_t st = (cudaStream_t)stream;
   p->cur ^= 1;  // build into the other set of batch tables; later calls use it
   if (p->batch_seq >= 0x7ffffff0) {  // sequence wrap: forget the old zero-degree tag
-    for (const char* nm : {"dims#0", "dims#1"})
-      if (cudaMemsetAsync(reinterpret_cast<int*>(p->buf[nm].ptr) + DIM_ZERO_DEG, 0, sizeof(int), st) != cudaSuccess)
+    for (const BatchTables& t : p->ws.t)
+      if (cudaMemsetAsync(t.dims + DIM_ZERO_DEG, 0, sizeof(int), st) != cudaSuccess)
         return fail(EIMS_ERR_CUDA, "cudaMemsetAsync failed");
     p->batch_seq = 0;
   }
   ++p->batch_seq;
-  p->eval_fwd = false;
-  STAGE(ST_K1, num_graphs > 1024 ? 2 : 1, launch_csr_build(ds, mol_ids, num_graphs, p->d.node_feat_dim, p->Nc, p->Ec, p->i("gptr"), p->i("eptr"),
-                            p->i("gid"), p->i("src"), p->i("dst"), p->i("rowptr"), p->i("col"), p->f("norm"),
-                            p->f("x"), p->i("dims"), st, p->f("a0"), p->batch_seq, indirect ? p->blk : nullptr, p->i("bids")));
-  p->state = 1;
+  const BatchTables& t = p->tab();
+  STAGE(ST_K1, num_graphs > 1024 ? 2 : 1, launch_csr_build(ds, mol_ids, num_graphs, p->d.node_feat_dim, p->Nc, p->Ec, t.gptr, t.eptr,
+                            t.gid, t.src, t.dst, t.rowptr, t.col, t.norm, t.x, t.dims, st, t.a0, p->batch_seq,
+                            indirect ? p->blk : nullptr, t.bids));
+  p->phase = Phase::built;
   return check_launch("eims_batch_build");
 }
 
@@ -640,94 +688,95 @@ int eims_step_block_upload(eims_plan* p, const eims_step* s, const int32_t* mol_
 int eims_forward(eims_plan* p, const float* params, float* bn_running, int32_t training, const eims_step* s,
                  eims_stream_t stream) {
   if (!p || !p->bound) return fail(EIMS_ERR_STATE, "plan not bound");
-  if (p->state < 1) return fail(EIMS_ERR_STATE, "eims_forward before eims_batch_build");
+  if (p->phase == Phase::unbuilt) return fail(EIMS_ERR_STATE, "eims_forward before eims_batch_build");
   if (!params || !bn_running) return fail(EIMS_ERR_ARG, "params / bn_running is NULL");
   cudaStream_t st = (cudaStream_t)stream;
   const eims_dims& d = p->d;
   const int H = d.hidden_dim, F = d.node_feat_dim, L = d.num_gcn_layers, M = d.max_mz, P = p->pool_dim();
-  const int* dims = p->i("dims");
+  const BatchTables& t = p->tab();
+  const Workspace& w = p->ws;
+  const int* dims = t.dims;
   const float drop_p = (training && d.dropout > 0.f) ? d.dropout : 0.f;
   const uint64_t seed = s ? s->seed : 0;
   const int step = s ? s->step : 0;
   if (s) p->last_step = *s;
-  auto L_ = [&](const char* b, int l) { return std::string(b) + std::to_string(l); };
   auto bn = [&](int l) -> int {
     float* rm = bn_running + (int64_t)l * 2 * H;
     float* rv = rm + H;
     if (training)
-      return launch_bn_stats(dims, p->f(L_("z", l)), H, params + p->off_bn_g(l), params + p->off_bn_b(l), rm, rv,
-                             p->f(L_("bn_mean", l)), p->f(L_("bn_invstd", l)), p->f(L_("bn_scale", l)),
-                             p->f(L_("bn_shift", l)), p->f("bn_partials"), p->Nc, st);
-    return launch_bn_eval_coeffs(params + p->off_bn_g(l), params + p->off_bn_b(l), rm, rv, H, p->f(L_("bn_scale", l)),
-                                 p->f(L_("bn_shift", l)), st, p->f(L_("bn_mean", l)), p->f(L_("bn_invstd", l)));
+      return launch_bn_stats(dims, w.z[l], H, params + p->off_bn_g(l), params + p->off_bn_b(l), rm, rv, w.bn_mean[l],
+                             w.bn_invstd[l], w.bn_scale[l], w.bn_shift[l], w.bn_partials, p->Nc, st);
+    return launch_bn_eval_coeffs(params + p->off_bn_g(l), params + p->off_bn_b(l), rm, rv, H, w.bn_scale[l], w.bn_shift[l],
+                                 st, w.bn_mean[l], w.bn_invstd[l]);
   };
   auto fuse = [&](int l) {
     float* rm = bn_running + (int64_t)l * 2 * H;
-    float* scratch = p->f("bn_partials");
-    return BnFuse{reinterpret_cast<double*>(scratch + 16), reinterpret_cast<unsigned int*>(scratch),
-                  params + p->off_bn_g(l), params + p->off_bn_b(l), rm, rm + H, p->f(L_("bn_mean", l)),
-                  p->f(L_("bn_invstd", l)), p->f(L_("bn_scale", l)), p->f(L_("bn_shift", l)), H};
+    return BnFuse{reinterpret_cast<double*>(w.bn_partials + 16), reinterpret_cast<unsigned int*>(w.bn_partials),
+                  params + p->off_bn_g(l), params + p->off_bn_b(l), rm, rm + H, w.bn_mean[l], w.bn_invstd[l], w.bn_scale[l],
+                  w.bn_shift[l], H};
   };
   {  // layer 0: dense transform of K1's 6-wide aggregate, BatchNorm statistics fused when training
     BnFuse bf{};
     if (training) bf = fuse(0);
-    float* zero = training ? p->f("u1") : nullptr;
-    const int64_t zero_bytes = reinterpret_cast<char*>(p->buf["dG"].ptr) + p->buf["dG"].bytes - reinterpret_cast<char*>(p->buf["u1"].ptr);
-    STAGE(ST_LAYER0_FWD, 1, launch_layer0_fwd(dims, p->f("norm"), p->f("a0"), F, params + p->off_gcn_w(0), params + p->off_gcn_b(0),
-                               H, p->f("z0"), p->Nc, st, training ? &bf : nullptr, zero, zero_bytes / 16));
+    // training: the kernel also zeroes the split-K head outputs, the range [u1, end of dG) (contiguous: eims_plan_create)
+    float* zero = training ? w.u1 : nullptr;
+    STAGE(ST_LAYER0_FWD, 1, launch_layer0_fwd(dims, t.norm, t.a0, F, params + p->off_gcn_w(0), params + p->off_gcn_b(0),
+                               H, w.z[0], p->Nc, st, training ? &bf : nullptr, zero, p->head_zero_bytes / 16));
     if (!training) STAGE(ST_BN_STATS, 1, bn(0));
   }
   // every launch from here on is at least two kernels after the batch build: sizes before the grid-dependency wait
   EarlyDimsScope early_scope(1);
   const bool planes = p->planes_on();
   if (planes)  // hi / lo planes of the GraphConv weights W_1 .. W_{L-1} (one pass over the range that holds them)
-    STAGE(ST_ELEMENTWISE, 1, launch_split_planes(params + p->off_gcn_w(1), p->f("wplanes"), p->f("wplanes") + p->w_plane, p->w_plane, st, true));
+    STAGE(ST_ELEMENTWISE, 1, launch_split_planes(params + p->off_gcn_w(1), w.wplanes, w.wplanes + p->w_plane, p->w_plane, st, true));
   for (int l = 1; l < L; ++l) {
     // training on the tensor-core path: the BatchNorm statistics of z_l come out of the GEMM epilogue
     const bool fuse_bn = training && p->gemm_backend == EIMS_GEMM_TCGEN05;
     BnFuse bf{};
     if (fuse_bn) bf = fuse(l);
-    STAGE(ST_SPMM_FWD, 1, launch_spmm_norm(dims, p->i("rowptr"), p->i("col"), p->f("norm"), p->f(L_("z", l - 1)), H,
-                              p->f(L_("bn_scale", l - 1)), p->f(L_("bn_shift", l - 1)),
-                              p->drop(drop_p, seed, step, l - 1), 0, p->f(L_("a", l)), p->Nc, st, nullptr, p->i("gptr"), p->Bc,
+    STAGE(ST_SPMM_FWD, 1, launch_spmm_norm(dims, t.rowptr, t.col, t.norm, w.z[l - 1], H, w.bn_scale[l - 1], w.bn_shift[l - 1],
+                              p->drop(drop_p, seed, step, l - 1), 0, w.a[l], p->Nc, st, nullptr, t.gptr, p->Bc,
                               p->tile_rows(), planes ? p->act_plane : 0));
     if (planes) {
-      GemmTmaProblem fw{p->map_a_k(l), p->map_w_mn(l), p->f(L_("z", l)), H, 0, 1, p->Nc, H, H, dims + DIM_N, nullptr, p->f("norm"),
-                        params + p->off_gcn_b(l), 1, 0, fuse_bn ? &bf : nullptr};
+      GemmTmaProblem fw{.ta = p->map_a_k(l), .tb = p->map_w_mn(l), .C = w.z[l], .ldc = H, .b_mn = 1, .M = p->Nc, .N = H,
+                        .K = H, .m_dev = dims + DIM_N, .row_scale = t.norm, .bias = params + p->off_gcn_b(l), .relu = 1,
+                        .bn = fuse_bn ? &bf : nullptr};
       STAGE(ST_GEMM_GCN_FWD, 1, launch_gemm_tma(&fw, nullptr, st));
     } else {
-      STAGE(ST_GEMM_GCN_FWD, 1, gemm(p, p->f(L_("a", l)), H, 0, params + p->off_gcn_w(l), H, 1, p->f(L_("z", l)), H, p->Nc, H, H,
-                    dims + DIM_N, nullptr, p->f("norm"), params + p->off_gcn_b(l), 1, 0, st, fuse_bn ? &bf : nullptr));
+      STAGE(ST_GEMM_GCN_FWD, 1, launch_gemm(p->gemm_backend,
+            GemmProblem{.A = w.a[l], .lda = H, .B = params + p->off_gcn_w(l), .ldb = H, .b_mn = 1, .C = w.z[l], .ldc = H,
+                        .M = p->Nc, .N = H, .K = H, .m_dev = dims + DIM_N, .row_scale = t.norm,
+                        .bias = params + p->off_gcn_b(l), .relu = 1, .bn = fuse_bn ? &bf : nullptr}, st));
     }
     if (!fuse_bn) STAGE(ST_BN_STATS, 1, bn(l));
   }
   // The 512-row head GEMMs cannot fill 148 SMs with output tiles, so in training they split K and
   // accumulate with float atomics (summation order varies in the last bit run to run); eval-mode
   // forwards keep plain stores and are bit-reproducible.
-  const int head_acc = training ? 3 : 0;  // 3 = split-K allowed, C already zeroed (by the layer-0 kernel)
-  STAGE(ST_READOUT, 1, launch_readout(dims, p->i("gptr"), p->f(L_("z", L - 1)), H, p->f(L_("bn_scale", L - 1)),
-                          p->f(L_("bn_shift", L - 1)), d.pooling, p->f("readout"), p->i("argmax"), p->Bc, st,
-                          training ? p->f("zstat") : nullptr, training ? p->f(L_("bn_mean", L - 1)) : nullptr));
-  STAGE(ST_GEMM_HEAD_FWD, 1, gemm(p, p->f("readout"), P, 0, params + p->off_head(0), P, 0, p->f("u1"), 2 * H, p->Bc, 2 * H, P,
-                dims + DIM_B, nullptr, nullptr, params + p->off_head(1), 0, head_acc, st));
-  STAGE(ST_LN_FWD, 1, launch_ln_fwd(dims, p->f("u1"), 2 * H, params + p->off_head(2), params + p->off_head(3),
-                         p->drop(drop_p, seed, step, L), p->f("y1"), p->f("ln1"), p->Bc, st));
-  STAGE(ST_GEMM_HEAD_FWD, 1, gemm(p, p->f("y1"), 2 * H, 0, params + p->off_head(4), 2 * H, 0, p->f("u2"), H, p->Bc, H, 2 * H,
-                dims + DIM_B, nullptr, nullptr, params + p->off_head(5), 0, head_acc, st));
-  STAGE(ST_LN_FWD, 1, launch_ln_fwd(dims, p->f("u2"), H, params + p->off_head(6), params + p->off_head(7),
-                         p->drop(drop_p, seed, step, L + 1), p->f("y2"), p->f("ln2"), p->Bc, st));
-  STAGE(ST_GEMM_HEAD_FWD, 1, gemm(p, p->f("y2"), H, 0, params + p->off_head(8), H, 0, p->f("logits"), M, p->Bc, M, H, dims + DIM_B,
-                nullptr, nullptr, params + p->off_head(9), 0, head_acc, st));
-  p->state = training ? 2 : 1;
-  p->last_training = training;
-  p->eval_fwd = !training;
+  const GemmAcc head_acc = training ? kGemmStoreSplitZeroed : kGemmStore;  // C zeroed by the layer-0 kernel
+  STAGE(ST_READOUT, 1, launch_readout(dims, t.gptr, w.z[L - 1], H, w.bn_scale[L - 1], w.bn_shift[L - 1], d.pooling, w.readout,
+                          w.argmax, p->Bc, st, training ? w.zstat : nullptr, training ? w.bn_mean[L - 1] : nullptr));
+  STAGE(ST_GEMM_HEAD_FWD, 1, launch_gemm(p->gemm_backend,
+        GemmProblem{.A = w.readout, .lda = P, .B = params + p->off_head(0), .ldb = P, .C = w.u1, .ldc = 2 * H, .M = p->Bc,
+                    .N = 2 * H, .K = P, .m_dev = dims + DIM_B, .bias = params + p->off_head(1), .accumulate = head_acc}, st));
+  STAGE(ST_LN_FWD, 1, launch_ln_fwd(dims, w.u1, 2 * H, params + p->off_head(2), params + p->off_head(3),
+                         p->drop(drop_p, seed, step, L), w.y1, w.ln1, p->Bc, st));
+  STAGE(ST_GEMM_HEAD_FWD, 1, launch_gemm(p->gemm_backend,
+        GemmProblem{.A = w.y1, .lda = 2 * H, .B = params + p->off_head(4), .ldb = 2 * H, .C = w.u2, .ldc = H, .M = p->Bc,
+                    .N = H, .K = 2 * H, .m_dev = dims + DIM_B, .bias = params + p->off_head(5), .accumulate = head_acc}, st));
+  STAGE(ST_LN_FWD, 1, launch_ln_fwd(dims, w.u2, H, params + p->off_head(6), params + p->off_head(7),
+                         p->drop(drop_p, seed, step, L + 1), w.y2, w.ln2, p->Bc, st));
+  STAGE(ST_GEMM_HEAD_FWD, 1, launch_gemm(p->gemm_backend,
+        GemmProblem{.A = w.y2, .lda = H, .B = params + p->off_head(8), .ldb = H, .C = w.logits, .ldc = M, .M = p->Bc, .N = M,
+                    .K = H, .m_dev = dims + DIM_B, .bias = params + p->off_head(9), .accumulate = head_acc}, st));
+  p->phase = training ? Phase::train_fwd : Phase::eval_fwd;
   return check_launch("eims_forward");
 }
 
 int eims_sigmoid(eims_plan* p, eims_stream_t stream) {
   if (!p || !p->bound) return fail(EIMS_ERR_STATE, "plan not bound");
   cudaStream_t st = (cudaStream_t)stream;
-  STAGE(ST_ELEMENTWISE, 1, launch_sigmoid(p->i("dims"), p->f("logits"), p->d.max_mz, p->f("prob"), p->Bc, (cudaStream_t)stream));
+  STAGE(ST_ELEMENTWISE, 1, launch_sigmoid(p->tab().dims, p->ws.logits, p->d.max_mz, p->ws.prob, p->Bc, (cudaStream_t)stream));
   return check_launch("eims_sigmoid");
 }
 
@@ -744,13 +793,15 @@ static int loss_impl(eims_plan* p, const float* targets, const int32_t* target_r
   if (!targets && !peaks && p->peak_targets.peak_ptr) peaks = &p->peak_targets;
   if (!targets && !peaks) return fail(EIMS_ERR_ARG, "targets is NULL (and no peak-list targets are set)");
   cudaStream_t st = (cudaStream_t)stream;
-  EarlyDimsScope early_scope(p->state >= 2 ? 1 : 0);  // after a forward, never right after a batch build
+  // after a training forward, never right after a batch build (nor after an eval forward, which may follow one)
+  EarlyDimsScope early_scope(p->after_train_fwd() ? 1 : 0);
   // metrics != NULL: the last block of the loss kernel also folds the row terms into the running
   // metrics (flags[0] is its ticket), which saves the separate one-block launch
-  STAGE(ST_LOSS, 1, launch_loss(p->i("dims"), p->f("logits"), targets, target_rows, p->d.max_mz, loss_kind, p->f("prob"),
-                       want_grad ? p->f("dlogits") : nullptr, p->f("row_loss"), p->f("row_cos"), p->Bc,
-                       (cudaStream_t)stream, metrics, reinterpret_cast<unsigned int*>(p->i("flags")), peaks));
-  if (want_grad && p->state == 2) p->state = 3;
+  const Workspace& w = p->ws;
+  STAGE(ST_LOSS, 1, launch_loss(p->tab().dims, w.logits, targets, target_rows, p->d.max_mz, loss_kind, w.prob,
+                       want_grad ? w.dlogits : nullptr, w.row_loss, w.row_cos, p->Bc,
+                       (cudaStream_t)stream, metrics, reinterpret_cast<unsigned int*>(w.flags), peaks));
+  if (want_grad && p->phase == Phase::train_fwd) p->phase = Phase::loss_grad;
   return check_launch("eims_loss");
 }
 
@@ -764,32 +815,33 @@ int eims_loss(eims_plan* p, const float* targets, const int32_t* target_rows, in
 // The callers have checked the plan's state.
 static int backward_impl(eims_plan* p, const float* params, const float* dprob, float* grads, int32_t part, float* dfeat,
                          bool eval, cudaStream_t st) {
-  EarlyDimsScope early_scope(1);  // backward always follows a forward (state >= 2, or an eval forward)
+  EarlyDimsScope early_scope(1);  // backward always follows a forward (training or eval)
   const eims_dims& d = p->d;
   const int H = d.hidden_dim, F = d.node_feat_dim, L = d.num_gcn_layers, M = d.max_mz, P = p->pool_dim();
-  const int* dims = p->i("dims");
+  const BatchTables& t = p->tab();
+  const Workspace& w = p->ws;
+  const int* dims = t.dims;
   // eval mode: no dropout, BatchNorm is the affine map of the running statistics (bn_mean<l> / bn_invstd<l> hold them,
   // written by the eval forward), so its backward has no batch-statistics terms: the two column means the apply pass
   // subtracts stay zero (the statistics passes get means == NULL)
   const float drop_p = (!eval && d.dropout > 0.f) ? d.dropout : 0.f;
   const float drop_scale = drop_p > 0.f ? 1.f / (1.f - drop_p) : 1.f;
-  float* means2 = eval ? nullptr : p->f("bn_means2");
+  float* means2 = eval ? nullptr : w.bn_means2;
   // the head data gradients: a training forward's layer-0 kernel zeroed dy2 / dy1 / dG (split-K allowed); an eval
   // forward zeroes nothing, so there they are plain stores
-  const int head_acc = eval ? 0 : 3;
+  const GemmAcc head_acc = eval ? kGemmStore : kGemmStoreSplitZeroed;
   const uint64_t seed = p->last_step.seed;
   const int step = p->last_step.step;
   const bool planes = p->planes_on();  // as in the forward that produced a_l (the backend must not change in between)
-  auto L_ = [&](const char* b, int l) { return std::string(b) + std::to_string(l); };
   if (eval) {
-    if (cudaMemsetAsync(p->f("bn_means2"), 0, 2 * (size_t)H * sizeof(float), st) != cudaSuccess)
+    if (cudaMemsetAsync(w.bn_means2, 0, 2 * (size_t)H * sizeof(float), st) != cudaSuccess)
       return fail(EIMS_ERR_CUDA, "cudaMemsetAsync failed");
     // prob of this forward (an eval forward leaves only the logits; eims_sigmoid may not have run)
-    STAGE(ST_ELEMENTWISE, 1, launch_sigmoid(dims, p->f("logits"), M, p->f("prob"), p->Bc, st));
+    STAGE(ST_ELEMENTWISE, 1, launch_sigmoid(dims, w.logits, M, w.prob, p->Bc, st));
   }
   if (part != EIMS_BWD_GCN) {
-  if (dprob) STAGE(ST_ELEMENTWISE, 1, launch_dprob_to_dlogits(dims, p->f("prob"), dprob, M, p->f("dlogits"), p->Bc, st));
-  float* dl = p->f("dlogits");
+  if (dprob) STAGE(ST_ELEMENTWISE, 1, launch_dprob_to_dlogits(dims, w.prob, dprob, M, w.dlogits, p->Bc, st));
+  float* dl = w.dlogits;
   // ---- head (GCN:341-352 backwards)
   const int* dB = dims + DIM_B;
   if (p->side) {  // fork: the bias gradient of the output layer is needed by AdamW only
@@ -802,20 +854,26 @@ static int backward_impl(eims_plan* p, const float* params, const float* dprob, 
     STAGE(ST_COLSUM, 1, launch_colsum(dims, DIM_B, dl, M, M, grads + p->off_head(9), p->Bc, st));
   }
   STAGE(ST_GEMM_HEAD_BWD, p->gemm_backend == EIMS_GEMM_TCGEN05 ? 1 : 2, gemm_pair(p,
-        GemmProblem{dl, M, 1, p->f("y2"), H, 1, grads + p->off_head(8), H, M, H, p->Bc, nullptr, dB, nullptr, nullptr, 0, 1, nullptr},
-        GemmProblem{dl, M, 0, params + p->off_head(8), H, 1, p->f("dy2"), H, p->Bc, H, M, dB, nullptr, nullptr, nullptr, 0, head_acc, nullptr}, st));
+        GemmProblem{.A = dl, .lda = M, .a_mn = 1, .B = w.y2, .ldb = H, .b_mn = 1, .C = grads + p->off_head(8), .ldc = H,
+                    .M = M, .N = H, .K = p->Bc, .k_dev = dB, .accumulate = kGemmAdd},
+        GemmProblem{.A = dl, .lda = M, .B = params + p->off_head(8), .ldb = H, .b_mn = 1, .C = w.dy2, .ldc = H, .M = p->Bc,
+                    .N = H, .K = M, .m_dev = dB, .accumulate = head_acc}, st));
   // LayerNorm backward also leaves the bias gradient of the Linear in front of it (column sums of du)
-  STAGE(ST_LN_BWD, 1, launch_ln_bwd(dims, p->f("u2"), p->f("y2"), p->f("dy2"), H, params + p->off_head(6), p->f("ln2"), drop_scale,
-                         p->f("dy2"), grads + p->off_head(6), grads + p->off_head(7), grads + p->off_head(5), p->Bc, st));
+  STAGE(ST_LN_BWD, 1, launch_ln_bwd(dims, w.u2, w.y2, w.dy2, H, params + p->off_head(6), w.ln2, drop_scale,
+                         w.dy2, grads + p->off_head(6), grads + p->off_head(7), grads + p->off_head(5), p->Bc, st));
   STAGE(ST_GEMM_HEAD_BWD, p->gemm_backend == EIMS_GEMM_TCGEN05 ? 1 : 2, gemm_pair(p,
-        GemmProblem{p->f("dy2"), H, 1, p->f("y1"), 2 * H, 1, grads + p->off_head(4), 2 * H, H, 2 * H, p->Bc, nullptr, dB, nullptr, nullptr, 0, 1, nullptr},
-        GemmProblem{p->f("dy2"), H, 0, params + p->off_head(4), 2 * H, 1, p->f("dy1"), 2 * H, p->Bc, 2 * H, H, dB, nullptr, nullptr, nullptr, 0, head_acc, nullptr}, st));
-  STAGE(ST_LN_BWD, 1, launch_ln_bwd(dims, p->f("u1"), p->f("y1"), p->f("dy1"), 2 * H, params + p->off_head(2), p->f("ln1"),
-                         drop_scale, p->f("dy1"), grads + p->off_head(2), grads + p->off_head(3), grads + p->off_head(1), p->Bc, st));
+        GemmProblem{.A = w.dy2, .lda = H, .a_mn = 1, .B = w.y1, .ldb = 2 * H, .b_mn = 1, .C = grads + p->off_head(4),
+                    .ldc = 2 * H, .M = H, .N = 2 * H, .K = p->Bc, .k_dev = dB, .accumulate = kGemmAdd},
+        GemmProblem{.A = w.dy2, .lda = H, .B = params + p->off_head(4), .ldb = 2 * H, .b_mn = 1, .C = w.dy1, .ldc = 2 * H,
+                    .M = p->Bc, .N = 2 * H, .K = H, .m_dev = dB, .accumulate = head_acc}, st));
+  STAGE(ST_LN_BWD, 1, launch_ln_bwd(dims, w.u1, w.y1, w.dy1, 2 * H, params + p->off_head(2), w.ln1,
+                         drop_scale, w.dy1, grads + p->off_head(2), grads + p->off_head(3), grads + p->off_head(1), p->Bc, st));
   STAGE(ST_GEMM_HEAD_BWD, p->gemm_backend == EIMS_GEMM_TCGEN05 ? 1 : 2, gemm_pair(p,
-        GemmProblem{p->f("dy1"), 2 * H, 1, p->f("readout"), P, 1, grads + p->off_head(0), P, 2 * H, P, p->Bc, nullptr, dB, nullptr, nullptr, 0, 1, nullptr},
-        GemmProblem{p->f("dy1"), 2 * H, 0, params + p->off_head(0), P, 1, p->f("dG"), P, p->Bc, P, 2 * H, dB, nullptr, nullptr, nullptr, 0, head_acc, nullptr}, st));
-  if (!eval) p->state = 4;  // head gradients final (the data-parallel reducer may start on that bucket)
+        GemmProblem{.A = w.dy1, .lda = 2 * H, .a_mn = 1, .B = w.readout, .ldb = P, .b_mn = 1, .C = grads + p->off_head(0),
+                    .ldc = P, .M = 2 * H, .N = P, .K = p->Bc, .k_dev = dB, .accumulate = kGemmAdd},
+        GemmProblem{.A = w.dy1, .lda = 2 * H, .B = params + p->off_head(0), .ldb = P, .b_mn = 1, .C = w.dG, .ldc = P,
+                    .M = p->Bc, .N = P, .K = 2 * H, .m_dev = dB, .accumulate = head_acc}, st));
+  if (!eval) p->phase = Phase::head_bwd;  // head gradients final (the data-parallel reducer may start on that bucket)
   }
   if (part == EIMS_BWD_HEAD) return check_launch("eims_backward_part");
   // ---- GCN layers, last to first (GCN:358-363 backwards)
@@ -824,48 +882,51 @@ static int backward_impl(eims_plan* p, const float* params, const float* dprob, 
     // from per-graph quantities; the layers below read the dh that the backward SpMM of the layer above wrote, and their
     // statistics pass rides on that SpMM when fuse_bn_bwd_stats (see below)
     const bool from_readout = (l == L - 1);
-    const float* dh_in = from_readout ? nullptr : p->f("dh");
+    const float* dh_in = from_readout ? nullptr : w.dh;
     if (from_readout) {
       if (eval)  // the per-graph sums a training readout leaves in zstat, about the running mean
-        STAGE(ST_BN_BWD_STATS, 1, launch_bn_eval_zstat(dims, p->i("gptr"), p->f(L_("z", l)), H, p->f(L_("bn_mean", l)), p->i("argmax"),
-                                     d.pooling, p->f("zstat"), p->Bc, st));
-      STAGE(ST_BN_BWD_STATS, 1, launch_bn_bwd_stats_top(dims, p->f("dG"), p->f("zstat"), p->i("gptr"), d.pooling, H, p->f(L_("bn_mean", l)),
-                                   p->f(L_("bn_invstd", l)), grads + p->off_bn_g(l), grads + p->off_bn_b(l), means2,
-                                   p->f("bn_partials"), p->Bc, st));
+        STAGE(ST_BN_BWD_STATS, 1, launch_bn_eval_zstat(dims, t.gptr, w.z[l], H, w.bn_mean[l], w.argmax, d.pooling, w.zstat,
+                                     p->Bc, st));
+      STAGE(ST_BN_BWD_STATS, 1, launch_bn_bwd_stats_top(dims, w.dG, w.zstat, t.gptr, d.pooling, H, w.bn_mean[l],
+                                   w.bn_invstd[l], grads + p->off_bn_g(l), grads + p->off_bn_b(l), means2,
+                                   w.bn_partials, p->Bc, st));
     } else if (!p->fuse_bn_bwd_stats) {
-      STAGE(ST_BN_BWD_STATS, 1, launch_bn_bwd_stats(dims, dh_in, p->f(L_("z", l)), H, p->f(L_("bn_mean", l)), p->f(L_("bn_invstd", l)),
-                                   grads + p->off_bn_g(l), grads + p->off_bn_b(l), means2, p->f("bn_partials"), p->Nc, st));
+      STAGE(ST_BN_BWD_STATS, 1, launch_bn_bwd_stats(dims, dh_in, w.z[l], H, w.bn_mean[l], w.bn_invstd[l],
+                                   grads + p->off_bn_g(l), grads + p->off_bn_b(l), means2, w.bn_partials, p->Nc, st));
     }
-    STAGE(ST_BN_BWD_APPLY, 1, launch_bn_bwd_apply(dims, dh_in, p->f("dG"), p->i("gid"), p->i("gptr"), p->i("argmax"), d.pooling,
-                                 p->f(L_("z", l)), H, p->f(L_("bn_mean", l)), p->f(L_("bn_invstd", l)), params + p->off_bn_g(l),
-                                 p->f("norm"), grads + p->off_gcn_b(l), p->f("bn_means2"), p->f("q"), p->Nc, st,
-                                 l == 0 ? p->f("a0") : nullptr, F, l == 0 ? grads + p->off_gcn_w(0) : nullptr,
+    STAGE(ST_BN_BWD_APPLY, 1, launch_bn_bwd_apply(dims, dh_in, w.dG, t.gid, t.gptr, w.argmax, d.pooling,
+                                 w.z[l], H, w.bn_mean[l], w.bn_invstd[l], params + p->off_bn_g(l),
+                                 t.norm, grads + p->off_gcn_b(l), w.bn_means2, w.q, p->Nc, st,
+                                 l == 0 ? t.a0 : nullptr, F, l == 0 ? grads + p->off_gcn_w(0) : nullptr,
                                  (planes && l > 0) ? p->act_plane : 0, l == 0 && dfeat));
     if (l > 0 && planes) {
       // one persistent launch: data gradient tiles (stores) + weight gradient k-slices (red.add), balanced on the device
-      GemmTmaProblem dg{p->map_q_k(), p->map_w_k(l), p->f("da"), H, 0, 0, p->Nc, H, H, dims + DIM_N, nullptr, nullptr, nullptr, 0, 0, nullptr};
-      GemmTmaProblem wg{p->map_a_mn(l), p->map_q_mn(), grads + p->off_gcn_w(l), H, 1, 1, H, H, p->Nc, nullptr, dims + DIM_N, nullptr, nullptr, 0, 1, nullptr};
+      GemmTmaProblem dg{.ta = p->map_q_k(), .tb = p->map_w_k(l), .C = w.da, .ldc = H, .M = p->Nc, .N = H, .K = H,
+                        .m_dev = dims + DIM_N};
+      GemmTmaProblem wg{.ta = p->map_a_mn(l), .tb = p->map_q_mn(), .C = grads + p->off_gcn_w(l), .ldc = H, .a_mn = 1, .b_mn = 1,
+                        .M = H, .N = H, .K = p->Nc, .k_dev = dims + DIM_N, .red = 1};
       STAGE(ST_GEMM_GCN_BWD, 1, launch_gemm_tma(&dg, &wg, st));
     } else if (l > 0) {
       STAGE(ST_GEMM_GCN_BWD, p->gemm_backend == EIMS_GEMM_TCGEN05 ? 1 : 2, gemm_pair(p,
-            GemmProblem{p->f(L_("a", l)), H, 1, p->f("q"), H, 1, grads + p->off_gcn_w(l), H, H, H, p->Nc, nullptr, dims + DIM_N, nullptr, nullptr, 0, 1, nullptr},
-            GemmProblem{p->f("q"), H, 0, params + p->off_gcn_w(l), H, 0, p->f("da"), H, p->Nc, H, H, dims + DIM_N, nullptr, nullptr, nullptr, 0, 0, nullptr}, st));
+            GemmProblem{.A = w.a[l], .lda = H, .a_mn = 1, .B = w.q, .ldb = H, .b_mn = 1, .C = grads + p->off_gcn_w(l), .ldc = H,
+                        .M = H, .N = H, .K = p->Nc, .k_dev = dims + DIM_N, .accumulate = kGemmAdd},
+            GemmProblem{.A = w.q, .lda = H, .B = params + p->off_gcn_w(l), .ldb = H, .C = w.da, .ldc = H, .M = p->Nc, .N = H,
+                        .K = H, .m_dev = dims + DIM_N}, st));
     }
     if (l > 0) {
-      float* scratch = p->f("bn_partials");
-      BnBwdFuse bf{p->f(L_("z", l - 1)), p->f(L_("bn_mean", l - 1)), p->f(L_("bn_invstd", l - 1)),
-                   reinterpret_cast<double*>(scratch + 16), reinterpret_cast<unsigned int*>(scratch),
+      BnBwdFuse bf{w.z[l - 1], w.bn_mean[l - 1], w.bn_invstd[l - 1],
+                   reinterpret_cast<double*>(w.bn_partials + 16), reinterpret_cast<unsigned int*>(w.bn_partials),
                    grads + p->off_bn_g(l - 1), grads + p->off_bn_b(l - 1), means2};
-      STAGE(ST_SPMM_BWD, 1, launch_spmm_norm(dims, p->i("rowptr"), p->i("col"), p->f("norm"), p->f("da"), H, nullptr, nullptr,
-                                p->drop(drop_p, seed, step, l - 1), 1, p->f("dh"), p->Nc, st,
-                                p->fuse_bn_bwd_stats ? &bf : nullptr, p->i("gptr"), p->Bc, p->tile_rows()));
+      STAGE(ST_SPMM_BWD, 1, launch_spmm_norm(dims, t.rowptr, t.col, t.norm, w.da, H, nullptr, nullptr,
+                                p->drop(drop_p, seed, step, l - 1), 1, w.dh, p->Nc, st,
+                                p->fuse_bn_bwd_stats ? &bf : nullptr, t.gptr, p->Bc, p->tile_rows()));
     } else if (dfeat) {
       // layer 0: dW0 came out of the apply pass above, which also left q_0 in q; da and dh are free here
-      STAGE(ST_GEMM_GCN_DGRAD, 1, launch_layer0_dgrad(dims, p->f("q"), H, params + p->off_gcn_w(0), F, p->f("da"), p->Nc, st));
-      STAGE(ST_SPMM_BWD, 1, launch_feat_grad(dims, p->i("rowptr"), p->i("col"), p->f("norm"), p->f("da"), F, dfeat, p->Nc, st));
+      STAGE(ST_GEMM_GCN_DGRAD, 1, launch_layer0_dgrad(dims, w.q, H, params + p->off_gcn_w(0), F, w.da, p->Nc, st));
+      STAGE(ST_SPMM_BWD, 1, launch_feat_grad(dims, t.rowptr, t.col, t.norm, w.da, F, dfeat, p->Nc, st));
     }  // l == 0 without dfeat: q_0 is never materialised
   }
-  if (!eval) p->state = 1;
+  if (!eval) p->phase = Phase::built;
   return check_launch("eims_backward");
 }
 
@@ -873,10 +934,10 @@ int eims_backward_part(eims_plan* p, const float* params, const float* dprob, fl
                        eims_stream_t stream) {
   if (!p || !p->bound) return fail(EIMS_ERR_STATE, "plan not bound");
   if (part < EIMS_BWD_ALL || part > EIMS_BWD_GCN) return fail(EIMS_ERR_ARG, "part must be one of EIMS_BWD_*");
-  if (p->state < 2 || !p->last_training) return fail(EIMS_ERR_STATE, "eims_backward needs a training-mode eims_forward first");
+  if (!p->after_train_fwd()) return fail(EIMS_ERR_STATE, "eims_backward needs a training-mode eims_forward first");
   if (part == EIMS_BWD_GCN) {
-    if (p->state != 4) return fail(EIMS_ERR_STATE, "EIMS_BWD_GCN needs EIMS_BWD_HEAD first");
-  } else if (!dprob && p->state != 3) {
+    if (p->phase != Phase::head_bwd) return fail(EIMS_ERR_STATE, "EIMS_BWD_GCN needs EIMS_BWD_HEAD first");
+  } else if (!dprob && p->phase != Phase::loss_grad) {
     return fail(EIMS_ERR_STATE, "eims_backward without dprob needs eims_loss(want_grad=1) first");
   }
   if (!params || !grads) return fail(EIMS_ERR_ARG, "params / grads is NULL");
@@ -890,12 +951,12 @@ int eims_backward(eims_plan* p, const float* params, const float* dprob, float* 
 int eims_backward_feat(eims_plan* p, const float* params, const float* dprob, float* grads, float* dfeat,
                        eims_stream_t stream) {
   if (!p || !p->bound) return fail(EIMS_ERR_STATE, "plan not bound");
-  const bool eval = p->eval_fwd;
+  const bool eval = p->phase == Phase::eval_fwd;
   if (!eval) {
-    if (p->state < 2 || !p->last_training)
+    if (!p->after_train_fwd())
       return fail(EIMS_ERR_STATE, "eims_backward_feat needs an eims_forward of the batch built last (and no backward since)");
-    if (p->state == 4) return fail(EIMS_ERR_STATE, "eims_backward_feat after EIMS_BWD_HEAD");
-    if (!dprob && p->state != 3) return fail(EIMS_ERR_STATE, "eims_backward_feat without dprob needs eims_loss(want_grad=1) first");
+    if (p->phase == Phase::head_bwd) return fail(EIMS_ERR_STATE, "eims_backward_feat after EIMS_BWD_HEAD");
+    if (!dprob && p->phase != Phase::loss_grad) return fail(EIMS_ERR_STATE, "eims_backward_feat without dprob needs eims_loss(want_grad=1) first");
   } else if (!dprob) {
     return fail(EIMS_ERR_ARG, "dprob is NULL: an eval-mode backward needs the gradient w.r.t. the spectrum");
   }
@@ -906,7 +967,7 @@ int eims_backward_feat(eims_plan* p, const float* params, const float* dprob, fl
 int eims_metrics_accumulate(eims_plan* p, float* metrics, eims_stream_t stream) {
   if (!p || !p->bound || !metrics) return fail(EIMS_ERR_STATE, "plan not bound / metrics NULL");
   cudaStream_t st = (cudaStream_t)stream;
-  STAGE(ST_METRICS, 1, launch_metrics(p->i("dims"), p->f("row_loss"), p->f("row_cos"), p->d.max_mz, metrics, (cudaStream_t)stream));
+  STAGE(ST_METRICS, 1, launch_metrics(p->tab().dims, p->ws.row_loss, p->ws.row_cos, p->d.max_mz, metrics, (cudaStream_t)stream));
   return check_launch("eims_metrics_accumulate");
 }
 
@@ -940,7 +1001,7 @@ static int enqueue_step(eims_plan* p, const StepCall& c) {
   if (c.part != EIMS_BWD_GCN) {
     const eims_step dummy{};  // indirect: seed / step are not used, the dropout keys come from the step block
     EIMS_TRY(eims_forward(p, c.params, c.bn_running, 1, indirect ? &dummy : c.s, stream));
-    EIMS_TRY(loss_impl(p, c.targets, indirect ? p->i("bids") : c.target_rows, c.loss_kind, 1, c.metrics, stream,
+    EIMS_TRY(loss_impl(p, c.targets, indirect ? p->tab().bids : c.target_rows, c.loss_kind, 1, c.metrics, stream,
                        c.targets ? nullptr : c.peaks));
   }
   if (c.part != EIMS_BWD_ALL) return eims_backward_part(p, c.params, nullptr, c.grads, c.part, stream);
@@ -1019,7 +1080,7 @@ int eims_infer_batch(eims_plan* p, const eims_dataset* ds, const int32_t* mol_id
   EIMS_TRY(eims_forward(p, params, const_cast<float*>(bn_running), 0, nullptr, stream));
   cudaStream_t st = (cudaStream_t)stream;
   EarlyDimsScope early_scope(1);
-  STAGE(ST_ELEMENTWISE, 1, launch_sigmoid(p->i("dims"), p->f("logits"), p->d.max_mz, prob_out ? prob_out : p->f("prob"), p->Bc,
+  STAGE(ST_ELEMENTWISE, 1, launch_sigmoid(p->tab().dims, p->ws.logits, p->d.max_mz, prob_out ? prob_out : p->ws.prob, p->Bc,
                           (cudaStream_t)stream));
   return check_launch("eims_infer_batch");
 }
@@ -1055,7 +1116,7 @@ const char* eims_plan_stage_name(int32_t k) { return (k >= 0 && k < ST_COUNT) ? 
 int eims_plan_check(eims_plan* p, int32_t* num_nodes, int32_t* num_edges, eims_stream_t stream) {
   if (!p || !p->bound) return fail(EIMS_ERR_STATE, "plan not bound");
   int h[8];
-  if (cudaMemcpyAsync(h, p->i("dims"), sizeof(h), cudaMemcpyDeviceToHost, (cudaStream_t)stream) != cudaSuccess ||
+  if (cudaMemcpyAsync(h, p->tab().dims, sizeof(h), cudaMemcpyDeviceToHost, (cudaStream_t)stream) != cudaSuccess ||
       cudaStreamSynchronize((cudaStream_t)stream) != cudaSuccess)
     return fail(EIMS_ERR_CUDA, "dims read-back failed: %s", cudaGetErrorString(cudaGetLastError()));
   if (num_nodes) *num_nodes = h[DIM_N];

@@ -260,9 +260,14 @@ int eims_plan_set_gemm_backend(eims_plan* p, int32_t backend);
 #define EIMS_PLANES_ON 1
 int eims_plan_set_gemm_planes(eims_plan* p, int32_t mode);
 
-/* Named views into the bound workspace (tests / host layer).  Names: "dims","gptr","eptr",
- * "gid","src","dst","rowptr","col","norm","x","prob","logits","row_loss","row_cos",
- * "readout","argmax","a<l>","z<l>","bn_mean<l>","bn_invstd<l>". */
+/* Named views into the bound workspace (tests / host layer).  EIMS_ERR_STATE before eims_plan_bind,
+ * EIMS_ERR_ARG for an unknown name.  Names:
+ *   batch tables, held twice: "dims","gptr","eptr","gid","bids","src","dst","rowptr","col","norm","x","a0"
+ *     - the bare name is the set the calls enqueued next use, "<name>#0" / "<name>#1" a given set;
+ *   per GCN layer l: "a<l>" (l >= 1),"z<l>","bn_mean<l>","bn_invstd<l>","bn_scale<l>","bn_shift<l>";
+ *   "flags","argmax","bn_means2","bn_partials","readout","zstat","u1","u2","logits","dy2","dy1","dG",
+ *   "y1","ln1","y2","ln2","prob","dlogits","row_loss","row_cos","dh","q","da";
+ *   "wplanes" (plans whose shapes allow the planes GEMM only). */
 int eims_plan_buffer(eims_plan* p, const char* name, void** ptr, int64_t* bytes);
 
 /* K1 on the plan's buffers. */
