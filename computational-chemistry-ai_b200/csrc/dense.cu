@@ -389,9 +389,11 @@ int launch_bn_bwd_stats_top(const int* dims, const float* dG, const float* zstat
 // LAYER0: q is consumed on the spot by the first GraphConv's weight gradient dW0[f,k] += sum_i a0[i,f] * q[i,k]
 // (F <= 8 rows); it is written (plain fp32) only when STORE_Q0, i.e. when the gradient w.r.t. the atom features is
 // wanted (bn_bwd_apply_q0_kernel), and never by bn_bwd_apply_kernel<true>.
+// DGRAD_ONLY (bn_apply_dgrad_kernel, the data-only eval backward of eims_attribute_peaks): q only - no bias gradient,
+// no dW0, and the two column means are those of eval mode (zero), so they are not read.
 constexpr int kMaxF0d = 8;
 
-template <bool LAYER0, bool STORE_Q0>
+template <bool LAYER0, bool STORE_Q0, bool DGRAD_ONLY = false>
 __device__ __forceinline__ void bn_bwd_apply_body(
     const int* __restrict__ dims, const DhSrc& src, const float* __restrict__ z, int H, const float* __restrict__ mean,
     const float* __restrict__ invstd, const float* __restrict__ gamma, const float* __restrict__ means,
@@ -407,7 +409,8 @@ __device__ __forceinline__ void bn_bwd_apply_body(
   for (int f = 0; f < (LAYER0 ? kMaxF0d : 1); ++f) w[f] = make_float4(0.f, 0.f, 0.f, 0.f);
   if (c < H) {
     const float4 mu = ldg4(mean + c), is = ldg4(invstd + c), ga = ldg4(gamma + c);
-    const float4 m1 = ldg4(means + c), m2 = ldg4(means + H + c);
+    const float4 m1 = DGRAD_ONLY ? make_float4(0.f, 0.f, 0.f, 0.f) : ldg4(means + c);
+    const float4 m2 = DGRAD_ONLY ? make_float4(0.f, 0.f, 0.f, 0.f) : ldg4(means + H + c);
     const int stride = gridDim.y * kRowLanes;
 #pragma unroll 4
     for (int r = blockIdx.y * kRowLanes + rl; r < N; r += stride) {
@@ -419,7 +422,7 @@ __device__ __forceinline__ void bn_bwd_apply_body(
       o.y = v.y > 0.f ? ga.y * is.y * (d.y - m1.y - (v.y - mu.y) * is.y * m2.y) : 0.f;
       o.z = v.z > 0.f ? ga.z * is.z * (d.z - m1.z - (v.z - mu.z) * is.z * m2.z) : 0.f;
       o.w = v.w > 0.f ? ga.w * is.w * (d.w - m1.w - (v.w - mu.w) * is.w * m2.w) : 0.f;
-      acc.x += o.x; acc.y += o.y; acc.z += o.z; acc.w += o.w;
+      if (!DGRAD_ONLY) { acc.x += o.x; acc.y += o.y; acc.z += o.z; acc.w += o.w; }
       o.x *= ci; o.y *= ci; o.z *= ci; o.w *= ci;
       if (LAYER0) {
 #pragma unroll
@@ -446,6 +449,7 @@ __device__ __forceinline__ void bn_bwd_apply_body(
       }
     }
   }
+  if (DGRAD_ONLY) return;
   red[rl][cl * 4 + 0] = acc.x; red[rl][cl * 4 + 1] = acc.y; red[rl][cl * 4 + 2] = acc.z; red[rl][cl * 4 + 3] = acc.w;
   __syncthreads();
   if (threadIdx.x < kSlab && c0 + threadIdx.x < H) {
@@ -489,6 +493,25 @@ __global__ void __launch_bounds__(256, 2) bn_bwd_apply_q0_kernel(
     const float* __restrict__ norm, float* __restrict__ q, float* __restrict__ dbias, const float* __restrict__ a0,
     int F, float* __restrict__ dW0, int early) {
   bn_bwd_apply_body<true, true>(dims, src, z, H, mean, invstd, gamma, means, norm, q, dbias, a0, F, dW0, early, 0);
+}
+
+// the data-only eval backward (eims_attribute_peaks): q = c * (gamma * invstd * dh) * [z > 0], nothing else
+__global__ void __launch_bounds__(256, 4) bn_apply_dgrad_kernel(
+    const int* __restrict__ dims, DhSrc src, const float* __restrict__ z, int H, const float* __restrict__ mean,
+    const float* __restrict__ invstd, const float* __restrict__ gamma, const float* __restrict__ norm,
+    float* __restrict__ q, int early, int64_t q_lo_off) {
+  bn_bwd_apply_body<false, false, true>(dims, src, z, H, mean, invstd, gamma, nullptr, norm, q, nullptr, nullptr, 0, nullptr,
+                                        early, q_lo_off);
+}
+
+int launch_bn_dgrad_apply(const int* dims, const float* dh, const float* dG, const int* gid, const int* gptr,
+                          const int* argmax, int pooling, const float* z, int H, const float* mean, const float* invstd,
+                          const float* gamma, const float* norm, float* q, int max_nodes, cudaStream_t st, int64_t q_lo_off) {
+  if (H % 4 || H > 4096 || (q_lo_off & 3)) return EIMS_ERR_ARG;
+  const DhSrc src{dh, dG, gid, gptr, argmax, pooling};
+  launch_pdl(bn_apply_dgrad_kernel, bn_grid(H, max_nodes), dim3(256), 0, st, dims, src, z, H, mean, invstd, gamma, norm, q,
+             dims_early_ref(), q_lo_off);
+  return 0;
 }
 
 int launch_bn_bwd_stats(const int* dims, const float* dh, const float* z, int H, const float* mean, const float* invstd,
@@ -688,6 +711,138 @@ int launch_ln_bwd(const int* dims, const float* u, const float* y, const float* 
 #undef EIMS_LN_B
     default: return EIMS_ERR_ARG;
   }
+  return 0;
+}
+
+// data-only backward of eval mode (eims_attribute_peaks): du only, no dgamma / dbeta / bias gradient (and so no shared
+// partials and no atomics); no dropout.  du may alias dy.  Warp per row, the arithmetic of ln_relu_drop_bwd_kernel.
+template <int NV>
+__global__ void __launch_bounds__(256) ln_relu_dgrad_kernel(const int* __restrict__ dims, const float* __restrict__ u,
+                                                            const float* __restrict__ y, const float* dy, int W,
+                                                            const float* __restrict__ gamma, const float* __restrict__ stats,
+                                                            float* du, int early) {
+  const int B = pdl_sync_dims(dims, early).B;
+  const int lane = threadIdx.x & 31;
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int nwarps = (gridDim.x * blockDim.x) >> 5;
+  const int nv4 = W >> 2;
+  for (int r = warp; r < B; r += nwarps) {
+    const float mean = stats[2 * r], rstd = stats[2 * r + 1];
+    float4 xh[NV], g[NV];
+    float s1 = 0.f, s2 = 0.f;
+#pragma unroll
+    for (int i = 0; i < NV; ++i) {
+      const int c4 = i * 32 + lane;
+      xh[i] = g[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (c4 < nv4) {
+        const int c = 4 * c4;
+        const float4 uu = ldg4(u + (int64_t)r * W + c), yy = ldg4(y + (int64_t)r * W + c), ga = ldg4(gamma + c);
+        const float4 d = *reinterpret_cast<const float4*>(dy + (int64_t)r * W + c);
+        xh[i].x = (uu.x - mean) * rstd; xh[i].y = (uu.y - mean) * rstd;
+        xh[i].z = (uu.z - mean) * rstd; xh[i].w = (uu.w - mean) * rstd;
+        g[i].x = yy.x > 0.f ? d.x * ga.x : 0.f; g[i].y = yy.y > 0.f ? d.y * ga.y : 0.f;
+        g[i].z = yy.z > 0.f ? d.z * ga.z : 0.f; g[i].w = yy.w > 0.f ? d.w * ga.w : 0.f;
+        s1 += g[i].x + g[i].y + g[i].z + g[i].w;
+        s2 += g[i].x * xh[i].x + g[i].y * xh[i].y + g[i].z * xh[i].z + g[i].w * xh[i].w;
+      }
+    }
+    const float m1 = warp_sum(s1) / (float)W, m2 = warp_sum(s2) / (float)W;
+#pragma unroll
+    for (int i = 0; i < NV; ++i) {
+      const int c4 = i * 32 + lane;
+      if (c4 < nv4) {
+        float4 o;
+        o.x = rstd * (g[i].x - m1 - xh[i].x * m2); o.y = rstd * (g[i].y - m1 - xh[i].y * m2);
+        o.z = rstd * (g[i].z - m1 - xh[i].z * m2); o.w = rstd * (g[i].w - m1 - xh[i].w * m2);
+        st4(du + (int64_t)r * W + 4 * c4, o);
+      }
+    }
+  }
+}
+
+int launch_ln_dgrad(const int* dims, const float* u, const float* y, const float* dy, int W, const float* gamma,
+                    const float* stats, float* du, int max_graphs, cudaStream_t st) {
+  if (W % 4 || W > 2048 || W < 4) return EIMS_ERR_ARG;
+  int blocks = (max_graphs + 7) / 8;  // 8 warps, one row each
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  if (blocks < 1) blocks = 1;
+  switch (ln_nv(W)) {
+#define EIMS_LN_D(NV) case NV: launch_pdl(ln_relu_dgrad_kernel<NV>, dim3(blocks), dim3(256), 0, st, dims, u, y, dy, W, gamma, stats, du, dims_early_ref()); break;
+    EIMS_LN_D(1) EIMS_LN_D(2) EIMS_LN_D(4) EIMS_LN_D(8) EIMS_LN_D(16)
+#undef EIMS_LN_D
+    default: return EIMS_ERR_ARG;
+  }
+  return 0;
+}
+
+// =========================================================================== peaks of eims_attribute_peaks
+// The head's first data gradient for dprob = one-hot(m_r) per row: dlogits is p (1 - p) at m_r and zero elsewhere, so
+// dy2[r, :] = p (1 - p) W3[m_r, :] with p = sigmoid(logits[r, m_r]) - a gather instead of the [B, M] x [M, H] GEMM.
+// Warp per row.
+__global__ void __launch_bounds__(256) peak_head_dgrad_kernel(const int* __restrict__ dims, const float* __restrict__ logits,
+                                                              int M, const int* __restrict__ bins, const float* __restrict__ W3,
+                                                              int H, float* __restrict__ dy2, int early) {
+  const int B = pdl_sync_dims(dims, early).B;
+  const int lane = threadIdx.x & 31;
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int nwarps = (gridDim.x * blockDim.x) >> 5;
+  for (int r = warp; r < B; r += nwarps) {
+    const int m = __ldg(bins + r);
+    const float p = 1.f / (1.f + expf(-__ldg(logits + (int64_t)r * M + m)));
+    const float s = p * (1.f - p);
+    for (int c = 4 * lane; c < H; c += 128) {
+      float4 w = ldg4(W3 + (int64_t)m * H + c);
+      w.x *= s; w.y *= s; w.z *= s; w.w *= s;
+      st4(dy2 + (int64_t)r * H + c, w);
+    }
+  }
+}
+
+// idx / val: the top-k table [rows, k] of the predicted spectra.  Graph r takes entry r mod k (the host layer puts every
+// molecule k times in a row, so the k replicas of a molecule take its k peaks).
+__global__ void peak_select_kernel(const int* __restrict__ dims, const int* __restrict__ idx, const float* __restrict__ val,
+                                   int k, int* __restrict__ bins, float* __restrict__ prob, int early) {
+  const int B = pdl_sync_dims(dims, early).B;
+  for (int r = blockIdx.x * blockDim.x + threadIdx.x; r < B; r += gridDim.x * blockDim.x) {
+    const int64_t e = (int64_t)r * k + r % k;
+    bins[r] = __ldg(idx + e);
+    prob[r] = __ldg(val + e);
+  }
+}
+
+// prob[r] = sigmoid(logits[r, bins[r]]) (the arithmetic of sigmoid_kernel)
+__global__ void peak_prob_kernel(const int* __restrict__ dims, const float* __restrict__ logits, int M,
+                                 const int* __restrict__ bins, float* __restrict__ prob, int early) {
+  const int B = pdl_sync_dims(dims, early).B;
+  for (int r = blockIdx.x * blockDim.x + threadIdx.x; r < B; r += gridDim.x * blockDim.x)
+    prob[r] = 1.f / (1.f + expf(-__ldg(logits + (int64_t)r * M + __ldg(bins + r))));
+}
+
+static inline int row_blocks(int rows, int per_block) {
+  int b = (rows + per_block - 1) / per_block;
+  if (b > 148 * 8) b = 148 * 8;
+  return b < 1 ? 1 : b;
+}
+
+int launch_peak_head_dgrad(const int* dims, const float* logits, int M, const int* bins, const float* W3, int H, float* dy2,
+                           int max_graphs, cudaStream_t st) {
+  if (H % 4) return EIMS_ERR_ARG;
+  launch_pdl(peak_head_dgrad_kernel, dim3(row_blocks(max_graphs, 8)), dim3(256), 0, st, dims, logits, M, bins, W3, H, dy2,
+             dims_early_ref());
+  return 0;
+}
+
+int launch_peak_select(const int* dims, const int* idx, const float* val, int k, int* bins, float* prob, int max_graphs,
+                       cudaStream_t st) {
+  launch_pdl(peak_select_kernel, dim3(row_blocks(max_graphs, 256)), dim3(256), 0, st, dims, idx, val, k, bins, prob,
+             dims_early_ref());
+  return 0;
+}
+
+int launch_peak_prob(const int* dims, const float* logits, int M, const int* bins, float* prob, int max_graphs,
+                     cudaStream_t st) {
+  launch_pdl(peak_prob_kernel, dim3(row_blocks(max_graphs, 256)), dim3(256), 0, st, dims, logits, M, bins, prob,
+             dims_early_ref());
   return 0;
 }
 

@@ -452,6 +452,20 @@ __global__ void __launch_bounds__(256) layer0_dgrad_kernel(const int* __restrict
   }
 }
 
+// (A da0)[j, :] for atom j: the sum over j's CSR row, ascending edge id
+__device__ __forceinline__ void feat_grad_gather(const int* __restrict__ rowptr, const int* __restrict__ col,
+                                                 const float* __restrict__ da0, int F, int j, float (&acc)[kMaxF0]) {
+#pragma unroll
+  for (int f = 0; f < kMaxF0; ++f) acc[f] = 0.f;
+  const int e0 = __ldg(rowptr + j), e1 = __ldg(rowptr + j + 1);
+  for (int e = e0; e < e1; ++e) {
+    const int i = __ldg(col + e);
+#pragma unroll
+    for (int f = 0; f < kMaxF0; ++f)
+      if (f < F) acc[f] += __ldg(da0 + (int64_t)i * F + f);
+  }
+}
+
 __global__ void __launch_bounds__(256) feat_grad_kernel(const int* __restrict__ dims, const int* __restrict__ rowptr,
                                                         const int* __restrict__ col, const float* __restrict__ norm,
                                                         const float* __restrict__ da0, int F, float* __restrict__ dx,
@@ -459,20 +473,44 @@ __global__ void __launch_bounds__(256) feat_grad_kernel(const int* __restrict__ 
   const int N = pdl_sync_dims(dims, early).N;
   for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < N; j += gridDim.x * blockDim.x) {
     float acc[kMaxF0];
-#pragma unroll
-    for (int f = 0; f < kMaxF0; ++f) acc[f] = 0.f;
-    const int e0 = __ldg(rowptr + j), e1 = __ldg(rowptr + j + 1);
-    for (int e = e0; e < e1; ++e) {
-      const int i = __ldg(col + e);
-#pragma unroll
-      for (int f = 0; f < kMaxF0; ++f)
-        if (f < F) acc[f] += __ldg(da0 + (int64_t)i * F + f);
-    }
+    feat_grad_gather(rowptr, col, da0, F, j, acc);
     const float cj = __ldg(norm + j);
 #pragma unroll
     for (int f = 0; f < kMaxF0; ++f)
       if (f < F) dx[(int64_t)j * F + f] = acc[f] * cj;
   }
+}
+
+// Integrated gradients (eims_attribute_peaks): the feature gradient dx = D A da0 of one path point, weighted and summed
+// into ig - ig = w dx on the first point, ig += w dx after it; on the last point (x != NULL) the sum is then multiplied
+// by the atom features.  One thread per atom: no atomics, the sum over the path points runs in their order.
+__global__ void __launch_bounds__(256) ig_feat_accum_kernel(const int* __restrict__ dims, const int* __restrict__ rowptr,
+                                                            const int* __restrict__ col, const float* __restrict__ norm,
+                                                            const float* __restrict__ da0, int F, float w, int first,
+                                                            const float* __restrict__ x, float* __restrict__ ig, int early) {
+  const int N = pdl_sync_dims(dims, early).N;
+  for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < N; j += gridDim.x * blockDim.x) {
+    float acc[kMaxF0];
+    feat_grad_gather(rowptr, col, da0, F, j, acc);
+    const float cj = __ldg(norm + j);
+#pragma unroll
+    for (int f = 0; f < kMaxF0; ++f)
+      if (f < F) {
+        const int64_t o = (int64_t)j * F + f;
+        float v = acc[f] * cj * w;
+        if (!first) v += ig[o];
+        if (x) v *= __ldg(x + o);
+        ig[o] = v;
+      }
+  }
+}
+
+// out[i] = alpha * in[i] over the batch's N x F values (a0 at a point alpha X of the path: a0 is linear in x)
+__global__ void __launch_bounds__(256) feat_scale_kernel(const int* __restrict__ dims, const float* __restrict__ in, int F,
+                                                         float alpha, float* __restrict__ out, int early) {
+  const int64_t n = (int64_t)pdl_sync_dims(dims, early).N * F;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+    out[i] = alpha * __ldg(in + i);
 }
 
 int launch_layer0_dgrad(const int* dims, const float* q0, int H, const float* W0, int F, float* da0, int max_nodes,
@@ -492,6 +530,23 @@ int launch_feat_grad(const int* dims, const int* rowptr, const int* col, const f
   if (blocks > 148 * 8) blocks = 148 * 8;
   launch_pdl(feat_grad_kernel, dim3(blocks < 1 ? 1 : blocks), dim3(256), 0, st, dims, rowptr, col, norm, da0, F, dx,
              dims_early_ref());
+  return 0;
+}
+
+int launch_ig_feat_accum(const int* dims, const int* rowptr, const int* col, const float* norm, const float* da0, int F,
+                         float w, bool first, const float* x, float* ig, int max_nodes, cudaStream_t st) {
+  if (F < 1 || F > kMaxF0) return EIMS_ERR_ARG;
+  int blocks = (max_nodes + 255) / 256;
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  launch_pdl(ig_feat_accum_kernel, dim3(blocks < 1 ? 1 : blocks), dim3(256), 0, st, dims, rowptr, col, norm, da0, F, w,
+             first ? 1 : 0, x, ig, dims_early_ref());
+  return 0;
+}
+
+int launch_feat_scale(const int* dims, const float* in, int F, float alpha, float* out, int max_nodes, cudaStream_t st) {
+  int64_t blocks = ((int64_t)max_nodes * F + 255) / 256;
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  launch_pdl(feat_scale_kernel, dim3(blocks < 1 ? 1 : (int)blocks), dim3(256), 0, st, dims, in, F, alpha, out, dims_early_ref());
   return 0;
 }
 

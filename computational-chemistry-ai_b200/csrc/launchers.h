@@ -38,6 +38,11 @@ int launch_layer0_dgrad(const int* dims, const float* q0, int H, const float* W0
                         cudaStream_t st);
 int launch_feat_grad(const int* dims, const int* rowptr, const int* col, const float* norm, const float* da0, int F,
                      float* dx, int max_nodes, cudaStream_t st);
+// integrated gradients (eims_attribute_peaks): ig (=|+=) w * D A da0, then ig *= x when x != NULL
+int launch_ig_feat_accum(const int* dims, const int* rowptr, const int* col, const float* norm, const float* da0, int F,
+                         float w, bool first, const float* x, float* ig, int max_nodes, cudaStream_t st);
+// out = alpha * in over the batch's N x F values
+int launch_feat_scale(const int* dims, const float* in, int F, float alpha, float* out, int max_nodes, cudaStream_t st);
 int launch_readout(const int* dims, const int* gptr, const float* z, int H, const float* bn_scale,
                    const float* bn_shift, int pooling, float* out, int* argmax, int max_graphs, cudaStream_t st,
                    float* zstat = nullptr, const float* bn_mean = nullptr);  // zstat [B][2H]: per graph, column sums of
@@ -83,11 +88,27 @@ int launch_bn_bwd_apply(const int* dims, const float* dh, const float* dG, const
                         cudaStream_t st, const float* a0 = nullptr, int F = 0, float* dW0 = nullptr,
                         int64_t q_lo_off = 0,     // != 0: q as stacked tf32 hi / lo planes
                         bool store_q0 = false);   // layer 0 (dW0 set): also store q_0 into q as plain fp32
+// the data-only eval backward (eims_attribute_peaks): q only, no bias gradient / dW0 / column means
+int launch_bn_dgrad_apply(const int* dims, const float* dh, const float* dG, const int* gid, const int* gptr,
+                          const int* argmax, int pooling, const float* z, int H, const float* mean, const float* invstd,
+                          const float* gamma, const float* norm, float* q, int max_nodes, cudaStream_t st,
+                          int64_t q_lo_off = 0);
 int launch_ln_fwd(const int* dims, const float* u, int W, const float* gamma, const float* beta, DropCfg drop, float* y,
                   float* stats, int max_graphs, cudaStream_t st);
 int launch_ln_bwd(const int* dims, const float* u, const float* y, const float* dy, int W, const float* gamma,
                   const float* stats, float drop_scale, float* du, float* dgamma, float* dbeta, float* dbias,
                   int max_graphs, cudaStream_t st);
+// eval mode, data gradient only (no dgamma / dbeta / bias gradient, no dropout)
+int launch_ln_dgrad(const int* dims, const float* u, const float* y, const float* dy, int W, const float* gamma,
+                    const float* stats, float* du, int max_graphs, cudaStream_t st);
+// peaks of eims_attribute_peaks: dy2[r] = p(1-p) W3[bins[r]]; bins / prob from the top-k table (entry r mod k);
+// prob[r] = sigmoid(logits[r, bins[r]])
+int launch_peak_head_dgrad(const int* dims, const float* logits, int M, const int* bins, const float* W3, int H, float* dy2,
+                           int max_graphs, cudaStream_t st);
+int launch_peak_select(const int* dims, const int* idx, const float* val, int k, int* bins, float* prob, int max_graphs,
+                       cudaStream_t st);
+int launch_peak_prob(const int* dims, const float* logits, int M, const int* bins, float* prob, int max_graphs,
+                     cudaStream_t st);
 int launch_loss(const int* dims, const float* logits, const float* targets, const int* target_rows, int M,
                 int loss_kind, float* prob, float* dlogits, float* row_loss, float* row_cos, int max_graphs,
                 cudaStream_t st, float* metrics = nullptr, unsigned int* ticket = nullptr,

@@ -810,11 +810,21 @@ int eims_loss(eims_plan* p, const float* targets, const int32_t* target_rows, in
   return loss_impl(p, targets, target_rows, loss_kind, want_grad, nullptr, stream);
 }
 
+// The data-only eval backward of eims_attribute_peaks: the gradient of prob[r, bins[r]] summed over the graphs, down to
+// the atom features only, weighted into the integrated gradients (launch_ig_feat_accum).
+struct PeakGrad {
+  const int* bins;  // m_r per graph
+  float weight;     // 1 / steps
+  bool first;       // the first path point: ig = weight * dx (later: ig += weight * dx)
+  const float* x;   // the last path point: the atom features ig is then multiplied by (else NULL)
+};
+
 // The backward of the forward enqueued last, for every public entry point: the training step's (eval = false, dfeat
-// NULL: eims_backward, eims_backward_part) and eims_backward_feat's (either mode, optionally down to the atom features).
+// NULL: eims_backward, eims_backward_part), eims_backward_feat's (either mode, optionally down to the atom features) and
+// eims_attribute_peaks' (pg != NULL: eval mode, no parameter gradients - grads is not touched - and into dfeat = ig).
 // The callers have checked the plan's state.
 static int backward_impl(eims_plan* p, const float* params, const float* dprob, float* grads, int32_t part, float* dfeat,
-                         bool eval, cudaStream_t st) {
+                         bool eval, cudaStream_t st, const PeakGrad* pg = nullptr) {
   EarlyDimsScope early_scope(1);  // backward always follows a forward (training or eval)
   const eims_dims& d = p->d;
   const int H = d.hidden_dim, F = d.node_feat_dim, L = d.num_gcn_layers, M = d.max_mz, P = p->pool_dim();
@@ -833,17 +843,30 @@ static int backward_impl(eims_plan* p, const float* params, const float* dprob, 
   const uint64_t seed = p->last_step.seed;
   const int step = p->last_step.step;
   const bool planes = p->planes_on();  // as in the forward that produced a_l (the backend must not change in between)
-  if (eval) {
+  const int* dB = dims + DIM_B;
+  if (pg) {
+    // ---- head, data gradients only: dy2 gathered from W3's row m_r, LayerNorm backward without its parameter
+    // gradients, and the two remaining products as plain data-gradient GEMMs
+    STAGE(ST_ELEMENTWISE, 1, launch_peak_head_dgrad(dims, w.logits, M, pg->bins, params + p->off_head(8), H, w.dy2, p->Bc, st));
+    STAGE(ST_LN_BWD, 1, launch_ln_dgrad(dims, w.u2, w.y2, w.dy2, H, params + p->off_head(6), w.ln2, w.dy2, p->Bc, st));
+    STAGE(ST_GEMM_HEAD_DGRAD, 1, launch_gemm(p->gemm_backend,
+          GemmProblem{.A = w.dy2, .lda = H, .B = params + p->off_head(4), .ldb = 2 * H, .b_mn = 1, .C = w.dy1, .ldc = 2 * H,
+                      .M = p->Bc, .N = 2 * H, .K = H, .m_dev = dB}, st));
+    STAGE(ST_LN_BWD, 1, launch_ln_dgrad(dims, w.u1, w.y1, w.dy1, 2 * H, params + p->off_head(2), w.ln1, w.dy1, p->Bc, st));
+    STAGE(ST_GEMM_HEAD_DGRAD, 1, launch_gemm(p->gemm_backend,
+          GemmProblem{.A = w.dy1, .lda = 2 * H, .B = params + p->off_head(0), .ldb = P, .b_mn = 1, .C = w.dG, .ldc = P,
+                      .M = p->Bc, .N = P, .K = 2 * H, .m_dev = dB}, st));
+  }
+  if (eval && !pg) {
     if (cudaMemsetAsync(w.bn_means2, 0, 2 * (size_t)H * sizeof(float), st) != cudaSuccess)
       return fail(EIMS_ERR_CUDA, "cudaMemsetAsync failed");
     // prob of this forward (an eval forward leaves only the logits; eims_sigmoid may not have run)
     STAGE(ST_ELEMENTWISE, 1, launch_sigmoid(dims, w.logits, M, w.prob, p->Bc, st));
   }
-  if (part != EIMS_BWD_GCN) {
+  if (part != EIMS_BWD_GCN && !pg) {
   if (dprob) STAGE(ST_ELEMENTWISE, 1, launch_dprob_to_dlogits(dims, w.prob, dprob, M, w.dlogits, p->Bc, st));
   float* dl = w.dlogits;
   // ---- head (GCN:341-352 backwards)
-  const int* dB = dims + DIM_B;
   if (p->side) {  // fork: the bias gradient of the output layer is needed by AdamW only
     if (cudaEventRecord(p->ev[0], st) != cudaSuccess || cudaStreamWaitEvent(p->side, p->ev[0], 0) != cudaSuccess)
       return fail(EIMS_ERR_CUDA, "side-branch fork failed: %s", cudaGetErrorString(cudaGetLastError()));
@@ -883,6 +906,30 @@ static int backward_impl(eims_plan* p, const float* params, const float* dprob, 
     // statistics pass rides on that SpMM when fuse_bn_bwd_stats (see below)
     const bool from_readout = (l == L - 1);
     const float* dh_in = from_readout ? nullptr : w.dh;
+    if (pg) {
+      // eval-mode BatchNorm backward: the statistics passes only produce dgamma / dbeta; layer 0 leaves q_0 plain
+      STAGE(ST_BN_BWD_APPLY, 1, launch_bn_dgrad_apply(dims, dh_in, w.dG, t.gid, t.gptr, w.argmax, d.pooling, w.z[l], H,
+                                   w.bn_mean[l], w.bn_invstd[l], params + p->off_bn_g(l), t.norm, w.q, p->Nc, st,
+                                   (planes && l > 0) ? p->act_plane : 0));
+      if (l > 0 && planes) {
+        GemmTmaProblem dg{.ta = p->map_q_k(), .tb = p->map_w_k(l), .C = w.da, .ldc = H, .M = p->Nc, .N = H, .K = H,
+                          .m_dev = dims + DIM_N};
+        STAGE(ST_GEMM_GCN_DGRAD, 1, launch_gemm_tma(&dg, nullptr, st));
+      } else if (l > 0) {
+        STAGE(ST_GEMM_GCN_DGRAD, 1, launch_gemm(p->gemm_backend,
+              GemmProblem{.A = w.q, .lda = H, .B = params + p->off_gcn_w(l), .ldb = H, .C = w.da, .ldc = H, .M = p->Nc,
+                          .N = H, .K = H, .m_dev = dims + DIM_N}, st));
+      }
+      if (l > 0) {
+        STAGE(ST_SPMM_BWD, 1, launch_spmm_norm(dims, t.rowptr, t.col, t.norm, w.da, H, nullptr, nullptr, make_drop(0.f, 0, 0, 0),
+                                  1, w.dh, p->Nc, st, nullptr, t.gptr, p->Bc, p->tile_rows()));
+      } else {
+        STAGE(ST_GEMM_GCN_DGRAD, 1, launch_layer0_dgrad(dims, w.q, H, params + p->off_gcn_w(0), F, w.da, p->Nc, st));
+        STAGE(ST_SPMM_BWD, 1, launch_ig_feat_accum(dims, t.rowptr, t.col, t.norm, w.da, F, pg->weight, pg->first, pg->x,
+                                     dfeat, p->Nc, st));
+      }
+      continue;
+    }
     if (from_readout) {
       if (eval)  // the per-graph sums a training readout leaves in zstat, about the running mean
         STAGE(ST_BN_BWD_STATS, 1, launch_bn_eval_zstat(dims, t.gptr, w.z[l], H, w.bn_mean[l], w.argmax, d.pooling, w.zstat,
@@ -962,6 +1009,48 @@ int eims_backward_feat(eims_plan* p, const float* params, const float* dprob, fl
   }
   if (!params || !grads) return fail(EIMS_ERR_ARG, "params / grads is NULL");
   return backward_impl(p, params, dprob, grads, EIMS_BWD_ALL, dfeat, eval, (cudaStream_t)stream);
+}
+
+int eims_attribute_peaks(eims_plan* p, const float* params, const float* bn_running, int32_t k, int32_t steps, int32_t* bins,
+                         float* peak_prob, float* base_prob, float* ig, void* scratch, eims_stream_t stream) {
+  if (!p || !p->bound) return fail(EIMS_ERR_STATE, "plan not bound");
+  if (p->phase == Phase::unbuilt) return fail(EIMS_ERR_STATE, "eims_attribute_peaks before eims_batch_build");
+  if (!params || !bn_running || !bins || !peak_prob || !base_prob || !ig || !scratch)
+    return fail(EIMS_ERR_ARG, "params / bn_running / bins / peak_prob / base_prob / ig / scratch is NULL");
+  if (k < 1 || k > p->d.max_mz || steps < 1) return fail(EIMS_ERR_ARG, "need 1 <= k <= max_mz and steps >= 1");
+  if (reinterpret_cast<uintptr_t>(scratch) & 255) return fail(EIMS_ERR_ARG, "scratch must be 256-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int F = p->d.node_feat_dim, M = p->d.max_mz;
+  const BatchTables& t = p->tab();
+  const Workspace& w = p->ws;
+  float* params_f = const_cast<float*>(params);
+  float* running = const_cast<float*>(bn_running);  // an eval forward only reads it
+  // scratch: the unscaled a0 [N, F], then the top-k table of the spectra at alpha = 1 (bins [B, k], values [B, k])
+  auto r = [](int64_t bytes) { return (bytes + 255) & ~(int64_t)255; };
+  char* c = reinterpret_cast<char*>(scratch);
+  float* a0 = reinterpret_cast<float*>(c);
+  int* top_idx = reinterpret_cast<int*>(c + r((int64_t)p->Nc * F * 4));
+  float* top_val = reinterpret_cast<float*>(c + r((int64_t)p->Nc * F * 4) + r((int64_t)p->Bc * k * 4));
+  STAGE(ST_ELEMENTWISE, 1, launch_feat_scale(t.dims, t.a0, F, 1.f, a0, p->Nc, st));
+  // alpha = 1: the predicted spectra and their peaks
+  EIMS_TRY(eims_forward(p, params_f, running, 0, nullptr, stream));
+  STAGE(ST_ELEMENTWISE, 1, launch_sigmoid(t.dims, w.logits, M, w.prob, p->Bc, st));
+  STAGE(ST_ELEMENTWISE, 1, launch_topk_peaks(w.prob, p->Bc, M, k, top_idx, top_val, st));
+  STAGE(ST_ELEMENTWISE, 1, launch_peak_select(t.dims, top_idx, top_val, k, bins, peak_prob, p->Bc, st));
+  // alpha = 0: the baseline
+  STAGE(ST_ELEMENTWISE, 1, launch_feat_scale(t.dims, a0, F, 0.f, t.a0, p->Nc, st));
+  EIMS_TRY(eims_forward(p, params_f, running, 0, nullptr, stream));
+  STAGE(ST_ELEMENTWISE, 1, launch_peak_prob(t.dims, w.logits, M, bins, base_prob, p->Bc, st));
+  // the path: a0 = A D (alpha x) = alpha a0, so the forward at alpha X starts from the scaled aggregate
+  for (int s = 0; s < steps; ++s) {
+    STAGE(ST_ELEMENTWISE, 1, launch_feat_scale(t.dims, a0, F, ((float)s + 0.5f) / (float)steps, t.a0, p->Nc, st));
+    EIMS_TRY(eims_forward(p, params_f, running, 0, nullptr, stream));
+    const PeakGrad pg{bins, 1.f / (float)steps, s == 0, s == steps - 1 ? t.x : nullptr};
+    EIMS_TRY(backward_impl(p, params, nullptr, nullptr, EIMS_BWD_ALL, ig, true, st, &pg));
+  }
+  STAGE(ST_ELEMENTWISE, 1, launch_feat_scale(t.dims, a0, F, 1.f, t.a0, p->Nc, st));  // the batch tables as K1 left them
+  p->phase = Phase::built;
+  return check_launch("eims_attribute_peaks");
 }
 
 int eims_metrics_accumulate(eims_plan* p, float* metrics, eims_stream_t stream) {

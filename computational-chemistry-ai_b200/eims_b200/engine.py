@@ -434,6 +434,29 @@ class Plan:
         batch's atom features written into it.  dprob may be None only after loss(want_grad=True) in training mode."""
         check(self.lib.eims_backward_feat(self.h, ptr(fp.params), ptr(dprob), ptr(fp.grads), ptr(dfeat), self.stream))
 
+    def attribute_scratch_bytes(self, k: int) -> int:
+        """Bytes of the scratch eims_attribute_peaks needs for top-k attribution on this plan (include/eims_b200.h)."""
+        return 4 * self.max_nodes * self.d.node_feat_dim + 8 * self.max_graphs * int(k) + 512
+
+    def attribute_peaks(self, fp: FlatParams, k: int, steps: int, num_graphs=None, num_nodes=None):
+        """Integrated gradients of every graph's (r mod k)-th predicted peak on the batch built last, in eval mode
+        (eims_attribute_peaks).  Returns device tensors bins int32 [B], peak_prob [B], base_prob [B] (the baseline of
+        all-zero features) and ig [N, F] in batch order.  B / N: the batch's sizes (default: those of the last build,
+        N read back from the device)."""
+        B = int(num_graphs if num_graphs is not None else self.num_graphs)
+        N = int(num_nodes if num_nodes is not None else self.check()[0])
+        dev = self.device
+        bins = torch.empty(B, dtype=torch.int32, device=dev)
+        peak_prob = torch.empty(B, dtype=torch.float32, device=dev)
+        base_prob = torch.empty(B, dtype=torch.float32, device=dev)
+        ig = torch.empty((N, self.d.node_feat_dim), dtype=torch.float32, device=dev)
+        scratch = torch.empty(self.attribute_scratch_bytes(k) + 256, dtype=torch.uint8, device=dev)
+        base = (scratch.data_ptr() + 255) // 256 * 256
+        check(self.lib.eims_attribute_peaks(self.h, ptr(fp.params), ptr(fp.bn_running), int(k), int(steps), ptr(bins),
+                                            ptr(peak_prob), ptr(base_prob), ptr(ig), C.c_void_p(base), self.stream))
+        self._attr_scratch = scratch  # alive until the kernels that use it have run
+        return bins, peak_prob, base_prob, ig
+
     def metrics_accumulate(self, metrics):
         check(self.lib.eims_metrics_accumulate(self.h, ptr(metrics), self.stream))
 

@@ -691,6 +691,47 @@ def predict_graphs(model, graphs, batch_size=4096, top_k=0):
             np.concatenate(vals) if vals else np.zeros((0, top_k), np.float32))
 
 
+def attribute_peaks(model, graphs, k=5, steps=32, batch_size=4096):
+    """Per-atom attribution of every molecule's k strongest predicted peaks by integrated gradients (eval mode, zero
+    baseline, midpoint rule with `steps` points; eims_attribute_peaks in include/eims_b200.h).  Each molecule is put k
+    times in a row, so one pass attributes all its peaks; a pass holds at most `batch_size` replica graphs.
+    Returns (bins int32 [n, k], prob [n, k], delta [n, k], ig) with bins / prob the peaks of `--mode predict`'s report
+    (value descending), delta = prob - prob at the all-zero baseline, and ig a list of n arrays [k, n_atoms, F]:
+    ig[j].sum() ~= delta[:, j] per molecule (completeness), ig[j].sum(1) the per-atom attribution of peak j."""
+    from .engine import PackedDataset
+    k, steps = int(k), int(steps)
+    if k < 1 or k > model.dims.max_mz or steps < 1:
+        raise ValueError(f"need 1 <= k <= max_mz ({model.dims.max_mz}) and steps >= 1")
+    model.eval()
+    per = max(1, int(batch_size) // k)   # molecules per pass
+    bins, prob, delta, ig = [], [], [], []
+    with torch.no_grad():
+        for s in range(0, len(graphs), per):
+            chunk = graphs[s:s + per]
+            g = batch([gr for gr in chunk for _ in range(k)]).to(model.flat.device)
+            plan, fp = model._engine(g.batch_size, g.num_nodes(), g.num_edges())
+            hb = g._packed
+            model._keep = (g, None)
+            model._fwd_seq += 1   # the activations of an earlier forward are overwritten
+            plan.batch_build(PackedDataset(g._dev_buf.data_ptr(), hb.offsets, hb.num_graphs), None, hb.num_graphs)
+            plan.check()          # raises ZeroInDegreeError like DGL's GraphConv
+            b, p, p0, x = plan.attribute_peaks(fp, k, steps, hb.num_graphs, g.num_nodes())
+            n = len(chunk)
+            bins.append(b.view(n, k).cpu().numpy())
+            p = p.view(n, k)
+            prob.append(p.cpu().numpy())
+            delta.append((p - p0.view(n, k)).cpu().numpy())
+            x = x.cpu().numpy()
+            start = 0
+            for gr in chunk:
+                na = gr.num_nodes()
+                ig.append(x[start:start + k * na].reshape(k, na, -1))
+                start += k * na
+    if not bins:
+        return (np.zeros((0, k), np.int32), np.zeros((0, k), np.float32), np.zeros((0, k), np.float32), [])
+    return np.concatenate(bins), np.concatenate(prob), np.concatenate(delta), ig
+
+
 # ------------------------------------------------------------------------------ data parallel (new; the reference is single-GPU)
 def _init_data_parallel():
     """(world, rank).  Under torchrun (WORLD_SIZE > 1 in the environment) joins the NCCL process group, one process

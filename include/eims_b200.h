@@ -302,6 +302,27 @@ int eims_backward(eims_plan* p, const float* params, const float* dprob, float* 
  * dfeat (may be NULL): d/dx of the batch's atom features, [N, F] in batch order, rows [0, N) overwritten. */
 int eims_backward_feat(eims_plan* p, const float* params, const float* dprob, float* grads, float* dfeat,
                        eims_stream_t stream);
+/* Per-atom attribution of each graph's top predicted peak by integrated gradients (IG), on the batch built last.
+ * Definition (new functionality; the reference has no attribution):
+ *   - eval mode: BatchNorm uses the running statistics, dropout is off;
+ *   - baseline: all-zero atom features on the same graph;
+ *   - the peak bin m_r of graph r is the (r mod k)-th largest bin of graph r's own predicted spectrum (the report of
+ *     eims_topk_peaks: value descending, exact ties to the higher bin);
+ *   - midpoint rule with S = steps points, alpha_s = (s + 1/2) / S, weight 1/S:
+ *       ig[i, f] = x[i, f] * (1/S) * sum_s  d prob_{m_r} / d x[i, f]  at alpha_s * X      (i an atom of graph r)
+ *     so that sum over graph r's atoms and features of ig ~= peak_prob[r] - base_prob[r] (completeness).
+ * A caller that puts each molecule k times in a row (replica j of molecule g is graph g*k + j) gets all k peaks of every
+ * molecule from one call.  Outputs: bins[B] (m_r), peak_prob[B] (prob_{m_r}(X)), base_prob[B] (prob_{m_r}(0)), ig[N, F]
+ * in batch order; rows past the batch are not written.
+ * scratch: caller-owned device memory, 256-byte aligned, of at least 4*N*F + 8*B*k + 512 bytes with N = max_nodes and
+ * B = max_graphs of the plan (an unscaled copy of K1's aggregate a0 and the top-k table).
+ * Each path point is an eval forward plus a backward to the atom features that computes no parameter gradient.  No
+ * float atomics: a molecule's outputs do not depend on the other graphs of the batch.
+ * EIMS_ERR_ARG: a NULL pointer, k outside [1, max_mz], steps < 1 or misaligned scratch; EIMS_ERR_STATE: no batch built.
+ * Parameters and running statistics are not touched.  The plan is left as after eims_batch_build: a backward call
+ * afterwards is refused until the next forward. */
+int eims_attribute_peaks(eims_plan* p, const float* params, const float* bn_running, int32_t k, int32_t steps, int32_t* bins,
+                         float* peak_prob, float* base_prob, float* ig, void* scratch, eims_stream_t stream);
 /* The same in two parts, EIMS_BWD_HEAD then EIMS_BWD_GCN: after the head part the gradients of
  * the 10 spectrum_predictor tensors (the tail of the flat buffer, 84 % of its bytes) are final,
  * so a data-parallel caller can start reducing that bucket while the GCN layers are
